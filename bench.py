@@ -5,6 +5,7 @@
     python bench.py --workload corona45|brca2_global|brca2_local|reads150|nw1m ...      # one workload only
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's CPU algorithm (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR    # also write what the kernels computed in the last timed step as DIR/*.npy
 
 A "step" is one pass of the hot path over the workload's batch of pairs:
   value      kernels only, sequences resident in HBM (gx_plan_execute / gx_band_execute), device-timed with CUDA events
@@ -19,10 +20,12 @@ torch is used for process-group plumbing (rendezvous, barrier, max over ranks) a
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -30,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree (which may be read-only)
 
 from genomics_rs_b200 import workloads as wl  # noqa: E402
 
@@ -79,6 +83,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.gpu), f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                                           "-lms", "200"], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)     # a run that fails before stop() must not leave the sampler running
             self.th = threading.Thread(target=self._pump, daemon=True)
             self.th.start()
         except OSError:
@@ -187,13 +192,14 @@ def cpu_baseline_sample(march_native: bool = True, rows: int = 12000, threads: i
     """The reference's algorithm as written (oracle faithful variant: 48 B cells, F-order table, i-outer/j-inner)
     on a bounded sample of the workload: the first `rows` x `rows` bases of corona pair (0,1), global + retrace."""
     from oracle import gxo
-    so = gxo.build(march="native") if march_native else None
     seqs, jobs = wl.corona_pairs()
     a, b = seqs[0][:rows], seqs[1][:rows]
     cells = (len(a) + 1) * (len(b) + 1)
-    t0 = time.perf_counter()
-    r = gxo.align_faithful(a, b, SCORES, False, so=so)
-    dt = time.perf_counter() - t0
+    with tempfile.TemporaryDirectory() as tmp:      # the host-tuned oracle is compiled outside the tree
+        so = gxo.build(march="native", out_dir=tmp) if march_native else None
+        t0 = time.perf_counter()
+        r = gxo.align_faithful(a, b, SCORES, False, so=so)
+        dt = time.perf_counter() - t0
     out = dict(value=cells / dt / 1e9, unit="GCUPS", cores=threads, kind="port",
                sample=f"oracle faithful variant (48 B cells, column-major, single thread like algo.rs), global NW + retrace of the "
                       f"first {rows}x{rows} bases of corona pair (Covid_Australia, Covid_Brazil): {cells} cells in {dt:.2f} s "
@@ -234,7 +240,8 @@ def run_reference(args):
         return
     from concurrent.futures import ThreadPoolExecutor
     from oracle import gxo
-    so = gxo.build(march="native")
+    tmp = tempfile.TemporaryDirectory()      # the host-tuned oracle is compiled outside the tree (removed on return)
+    so = gxo.build(march="native", out_dir=tmp.name)
     ncpu = os.cpu_count() or 1
     threads = max(1, min(ncpu, 32))
     # the largest prefix whose 48 B/cell tables fit a third of the free host memory with one aligner per thread
@@ -353,6 +360,27 @@ def check_gold(w, res, ops, ops_off) -> bool:
     return bool(ok)
 
 
+RESULT_FIELDS = ("score", "start_i", "start_j", "end_i", "end_j", "n_ops", "matches", "mismatches", "gap_extensions",
+                 "opening_gaps")
+SCORE_SAMPLE = 1 << 20      # score-only batches with more pairs are dumped as this many pairs, a fixed seeded sample
+
+
+def dump_outputs(args, env, workload: str, arrays: dict) -> None:
+    """--dump-outputs DIR: what this rank's last timed step computed, as DIR/<workload>_<array>.npy (float64; the op
+    codes float32).  With several ranks every rank writes its own shard, the file names ending in _rank<r>."""
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    tag = f"_rank{env.rank}" if env.world > 1 else ""
+    for key, v in arrays.items():
+        np.save(os.path.join(args.dump_outputs, f"{workload}_{key}{tag}.npy"), np.asarray(v, np.float32 if key == "ops" else np.float64))
+
+
+def traceback_outputs(res, ops, ops_off) -> dict:
+    """per-pair results, and the op codes of every pair in walk order, concatenated (ops_off holds capacities)"""
+    out = {f: res[f] for f in RESULT_FIELDS}
+    out["ops"] = np.concatenate([ops[int(o):int(o) + int(k)] for o, k in zip(ops_off[:-1], res["n_ops"])])
+    return out
+
+
 def run_plan_workload(env, args, name: str, steps: int, warmup: int, headline: bool):
     """corona45 / brca2_* / reads150 through a resident plan (kernels only) and the public host-buffer call (e2e)."""
     import genomics_rs_b200 as gx
@@ -394,6 +422,12 @@ def run_plan_workload(env, args, name: str, steps: int, warmup: int, headline: b
     if w["traceback"]:
         res, ops, ops_off = plan.fetch()
         parity["goldens"] = check_gold(w, res, ops, ops_off)
+        if args.dump_outputs:
+            dump_outputs(args, env, name, traceback_outputs(res, ops, ops_off))
+    elif args.dump_outputs:
+        scores = plan.fetch_scores()
+        pick = np.arange(n) if n <= SCORE_SAMPLE else np.sort(np.random.default_rng(0).choice(n, SCORE_SAMPLE, replace=False))
+        dump_outputs(args, env, name, {"pair": w["first"] + pick, "score": scores[pick]})
     # ---- end to end: host buffers in, host buffers out, through the public batch call
     if w["traceback"]:
         res = np.zeros(n, dtype=gx.RESULT_DTYPE)
@@ -571,11 +605,10 @@ def run_banded(env, args, steps: int, warmup: int, headline: bool = False):
     e2e_step()
     env.sync_all()
     t0 = time.perf_counter()
-    e2e_steps = max(1, min(steps, 3))
-    for _ in range(e2e_steps):
+    for _ in range(steps):
         e2e_score = e2e_step()
     env.sync_all()
-    e2e_ms = (time.perf_counter() - t0) * 1e3 / e2e_steps
+    e2e_ms = (time.perf_counter() - t0) * 1e3 / steps
 
     banded.clear_cache()
     ms_step, e2e_step_ms, fill_max = env.reduce([wall_ms, e2e_ms, fill_ms / steps], "max")
@@ -586,6 +619,8 @@ def run_banded(env, args, steps: int, warmup: int, headline: bool = False):
     out = None
     if rank == 0:
         final_score = int(final_score)
+        if args.dump_outputs:
+            dump_outputs(args, env, "nw1m", {"score": [final_score]})
         full_ok = (gold is None) or (final_score == gold and e2e_score == gold)
         par = dict(band_parity)
         par[str(n)] = bool(full_ok)
@@ -649,7 +684,10 @@ def main():
     ap.add_argument("--length", type=int, default=1_000_000, help="nw1m: bases per sequence")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-k0", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of every workload's last timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -669,12 +707,12 @@ def main():
         line = run_plan_workload(env, args, head_name, args.steps, args.warmup, headline=True)
     if args.workload == "all" and not args.only_headline:
         configs = {}
-        sec_steps, sec_warm = max(1, min(args.steps, 5)), max(3, min(args.warmup, 3))
+        sec_warm = max(3, min(args.warmup, 3))
         for name in SECONDARY:
             t0 = time.perf_counter()
             try:
-                rec = run_banded(env, args, min(sec_steps, 3), sec_warm) if name == "nw1m" else \
-                    run_plan_workload(env, args, name, sec_steps, sec_warm, headline=False)
+                rec = run_banded(env, args, args.steps, sec_warm) if name == "nw1m" else \
+                    run_plan_workload(env, args, name, args.steps, sec_warm, headline=False)
                 if env.rank == 0:
                     configs[CONFIG_KEY[name]] = slim(rec)
                     configs[CONFIG_KEY[name]]["bench_seconds"] = time.perf_counter() - t0

@@ -55,13 +55,14 @@ class OracleAlignment:
         return [(CHOICE_NAMES[c], int(i), int(j)) for c, i, j in zip(self.ops, self.ops_i, self.ops_j)]
 
 
-def build(march: Optional[str] = None, force: bool = False) -> str:
-    """Compile the oracle with gcc.  `march="native"` builds a host-tuned copy (bench cpu_baseline)."""
+def build(march: Optional[str] = None, force: bool = False, out_dir: Optional[str] = None) -> str:
+    """Compile the oracle with gcc.  `march="native"` builds a host-tuned copy (bench cpu_baseline) into `out_dir`
+    (default oracle/_build)."""
     if march is None:
         if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(os.path.join(_HERE, "gx_oracle.c")):
             subprocess.check_call(["make", "-C", _HERE, "-s"] + (["-B"] if force else []))
         return _SO
-    out = os.path.join(_HERE, "_build", f"libgxoracle_{march}.so")
+    out = os.path.join(out_dir or os.path.join(_HERE, "_build"), f"libgxoracle_{march}.so")
     os.makedirs(os.path.dirname(out), exist_ok=True)
     cc = "/usr/bin/gcc" if os.path.exists("/usr/bin/gcc") else "gcc"
     subprocess.check_call([cc, "-O3", f"-march={march}", "-fPIC", "-std=c11", "-shared", "-o", out,
