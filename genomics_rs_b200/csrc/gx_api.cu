@@ -222,6 +222,7 @@ struct gx_plan {
     float fill_ms = 0, walk_ms = 0;
     int launches = 0;
     int retries = 0;                   // resident-strips executes that were repeated in ticket mode
+    int reads_bits = 0;                // read plans: lane width of the kernel the last execute ran (16: s16x2, 32)
     bool code_band = false;            // global traceback plan in ticket mode: only tiles near the diagonal write direction codes
     uint8_t *d_tile_codes = nullptr;   // one flag per tile (indexed like tile_best)
     int band_fallbacks = 0;            // executes repeated with codes everywhere because a path left the band
@@ -372,7 +373,10 @@ static int check_scores_impl(gx_scores sc, uint64_t m, uint64_t n, bool local) {
     if ((long long)(m + n + 2) * mx + std::llabs((long long)sc.h) >= lim) return GX_ERR_RANGE;
     if (local) {
         long long vmax = (long long)std::min(m, n) * std::max<long long>(sc.s_match, 0);
-        if (vmax >= (1ll << 26)) return GX_ERR_RANGE;  // (V << log2 K) | k must stay in int32 for K <= 16
+        // start-cell keys, K <= 16: the classic form keys (V << log2 K) | k, which this bound keeps in int32; the CHAIN1
+        // form keys (E << log2 K) | k with E = V + (h+g), which also needs -(h+g) < 2^(31 - log2 K): plan_create_locked
+        // keeps local start-cell plans that break it on the classic form instead of refusing them
+        if (vmax >= (1ll << 26)) return GX_ERR_RANGE;
     }
     return GX_OK;
 }
@@ -670,6 +674,12 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
             pl->n_strips = strips;
         }
         if (pl->tun.chain1 >= 0) pl->chain1 = pl->tun.chain1 != 0;
+        // CHAIN1 takes the start-cell keys of a local plan in E-space, ((V + (h+g)) << log2 K) | k.  The score contract
+        // bounds V but not h+g against 2^(31 - log2 K): from there the key of a small V wraps.  Such plans take the
+        // classic form, whose keys (V << log2 K) | k fit every valid scoring.  Applied after the GX_K / GX_CHAIN1
+        // overrides, so that no switch selects a form that cannot represent the keys.
+        const int kb = pl->K == 16 ? 4 : pl->K == 8 ? 3 : 2;
+        if (pl->track == 2 && pl->chain1 && -((long long)sc.h + sc.g) >= (1ll << (31 - kb))) pl->chain1 = false;
     }
     const int K = pl->K, R = pl->R, W = 32 * K;
     // resident-strips mode: every strip of the plan fits a warp slot of its own (single-warp CTAs, 16 per SM: the
@@ -1216,7 +1226,7 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
         rp.h = sc.h;
         rp.is_local = pl->is_local;
         CK(cudaEventRecord(c->ev[0], c->stream));
-        int rc = launch_reads(rp, (int)pl->max_len, c->sm_count, c->stream, pl->tun.reads32 != 0);
+        int rc = launch_reads(rp, (int)pl->max_len, c->sm_count, c->stream, pl->tun.reads32 != 0, &pl->reads_bits);
         if (rc == -1) return GX_ERR_UNSUPPORTED;
         CK(cudaGetLastError());
         CK(cudaEventRecord(c->ev[1], c->stream));
@@ -1536,6 +1546,8 @@ double gx_plan_stat(const gx_plan *pl, int what) {
         case 21: return pl->resident ? 1.0 : 0.0;
         case 17: return pl->chain1 ? 1.0 : 0.0;
         case 18: return pl->lcs_ms;
+        case 25: return pl->prof ? 1.0 : 0.0;
+        case 26: return (double)pl->reads_bits;
         case 10: case 11: case 12: case 13: case 14: return (double)pl->h_stats[what - 10];
         default: return -1.0;
     }

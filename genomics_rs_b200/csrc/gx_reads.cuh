@@ -284,12 +284,14 @@ static int launch_reads_gk(const ReadsParams &rp, int sm_count, cudaStream_t st)
     return 0;
 }
 
-// returns -1 if max_len is not supported by this kernel family
-static int launch_reads(const ReadsParams &rp, int max_len, int sm_count, cudaStream_t st, bool force32 = false) {
-    if (reads16_ok(rp, max_len) && !force32) {
+// returns -1 if max_len is not supported by this kernel family; *bits (if given) = lane width of the kernel launched
+static int launch_reads(const ReadsParams &rp, int max_len, int sm_count, cudaStream_t st, bool force32 = false, int *bits = nullptr) {
+    const bool s16 = reads16_ok(rp, max_len) && !force32 && max_len <= 32 * 20;
+    if (bits) *bits = s16 ? 16 : 32;
+    if (s16) {
         if (max_len <= 8 * 19) return launch_reads16_gk<8, 19>(rp, sm_count, st);
         if (max_len <= 16 * 20) return launch_reads16_gk<16, 20>(rp, sm_count, st);
-        if (max_len <= 32 * 20) return launch_reads16_gk<32, 20>(rp, sm_count, st);
+        return launch_reads16_gk<32, 20>(rp, sm_count, st);
     }
     if (max_len <= 8 * 19) return launch_reads_gk<8, 19>(rp, sm_count, st);
     if (max_len <= 16 * 20) return launch_reads_gk<16, 20>(rp, sm_count, st);

@@ -114,10 +114,18 @@ def test_local_all_zero_table(gx, oracle, k, r, chain1, monkeypatch):
                     _same(r, o, oracle, f"m={len(a)} n={len(b)} K={k} chain1={chain1}")
 
 
-@pytest.mark.parametrize("scores", [(120, -100, -20, -30), (127, -128, -1, 0), (60, -70, -50, -9), (-3, -7, -2, -4)])
+# scoring -> whether it takes the IDP.4A path: a, b, a-(h+g) and b-(h+g) must all fit a signed byte
+_BYTE_PATH = {(120, -100, -20, -30): False, (127, -128, -1, 0): False, (60, -70, -50, -9): True, (-3, -7, -2, -4): True,
+              (120, -5, -3, -4): True, (121, -5, -3, -4): False,        # a-(h+g) = 127 / 128
+              (5, -128, -1, 0): True, (5, -129, -2, 0): False,          # b = -128 / -129
+              (3, -130, -1, -1): False, (3, -131, -1, -1): False}       # b-(h+g) = -128 / -129 (b itself is out of range)
+
+
+@pytest.mark.parametrize("scores", list(_BYTE_PATH))
 def test_score_byte_range_paths(gx, oracle, scores):
     """4-letter batches score through one IDP.4A per cell when (score - (h+g)) fits a signed byte and through the compare
-    path otherwise: scorings on both sides of that edge (and an all-negative one) against the faithful oracle"""
+    path otherwise: scorings on both sides of each edge of that range (and an all-negative one) against the faithful
+    oracle, and the path the plan took (gx_plan_stat 25)"""
     rng = np.random.default_rng(sum(scores) & 0xffff)
     pairs = [random_pair(rng, int(rng.integers(1, 90)), int(rng.integers(1, 90)), similar=bool(k % 2)) for k in range(120)]
     pairs += [random_pair(rng, 300, 520), random_pair(rng, 4100, 140)]
@@ -126,6 +134,11 @@ def test_score_byte_range_paths(gx, oracle, scores):
         for (a, b), r in zip(pairs, got):
             o = oracle.align_faithful(a, b, scores, is_local) if len(a) < 1000 else oracle.align_linear(a, b, scores, is_local)
             _same(r, o, oracle, f"m={len(a)} n={len(b)} {scores} local={is_local}")
+        blob, off1, len1, off2, len2 = gx.pack_pairs(pairs)
+        plan = gx.Plan(len1, len2, scores, is_local, traceback=False)
+        plan.upload(blob, off1, off2)
+        assert plan.stat(25) == float(_BYTE_PATH[scores]), (scores, is_local)
+        plan.close()
 
 
 @pytest.mark.parametrize("scores", [CONFIG_TOML, TEST_CONFIG, (2, -1, -1, 0), (5, -4, -3, -10), (1, 0, -1, -1), (3, 1, -2, -2)])
