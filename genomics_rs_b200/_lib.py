@@ -19,7 +19,7 @@ GX_FLAG_START_CELL = 4
 
 EXPORTS = [
     "gx_init", "gx_shutdown", "gx_device_count", "gx_strerror", "gx_last_error", "gx_version", "gx_check_scores",
-    "gx_align_pair", "gx_align_batch", "gx_score_batch", "gx_plan_create", "gx_plan_upload", "gx_plan_execute",
+    "gx_align_pair", "gx_align_batch", "gx_score_batch", "gx_score_batch_cells", "gx_plan_create", "gx_plan_upload", "gx_plan_execute",
     "gx_plan_fetch", "gx_plan_fetch_scores", "gx_plan_destroy", "gx_plan_stat", "gx_plan_debug_timeline", "gx_replay_ops", "gx_k0_measure",
     "gx_band_range", "gx_band_create", "gx_band_export", "gx_band_connect", "gx_band_upload", "gx_band_execute",
     "gx_band_score", "gx_band_stat", "gx_band_destroy", "gx_nw_score_banded", "gx_debug_planes", "gx_debug_tile_order",
@@ -78,6 +78,8 @@ def load() -> C.CDLL:
         lib.gx_align_batch.restype = i32
         lib.gx_score_batch.argtypes = [vp, u64, vp, vp, vp, vp, u64, GxScores, i32, vp]
         lib.gx_score_batch.restype = i32
+        lib.gx_score_batch_cells.argtypes = [vp, u64, vp, vp, vp, vp, u64, GxScores, i32, vp, vp, vp]
+        lib.gx_score_batch_cells.restype = i32
         lib.gx_plan_create.argtypes = [vp, vp, u64, GxScores, i32, i32, C.POINTER(vp)]; lib.gx_plan_create.restype = i32
         lib.gx_plan_upload.argtypes = [vp, vp, u64, vp, vp]; lib.gx_plan_upload.restype = i32
         lib.gx_plan_execute.argtypes = [vp]; lib.gx_plan_execute.restype = i32

@@ -323,15 +323,25 @@ def score_planes(s1, s2, scores, is_local: bool):
     return tuple(out)
 
 
-def score_batch(blob: np.ndarray, off1, len1, off2, len2, scores, is_local: bool, out: Optional[np.ndarray] = None) -> np.ndarray:
+def score_batch(blob: np.ndarray, off1, len1, off2, len2, scores, is_local: bool, out: Optional[np.ndarray] = None,
+                start_cells: bool = False):
     """gx_score_batch: scores only (int64), the short-read workload's entry point.
-    `out` (int64, one entry per pair) may be supplied to keep the result buffer across calls."""
+    `out` (int64, one entry per pair) may be supplied to keep the result buffer across calls.
+    start_cells=True (gx_score_batch_cells) -> (scores, start_i, start_j): each pair's start cell as uint64 arrays, the
+    last cell that attains the maximum for local batches ((m, n) when that maximum is 0), (m, n) for global ones."""
     lib = _lib.ensure_init()
     blob = np.ascontiguousarray(blob, np.uint8)
     off1, len1, off2, len2 = [np.ascontiguousarray(x, np.uint64) for x in (off1, len1, off2, len2)]
     if out is None:
         out = np.empty(off1.size, np.int64)
     assert out.dtype == np.int64 and out.size == off1.size and out.flags.c_contiguous
+    if start_cells:
+        si, sj = np.empty(off1.size, np.uint64), np.empty(off1.size, np.uint64)
+        _lib.check(lib.gx_score_batch_cells(blob.ctypes.data if blob.size else None, blob.size, off1.ctypes.data,
+                                            len1.ctypes.data, off2.ctypes.data, len2.ctypes.data, off1.size,
+                                            _scores_struct(scores), int(bool(is_local)), out.ctypes.data, si.ctypes.data,
+                                            sj.ctypes.data))
+        return out, si, sj
     _lib.check(lib.gx_score_batch(blob.ctypes.data if blob.size else None, blob.size, off1.ctypes.data, len1.ctypes.data,
                                   off2.ctypes.data, len2.ctypes.data, off1.size, _scores_struct(scores), int(bool(is_local)),
                                   out.ctypes.data))

@@ -43,6 +43,8 @@ struct Ctx {
     int *lane_scores_host[NLANES] = {nullptr, nullptr, nullptr};   // pinned
     uint4 *lane_rec_host[NLANES] = {nullptr, nullptr, nullptr};    // pinned: per-pair records of the chunk in flight
     size_t lane_scores_cap = 0;
+    uint32_t *lane_cells_host[NLANES] = {nullptr, nullptr, nullptr};   // pinned: start cells (gx_score_batch_cells, local)
+    size_t lane_cells_cap = 0;
     int host_threads = 1;                             // worker threads for the host passes over a chunk
     uint8_t *ops_stage = nullptr;                     // pinned D2H staging of op lists (grown on demand)
     size_t ops_stage_cap = 0;
@@ -217,6 +219,7 @@ struct gx_plan {
     uint64_t *d_off1 = nullptr, *d_off2 = nullptr;
     uint32_t *d_len1 = nullptr, *d_len2 = nullptr;
     int *d_scores = nullptr;
+    uint32_t *d_cells = nullptr;       // local start-cell read plans: i << 16 | j per pair
     uint32_t parity = 0;
     bool uploaded = false, executed = false, colbuf_dirty = true;
     float fill_ms = 0, walk_ms = 0;
@@ -384,7 +387,7 @@ static int check_scores_impl(gx_scores sc, uint64_t m, uint64_t n, bool local) {
 static void plan_release(gx_plan *pl) {
     Ctx *c = pl->ctx;
     void *ptrs[] = {pl->d_tile_codes, pl->d_blob, pl->d_blob_sym, pl->d_lut, pl->d_stats, pl->d_timeline, pl->d_pairs, pl->d_tiles, pl->d_strips, pl->d_ctrl, pl->d_colbuf, pl->d_top, pl->d_codes, pl->d_best, pl->d_first, pl->d_masks, pl->d_carry,
-                    pl->d_results, pl->d_ops, pl->d_off1, pl->d_off2, pl->d_len1, pl->d_len2, pl->d_scores};
+                    pl->d_results, pl->d_ops, pl->d_off1, pl->d_off2, pl->d_len1, pl->d_len2, pl->d_scores, pl->d_cells};
     for (void *p : ptrs) pool_free(c, p);
 }
 
@@ -497,6 +500,7 @@ void gx_shutdown(void) {
         if (g_ctx->lane_done[k]) cudaEventDestroy(g_ctx->lane_done[k]);
         if (g_ctx->lane_scores_host[k]) cudaFreeHost(g_ctx->lane_scores_host[k]);
         if (g_ctx->lane_rec_host[k]) cudaFreeHost(g_ctx->lane_rec_host[k]);
+        if (g_ctx->lane_cells_host[k]) cudaFreeHost(g_ctx->lane_cells_host[k]);
     }
     if (g_ctx->ops_stage) cudaFreeHost(g_ctx->ops_stage);
     cudaStreamDestroy(g_ctx->stream);
@@ -599,7 +603,7 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
     pl->max_len = max_len;
     for (uint64_t q = 0; q < n_pairs; ++q) pl->cells += (len1[q] + 1) * (len2[q] + 1);
 
-    // short-read batches without traceback go to the inter-task kernel (K4)
+    // short-read batches without traceback go to the inter-task kernel (K4), local start-cell plans included
     pl->lcs = (flags & GX_FLAG_LCS_AT_MAX) != 0 && !band_col0;
     if (pl->lcs) {
         // the first-maximum keys are (V << log2 K) | k in int32 for every cell, global mode included
@@ -609,7 +613,7 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
             return n_pairs > 65536 ? GX_ERR_UNSUPPORTED : GX_ERR_RANGE;
         }
     }
-    const bool reads = !pl->lcs && !band_col0 && !pl->traceback && pl->track != 2 && n_pairs >= 1024 && max_len <= (uint64_t)READS_MAX_LEN &&
+    const bool reads = !pl->lcs && !band_col0 && !pl->traceback && n_pairs >= 1024 && max_len <= (uint64_t)READS_MAX_LEN &&
                        (!is_local || sc.s_mismatch < 0);
     pl->kind = reads ? KIND_READS : KIND_WAVEFRONT;
     int rc = GX_OK;
@@ -625,6 +629,7 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
         A(n_pairs * 4, (void **)&pl->d_len1);
         A(n_pairs * 4, (void **)&pl->d_len2);
         A(n_pairs * 4, (void **)&pl->d_scores);
+        if (pl->track == 2) A(n_pairs * 4, (void **)&pl->d_cells);
         if (rc == GX_OK) {
             std::vector<uint32_t> l1(n_pairs), l2(n_pairs);
             for (uint64_t q = 0; q < n_pairs; ++q) {
@@ -867,9 +872,10 @@ static void host_parallel(int threads, uint64_t n, F &&f) {   // f(tid, lo, hi) 
     for (auto &t : th) t.join();
 }
 
+// start_i / start_j (both or neither): also each pair's start cell -- the read kernels' for local batches, (m, n) for global.
 static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const uint64_t *off1, const uint64_t *len1,
                                 const uint64_t *off2, const uint64_t *len2, uint64_t n_pairs, gx_scores sc, int is_local,
-                                int64_t *scores, bool force32) {
+                                int64_t *scores, uint64_t *start_i, uint64_t *start_j, bool force32) {
     std::lock_guard<std::recursive_mutex> lk(g_mu);
     if (!g_ctx) return GX_ERR_NOT_INIT;
     Ctx *c = g_ctx;
@@ -895,21 +901,35 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
         }
         c->lane_scores_cap = CH;
     }
+    const bool cells = start_i && is_local;   // global start cells are (m, n): written by the host in drain()
+    if (cells && c->lane_cells_cap < CH) {
+        for (int k = 0; k < NL; ++k) {
+            if (c->lane_cells_host[k]) cudaFreeHost(c->lane_cells_host[k]);
+            c->lane_cells_host[k] = nullptr;
+            if (cudaHostAlloc((void **)&c->lane_cells_host[k], CH * sizeof(uint32_t), cudaHostAllocDefault) != cudaSuccess) {
+                cudaGetLastError();
+                c->lane_cells_cap = 0;
+                return GX_ERR_NOMEM;
+            }
+        }
+        c->lane_cells_cap = CH;
+    }
     struct Lane {
         uint8_t *blob = nullptr;
         size_t blob_cap = 0;
         uint4 *rec = nullptr;
         int *scores = nullptr;
+        uint32_t *cells = nullptr;
         uint64_t first = 0, count = 0;
         bool busy = false;
     } lane[NL];
     auto release = [&]() {
         for (auto &L : lane) {
-            void *ptrs[] = {L.blob, L.rec, L.scores};
+            void *ptrs[] = {L.blob, L.rec, L.scores, L.cells};
             for (void *p : ptrs) pool_free(c, p);
         }
     };
-    auto drain = [&](int k) -> int {   // scores of the chunk that ran on lane k -> caller's int64 array
+    auto drain = [&](int k) -> int {   // scores (and start cells) of the chunk that ran on lane k -> caller's arrays
         Lane &L = lane[k];
         if (!L.busy) return GX_OK;
         cudaError_t e = cudaEventSynchronize(c->lane_done[k]);
@@ -917,6 +937,18 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
         const int *src = c->lane_scores_host[k];
         int64_t *dst = scores + L.first;
         for (uint64_t q = 0; q < L.count; ++q) dst[q] = src[q];
+        if (cells) {
+            const uint32_t *cs = c->lane_cells_host[k];
+            for (uint64_t q = 0; q < L.count; ++q) {
+                start_i[L.first + q] = cs[q] >> 16;
+                start_j[L.first + q] = cs[q] & 0xffffu;
+            }
+        } else if (start_i) {
+            for (uint64_t q = L.first; q < L.first + L.count; ++q) {
+                start_i[q] = len1[q];
+                start_j[q] = len2[q];
+            }
+        }
         L.busy = false;
         return GX_OK;
     };
@@ -924,6 +956,7 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
         Lane &L = lane[k];
         rc = pool_alloc(c, CH * sizeof(uint4), (void **)&L.rec);
         if (!rc) rc = pool_alloc(c, CH * 4, (void **)&L.scores);
+        if (!rc && cells) rc = pool_alloc(c, CH * 4, (void **)&L.cells);
     }
     struct Part {
         uint64_t lo = UINT64_MAX, hi = 0, maxlen = 0, sum = 0, bad = 0;
@@ -1009,12 +1042,14 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
         rp.g = sc.g;
         rp.h = sc.h;
         rp.is_local = is_local ? 1 : 0;
+        rp.cells = cells ? L.cells : nullptr;
         if (launch_reads(rp, (int)maxlen, c->sm_count, st, force32) != 0) {
             rc = GX_ERR_UNSUPPORTED;
             break;
         }
         CKB(cudaGetLastError());
         CKB(cudaMemcpyAsync(c->lane_scores_host[k], L.scores, count * 4, cudaMemcpyDeviceToHost, st));
+        if (cells) CKB(cudaMemcpyAsync(c->lane_cells_host[k], L.cells, count * 4, cudaMemcpyDeviceToHost, st));
         CKB(cudaEventRecord(c->lane_done[k], st));
         L.first = first;
         L.count = count;
@@ -1225,6 +1260,7 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
         rp.g = sc.g;
         rp.h = sc.h;
         rp.is_local = pl->is_local;
+        rp.cells = pl->d_cells;
         CK(cudaEventRecord(c->ev[0], c->stream));
         int rc = launch_reads(rp, (int)pl->max_len, c->sm_count, c->stream, pl->tun.reads32 != 0, &pl->reads_bits);
         if (rc == -1) return GX_ERR_UNSUPPORTED;
@@ -1408,15 +1444,18 @@ int gx_plan_fetch(gx_plan *pl, gx_result *out, uint8_t *ops_blob, const uint64_t
     if (pl->n_pairs == 0) return GX_OK;
     if (pl->kind == KIND_READS) {
         std::vector<int> sc32(pl->n_pairs);
+        std::vector<uint32_t> cells(pl->d_cells ? pl->n_pairs : 0);
         CK(cudaMemcpyAsync(sc32.data(), pl->d_scores, pl->n_pairs * 4, cudaMemcpyDeviceToHost, c->stream));
+        if (pl->d_cells) CK(cudaMemcpyAsync(cells.data(), pl->d_cells, pl->n_pairs * 4, cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
-        pl->d2h_bytes = pl->n_pairs * 4;
+        pl->d2h_bytes = pl->n_pairs * (pl->d_cells ? 8 : 4);
         for (uint64_t q = 0; q < pl->n_pairs; ++q) {
             gx_result r;
             memset(&r, 0, sizeof r);
             r.score = sc32[q];
-            r.start_i = r.end_i = pl->len1[q];
-            r.start_j = r.end_j = pl->len2[q];
+            // start cell = end cell, as gx_walk_kernel reports it for score-only plans; (m, n) without start cells
+            r.start_i = r.end_i = pl->d_cells ? cells[q] >> 16 : pl->len1[q];
+            r.start_j = r.end_j = pl->d_cells ? cells[q] & 0xffffu : pl->len2[q];
             r.fill_ms = pl->fill_ms;
             out[q] = r;
         }
@@ -1901,7 +1940,7 @@ int gx_score_batch(const uint8_t *seq_blob, uint64_t blob_len, const uint64_t *o
     // large read sets stream through two copy/compute lanes; everything else goes through a plan
     if (!getenv("GX_NO_STREAM")) {   // debug switch, read once per batch call
         const int rcs = score_batch_streamed(seq_blob, blob_len, off1, len1, off2, len2, n_pairs, sc, is_local, scores,
-                                             getenv("GX_READS32") != nullptr);
+                                             nullptr, nullptr, getenv("GX_READS32") != nullptr);
         if (rcs != GX_ERR_UNSUPPORTED) return rcs;
     }
     std::lock_guard<std::recursive_mutex> lk(g_mu);
@@ -1913,6 +1952,39 @@ int gx_score_batch(const uint8_t *seq_blob, uint64_t blob_len, const uint64_t *o
     if (!rc) rc = gx_plan_fetch_scores(pl, scores);
     if (rc) plan_cache_drop();
     return rc;
+}
+GX_GUARD_END
+
+int gx_score_batch_cells(const uint8_t *seq_blob, uint64_t blob_len, const uint64_t *off1, const uint64_t *len1,
+                         const uint64_t *off2, const uint64_t *len2, uint64_t n_pairs, gx_scores sc, int is_local,
+                         int64_t *scores, uint64_t *start_i, uint64_t *start_j) try {
+    if ((!seq_blob && blob_len) || ((!off1 || !len1 || !off2 || !len2 || !scores || !start_i || !start_j) && n_pairs))
+        return GX_ERR_ARG;
+    if (!getenv("GX_NO_STREAM")) {
+        const int rcs = score_batch_streamed(seq_blob, blob_len, off1, len1, off2, len2, n_pairs, sc, is_local, scores,
+                                             start_i, start_j, getenv("GX_READS32") != nullptr);
+        if (rcs != GX_ERR_UNSUPPORTED) return rcs;
+    }
+    // everything the streamed path declines: a plan with start cells (read kernels when the batch qualifies, else the
+    // wavefront fill and its start-cell reduction)
+    std::lock_guard<std::recursive_mutex> lk(g_mu);
+    gx_plan *pl = nullptr;
+    int rc = cached_plan(len1, len2, n_pairs, sc, is_local, GX_FLAG_START_CELL, &pl);
+    if (rc) return rc;
+    std::vector<gx_result> res(n_pairs);
+    rc = gx_plan_upload(pl, seq_blob, blob_len, off1, off2);
+    if (!rc) rc = gx_plan_execute(pl);
+    if (!rc) rc = gx_plan_fetch(pl, res.data(), nullptr, nullptr);
+    if (rc) {
+        plan_cache_drop();
+        return rc;
+    }
+    for (uint64_t q = 0; q < n_pairs; ++q) {
+        scores[q] = res[q].score;
+        start_i[q] = res[q].start_i;
+        start_j[q] = res[q].start_j;
+    }
+    return GX_OK;
 }
 GX_GUARD_END
 

@@ -1,4 +1,4 @@
-// gx_reads.cuh -- K4: inter-task batch kernel for many short pairs (score only).
+// gx_reads.cuh -- K4: inter-task batch kernel for many short pairs (score, and on request the local start cell).
 //
 // Same recurrences as gx_fill.cuh (reference: /root/reference/src/alignment/algo.rs:191-268), but the
 // unit of parallelism is the PAIR: a group of G lanes owns one pair, each lane K register-blocked
@@ -9,6 +9,10 @@
 // never-matching character, which (for s_mismatch < 0) makes every such cell strictly smaller than a
 // real cell it derives from, so the running maximum is unaffected.  Global mode freezes a lane's
 // state outside rows 0..m-1 (two selects per cell) and reads E[m][n] from the lane that owns column n.
+//
+// TRACK (local only): also the start cell, the last cell in row-major order that attains the table maximum
+// (algo.rs:306-323), (m, n) when that maximum is 0.  By the argument above no cell outside the table can tie a
+// positive maximum, so only the zero rule needs handling.  Output: one uint32 per pair, i << 16 | j.
 #pragma once
 #include <cstdlib>
 
@@ -30,7 +34,13 @@ struct ReadsParams {
     int *scores;
     DevResult *results;   // may be null
     int a, b, g, h, is_local;
+    uint32_t *cells;      // local start cells (i << 16 | j), or null: score only
 };
+
+// start cell of a local pair from its best (V, i, j): the zero rule of gx_walk.cuh applies to an empty table too
+__device__ __forceinline__ uint32_t reads_cell(int v, uint32_t i, uint32_t j, int m, int n) {
+    return (v <= 0 || m == 0 || n == 0) ? ((uint32_t)m << 16 | (uint32_t)n) : (i << 16 | j);
+}
 
 // geometry of pair q: sequence pointers and lengths (have == false: an empty pair at the blob's start)
 __device__ __forceinline__ void reads_pair(const ReadsParams &P, uint64_t q, bool have, const uint8_t *&s1, const uint8_t *&s2, int &m,
@@ -49,8 +59,9 @@ __device__ __forceinline__ void reads_pair(const ReadsParams &P, uint64_t q, boo
     }
 }
 
-template <int G, int K, bool LOCAL>
+template <int G, int K, bool LOCAL, bool TRACK>
 __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
+    static_assert(!TRACK || (LOCAL && K <= 32), "start cells: local only, column index in 5 bits");
     constexpr unsigned FULLM = 0xffffffffu;
     constexpr int GPW = 32 / G;  // groups per warp
     const int lane = threadIdx.x & 31;
@@ -84,6 +95,7 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
 
         // local: lanes that have not reached row 0 yet must see "V = 0, I = 0" from their left neighbour
         int elast = LOCAL ? hg : 0, ilast = 0, best = 0;
+        int brow = 0;   // TRACK: best holds the key (V << 5) | k of the lane's best cell, brow its row
         int c1n = (m > 0 && lg == 0) ? (int)__ldg(s1) : -1;
         for (int t = 0; t < steps; ++t) {
             const int r = t - lg;
@@ -100,6 +112,7 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
             }
             const bool active = LOCAL ? true : (r >= 0 && r < m);  // global: state is frozen outside rows 0..m-1
             int e = el, irun = il, ed = vd;
+            int rkey = 0;   // TRACK: largest (V << 5) | k of this row: the last column that attains the row's maximum
 #pragma unroll
             for (int k = 0; k < K; ++k) {
                 const int In = LOCAL ? __viaddmax_s32_relu(irun, g, e) : __viaddmax_s32(irun, g, e);
@@ -111,7 +124,10 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
                 if (LOCAL) {
                     eu[k] = En;
                     du[k] = Dn;
-                    best = max(best, Vn);
+                    // The key cannot wrap: the score contract (check_scores_impl) refuses every local scoring with
+                    // min(m, n) * max(s_match, 0) >= 2^26, so 0 <= V < 2^26 and (V << 5) | 31 < 2^31.
+                    if (TRACK) rkey = max(rkey, Vn * 32 + k);
+                    else best = max(best, Vn);
                 } else {
                     eu[k] = active ? En : eu[k];
                     du[k] = active ? Dn : du[k];
@@ -122,9 +138,23 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
             vd = active ? el : vd;
             elast = e;
             ilast = irun;
+            if (TRACK && rkey >= (best & ~31)) {   // V of the row >= the lane's best V: later rows win ties
+                best = rkey;
+                brow = r;
+            }
         }
         int score;
-        if (LOCAL) {
+        if (TRACK) {
+            // (V, i, j) of the group's best cell: the largest 64-bit key V << 32 | i << 16 | j.  A cell outside the table
+            // (r < 0, r >= m or column >= n) may be a lane's best but never ties a positive table maximum, so it can
+            // only win the reduction when that maximum is 0, which the zero rule replaces.
+            unsigned long long key = (unsigned long long)(best >> 5) << 32 |
+                                     ((uint32_t)(brow + 1) & 0xffffu) << 16 | (uint32_t)(jl + (best & 31) + 1);
+#pragma unroll
+            for (int off = G / 2; off > 0; off >>= 1) key = max(key, __shfl_xor_sync(FULLM, key, off));
+            score = (m == 0 || n == 0) ? 0 : (int)(key >> 32);
+            if (have && lg == 0) P.cells[q] = reads_cell(score, (uint32_t)key >> 16, (uint32_t)key & 0xffffu, m, n);
+        } else if (LOCAL) {
             score = best;
 #pragma unroll
             for (int off = G / 2; off > 0; off >>= 1) score = max(score, __shfl_xor_sync(FULLM, score, off));
@@ -159,7 +189,11 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
 //     V     = max(Vhat - beta, 0)             one VIADDMNMX.S16x2.RELU
 // match/mismatch: x = c1 ^ c2 (halves 0 iff equal), ne = min_u16x2(x, 1), sub = (a+beta) - ne*(a-b)  (IMAD).
 // Needs s_mismatch < 0, s_mismatch + beta >= 0 and min(m,n)*s_match + beta < 2^15 (host checks).
-template <int G, int K>
+//
+// TRACK: no (V, k) key fits a 16-bit half, so the running maximum becomes a per-row maximum; once per step each half
+// compares it with the lane's best (Vhat frame: for V > 0, Vhat = V + beta, so ties on Vhat are ties on V), and only on
+// steps where some lane of the warp improves does it search its K columns for the last one that attains the row maximum.
+template <int G, int K, bool TRACK>
 __global__ void __launch_bounds__(256, 2) gx_reads16_kernel(const ReadsParams P) {
     constexpr unsigned FULLM = 0xffffffffu;
     constexpr int GPW = 32 / G;  // groups per warp; each group aligns 2 pairs
@@ -201,6 +235,7 @@ __global__ void __launch_bounds__(256, 2) gx_reads16_kernel(const ReadsParams P)
         for (int off = 16; off > 0; off >>= 1) steps = max(steps, __shfl_xor_sync(FULLM, steps, off));
 
         uint32_t vlast = 0u, ilast = 0u, best = 0u;
+        uint32_t brow = 0u, bcol = 0u;   // TRACK, per half: row + 1 and k + 1 of the lane's best cell
         auto row_chars = [&](int r) -> uint32_t {
             const uint32_t ca = (r >= 0 && r < ma) ? (uint32_t)__ldg(s1a + r) : 0x100u;
             const uint32_t cb = (r >= 0 && r < mb) ? (uint32_t)__ldg(s1b + r) : 0x100u;
@@ -217,6 +252,7 @@ __global__ void __launch_bounds__(256, 2) gx_reads16_kernel(const ReadsParams P)
                 il = ninf2;      // I = -inf
             }
             uint32_t v = vl, irun = il, dg = vd;
+            uint32_t rmax = 0u;   // TRACK: Vhat maximum of the row
 #pragma unroll
             for (int k = 0; k < K; ++k) {
                 const uint32_t ne = __vminu2(c1 ^ c2[k], 0x00010001u);
@@ -226,7 +262,8 @@ __global__ void __launch_bounds__(256, 2) gx_reads16_kernel(const ReadsParams P)
                 const uint32_t Sn = dg + sub;
                 const uint32_t Vh = __vimax3_s16x2(In, Dn, Sn);
                 const uint32_t Vn = __viaddmax_s16x2_relu(Vh, hg2, 0u);
-                best = __vmaxs2(best, Vh);
+                if (TRACK) rmax = (k == 0) ? Vh : __vmaxs2(rmax, Vh);
+                else best = __vmaxs2(best, Vh);
                 dg = vu[k];
                 vu[k] = Vn;
                 du[k] = Dn;
@@ -236,14 +273,59 @@ __global__ void __launch_bounds__(256, 2) gx_reads16_kernel(const ReadsParams P)
             vd = vl;
             vlast = v;
             ilast = irun;
-        }
+            if (TRACK) {
+                const uint32_t ge = __vcmpges2(rmax, best);   // 0xffff in the halves whose row reaches the lane's best
+                if (__any_sync(FULLM, ge != 0u)) {
+                    // last column of the row whose V equals the row maximum: d = rmaxV - V >= 0 in both halves (no
+                    // borrow), ne = 0 where equal; the largest (1 - ne) * (k + 1) is the last such k, plus one
+                    const uint32_t rv = __viaddmax_s16x2_relu(rmax, hg2, 0u);
+                    uint32_t col = 0u;
 #pragma unroll
-        for (int off = G / 2; off > 0; off >>= 1) best = __vmaxs2(best, __shfl_xor_sync(FULLM, best, off));
-        if (lg == 0) {
-            const int sa = max((int)(short)(best & 0xffffu) - beta, 0);
-            const int sb = max((int)(short)(best >> 16) - beta, 0);
-            if (ha) P.scores[qa] = (ma == 0 || na == 0) ? 0 : sa;
-            if (hb) P.scores[qb] = (mb == 0 || nb == 0) ? 0 : sb;
+                    for (int k = 0; k < K; ++k) {
+                        const uint32_t ne = __vminu2(rv - vu[k], 0x00010001u);
+                        col = __vmaxu2(col, (uint32_t)(k + 1) * 0x00010001u - ne * (uint32_t)(k + 1));
+                    }
+                    const uint32_t row2 = ((uint32_t)(t - lg + 1) & 0xffffu) * 0x00010001u;
+                    best = (rmax & ge) | (best & ~ge);
+                    bcol = (col & ge) | (bcol & ~ge);
+                    brow = (row2 & ge) | (brow & ~ge);
+                }
+            }
+        }
+        if constexpr (TRACK) {
+            // per half, the group's best (Vhat, i, j) as one 64-bit key (Vhat biased to unsigned); cells outside a
+            // pair's table never tie its positive maximum, and a maximum of 0 takes the zero rule (see gx_reads_kernel)
+            auto half_key = [&](int sh) -> unsigned long long {
+                const uint32_t vh = (uint32_t)((int)(short)(best >> sh) + 32768);
+                const uint32_t j = (uint32_t)jl + ((bcol >> sh) & 0xffffu);
+                return (unsigned long long)vh << 32 | ((brow >> sh) & 0xffffu) << 16 | j;
+            };
+            unsigned long long ka = half_key(0), kb = half_key(16);
+#pragma unroll
+            for (int off = G / 2; off > 0; off >>= 1) {
+                ka = max(ka, __shfl_xor_sync(FULLM, ka, off));
+                kb = max(kb, __shfl_xor_sync(FULLM, kb, off));
+            }
+            if (lg == 0) {
+                const int va = max((int)(ka >> 32) - 32768 - beta, 0), vb = max((int)(kb >> 32) - 32768 - beta, 0);
+                if (ha) {
+                    P.scores[qa] = (ma == 0 || na == 0) ? 0 : va;
+                    P.cells[qa] = reads_cell(va, (uint32_t)ka >> 16, (uint32_t)ka & 0xffffu, ma, na);
+                }
+                if (hb) {
+                    P.scores[qb] = (mb == 0 || nb == 0) ? 0 : vb;
+                    P.cells[qb] = reads_cell(vb, (uint32_t)kb >> 16, (uint32_t)kb & 0xffffu, mb, nb);
+                }
+            }
+        } else {
+#pragma unroll
+            for (int off = G / 2; off > 0; off >>= 1) best = __vmaxs2(best, __shfl_xor_sync(FULLM, best, off));
+            if (lg == 0) {
+                const int sa = max((int)(short)(best & 0xffffu) - beta, 0);
+                const int sb = max((int)(short)(best >> 16) - beta, 0);
+                if (ha) P.scores[qa] = (ma == 0 || na == 0) ? 0 : sa;
+                if (hb) P.scores[qb] = (mb == 0 || nb == 0) ? 0 : sb;
+            }
         }
     }
 }
@@ -257,7 +339,8 @@ static int launch_reads16_gk(const ReadsParams &rp, int sm_count, cudaStream_t s
     uint64_t cap = (uint64_t)sm_count * 8;
     int grid = (int)(want < cap ? want : cap);
     if (grid < 1) grid = 1;
-    gx_reads16_kernel<G, K><<<grid, threads, 0, st>>>(rp);
+    if (rp.cells) gx_reads16_kernel<G, K, true><<<grid, threads, 0, st>>>(rp);
+    else gx_reads16_kernel<G, K, false><<<grid, threads, 0, st>>>(rp);
     return 0;
 }
 
@@ -279,12 +362,14 @@ static int launch_reads_gk(const ReadsParams &rp, int sm_count, cudaStream_t st)
     uint64_t cap = (uint64_t)sm_count * 8;
     int grid = (int)(want < cap ? want : cap);
     if (grid < 1) grid = 1;
-    if (rp.is_local) gx_reads_kernel<G, K, true><<<grid, threads, 0, st>>>(rp);
-    else gx_reads_kernel<G, K, false><<<grid, threads, 0, st>>>(rp);
+    if (rp.is_local && rp.cells) gx_reads_kernel<G, K, true, true><<<grid, threads, 0, st>>>(rp);
+    else if (rp.is_local) gx_reads_kernel<G, K, true, false><<<grid, threads, 0, st>>>(rp);
+    else gx_reads_kernel<G, K, false, false><<<grid, threads, 0, st>>>(rp);
     return 0;
 }
 
-// returns -1 if max_len is not supported by this kernel family; *bits (if given) = lane width of the kernel launched
+// returns -1 if max_len is not supported by this kernel family; *bits (if given) = lane width of the kernel launched.
+// rp.cells != null (local only): the start-cell variants, which also write each pair's start cell there.
 static int launch_reads(const ReadsParams &rp, int max_len, int sm_count, cudaStream_t st, bool force32 = false, int *bits = nullptr) {
     const bool s16 = reads16_ok(rp, max_len) && !force32 && max_len <= 32 * 20;
     if (bits) *bits = s16 ? 16 : 32;

@@ -72,4 +72,9 @@ extern "C" {
         seq_blob: *const u8, blob_len: u64, off1: *const u64, len1: *const u64, off2: *const u64, len2: *const u64,
         n_pairs: u64, sc: gx_scores, is_local: c_int, scores: *mut i64,
     ) -> c_int;
+    // gx_score_batch plus each pair's start cell (local: last argmax, (m, n) when the maximum is 0; global: (m, n))
+    pub fn gx_score_batch_cells(
+        seq_blob: *const u8, blob_len: u64, off1: *const u64, len1: *const u64, off2: *const u64, len2: *const u64,
+        n_pairs: u64, sc: gx_scores, is_local: c_int, scores: *mut i64, start_i: *mut u64, start_j: *mut u64,
+    ) -> c_int;
 }

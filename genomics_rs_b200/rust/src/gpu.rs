@@ -112,3 +112,34 @@ pub fn nw_score_banded(s1: &[u8], s2: &[u8], scores: &Scores, n_bands: i32) -> R
     }
     Ok(score)
 }
+
+/// Scores and start cells of many short pairs (reads), pair p = (s1[p], s2[p]).  The start cell is where retrace would
+/// begin (algo.rs:306-323): the last cell in row-major order that attains the maximum for local mode ((m, n) when that
+/// maximum is 0), (m, n) for global mode.  -> (scores, start cells)
+pub fn score_batch_cells(pairs: &[(&[u8], &[u8])], scores: &Scores, is_local: bool) -> Result<(Vec<i64>, Vec<(usize, usize)>), String> {
+    let narrow = |v: i64| i32::try_from(v).map_err(|_| "score does not fit int32".to_string());
+    let gs = gx_scores { s_match: narrow(scores.s_match)?, s_mismatch: narrow(scores.s_mismatch)?, g: narrow(scores.g)?, h: narrow(scores.h)? };
+    let n = pairs.len();
+    let mut blob = Vec::new();
+    let (mut off1, mut len1, mut off2, mut len2) = (Vec::with_capacity(n), Vec::with_capacity(n), Vec::with_capacity(n), Vec::with_capacity(n));
+    for (a, b) in pairs {
+        off1.push(blob.len() as u64);
+        len1.push(a.len() as u64);
+        blob.extend_from_slice(a);
+        off2.push(blob.len() as u64);
+        len2.push(b.len() as u64);
+        blob.extend_from_slice(b);
+    }
+    let (mut sc, mut si, mut sj) = (vec![0i64; n], vec![0u64; n], vec![0u64; n]);
+    let rc = unsafe {
+        let rc = gx_init(-1);
+        if rc != GX_OK { rc } else {
+            gx_score_batch_cells(blob.as_ptr(), blob.len() as u64, off1.as_ptr(), len1.as_ptr(), off2.as_ptr(), len2.as_ptr(),
+                                 n as u64, gs, is_local as i32, sc.as_mut_ptr(), si.as_mut_ptr(), sj.as_mut_ptr())
+        }
+    };
+    if rc != GX_OK {
+        return Err(format!("gxalign status {rc}"));
+    }
+    Ok((sc, si.iter().zip(&sj).map(|(&i, &j)| (i as usize, j as usize)).collect()))
+}

@@ -60,7 +60,8 @@ enum {
 enum {
     GX_FLAG_TRACEBACK = 1,    /* fill direction codes and walk them (retrace, algo.rs:287-441) */
     GX_FLAG_LCS_AT_MAX = 2,   /* also return alignment_table's 2nd value (algo.rs:279-281): max_matches at the first max cell */
-    GX_FLAG_START_CELL = 4    /* score-only local: also report the start cell (last argmax, algo.rs:311-322) */
+    GX_FLAG_START_CELL = 4    /* score-only local: also report the start cell (last argmax, algo.rs:311-322); read plans
+                               * (>= 1024 pairs of <= 640 bp, s_mismatch < 0) compute it in the read kernels */
 };
 
 /* ---- AlignedSequences minus the sequence clones: algo.rs:135-146.
@@ -114,6 +115,15 @@ int gx_score_batch(const uint8_t *seq_blob, uint64_t blob_len,
                    const uint64_t *off1, const uint64_t *len1,
                    const uint64_t *off2, const uint64_t *len2, uint64_t n_pairs,
                    gx_scores sc, int is_local, int64_t *scores);
+
+/* gx_score_batch plus each pair's start cell: local = the last argmax (algo.rs:306-323), (m,n) when the maximum is 0;
+ * global = (m,n).  Same inputs, routing, checks and status codes as gx_score_batch; start_i / start_j must not be NULL
+ * when n_pairs > 0.  Read batches carry 8 bytes per pair back from the GPU (score and packed start cell). */
+int gx_score_batch_cells(const uint8_t *seq_blob, uint64_t blob_len,
+                         const uint64_t *off1, const uint64_t *len1,
+                         const uint64_t *off2, const uint64_t *len2, uint64_t n_pairs,
+                         gx_scores sc, int is_local,
+                         int64_t *scores, uint64_t *start_i, uint64_t *start_j);
 
 /* ---- the same, split into phases so that callers can keep inputs resident in HBM, overlap
  * copies, and time the kernels alone.  gx_align_batch == create + upload + execute + fetch (+ destroy, deferred).
