@@ -20,7 +20,7 @@ GX_FLAG_START_CELL = 4
 EXPORTS = [
     "gx_init", "gx_shutdown", "gx_device_count", "gx_strerror", "gx_last_error", "gx_version", "gx_check_scores",
     "gx_align_pair", "gx_align_batch", "gx_score_batch", "gx_score_batch_cells", "gx_plan_create", "gx_plan_upload", "gx_plan_execute",
-    "gx_plan_fetch", "gx_plan_fetch_scores", "gx_plan_destroy", "gx_plan_stat", "gx_plan_debug_timeline", "gx_replay_ops", "gx_k0_measure",
+    "gx_plan_fetch", "gx_plan_fetch_scores", "gx_plan_destroy", "gx_plan_stat", "gx_replay_ops", "gx_k0_measure",
     "gx_band_range", "gx_band_create", "gx_band_export", "gx_band_connect", "gx_band_upload", "gx_band_execute",
     "gx_band_score", "gx_band_stat", "gx_band_destroy", "gx_nw_score_banded", "gx_debug_planes", "gx_debug_tile_order",
 ]
@@ -87,7 +87,6 @@ def load() -> C.CDLL:
         lib.gx_plan_fetch_scores.argtypes = [vp, vp]; lib.gx_plan_fetch_scores.restype = i32
         lib.gx_plan_destroy.argtypes = [vp]; lib.gx_plan_destroy.restype = None
         lib.gx_plan_stat.argtypes = [vp, i32]; lib.gx_plan_stat.restype = C.c_double
-        lib.gx_plan_debug_timeline.argtypes = [vp, vp, u64]; lib.gx_plan_debug_timeline.restype = i32
         lib.gx_replay_ops.argtypes = [vp, u64, u64, u64, vp, vp]; lib.gx_replay_ops.restype = i32
         lib.gx_k0_measure.argtypes = [vp, i32]; lib.gx_k0_measure.restype = i32
         lib.gx_band_range.argtypes = [u64, i32, i32, C.POINTER(u64), C.POINTER(u64)]; lib.gx_band_range.restype = i32

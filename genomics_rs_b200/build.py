@@ -1,5 +1,5 @@
 """Builds libgxalign.so (C ABI + CUDA kernels, sm_100a) in-tree with nvcc.  No torch involved.
-The fill kernel is instantiated once per (K, R, CHAIN1) in its own object so that the objects compile in parallel."""
+The fill kernel is instantiated once per (K, CHAIN1) in its own object so that the objects compile in parallel."""
 from __future__ import annotations
 
 import os
@@ -9,19 +9,19 @@ from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-# A/B builds: GX_BUILD_TAG=b16 GX_BUILD_DEFS="-DGX_BMIN=16" python -m genomics_rs_b200.build  ->  libgxalign_b16.so
+# Tagged builds: GX_BUILD_TAG=chk GX_BUILD_DEFS="-DGX_CHECKED" python -m genomics_rs_b200.build  ->  libgxalign_chk.so
 TAG = os.environ.get("GX_BUILD_TAG", "")
 OBJ = os.path.join(HERE, "csrc", "_obj" + ("_" + TAG if TAG else ""))
 OUT = os.path.join(HERE, "libgxalign" + ("_" + TAG if TAG else "") + ".so")
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith(".cuh")) + [os.path.join("..", "..", "include", "gxalign.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 CFLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-Xcompiler", "-fPIC"] + os.environ.get("GX_BUILD_DEFS", "").split()
-# (K, R) register tiles of the fill kernel -- keep in step with GX_COMBOS in csrc/gx_api.cu
-COMBOS = [(4, 1), (8, 1), (16, 1)]
+# columns per lane of the fill kernel -- keep in step with GX_COMBOS in csrc/gx_api.cu
+COMBOS = [4, 8, 16]
 # (object name, source, extra flags)
 UNITS = [("gx_api.o", "gx_api.cu", []), ("gx_k0.o", "gx_k0.cu", [])] + [
-    (f"gx_fill_k{k}_r{r}_c{c}.o", "gx_fill_inst.cu", [f"-DGX_INST_K={k}", f"-DGX_INST_R={r}", f"-DGX_INST_CHAIN={c}"])
-    for k, r in COMBOS for c in (0, 1)]
+    (f"gx_fill_k{k}_c{c}.o", "gx_fill_inst.cu", [f"-DGX_INST_K={k}", f"-DGX_INST_CHAIN={c}"])
+    for k in COMBOS for c in (0, 1)]
 
 
 def _newest_header() -> float:

@@ -20,8 +20,7 @@ namespace gx {
 
 static_assert(sizeof(DevResult) == sizeof(gx_result), "DevResult must mirror gx_result");
 static_assert(sizeof(PairDesc) == 104, "PairDesc layout");
-static_assert(warp_smem_bytes(2) % 16 == 0 && warp_smem_bytes(4) % 16 == 0 && warp_smem_bytes(8) % 16 == 0 && warp_smem_bytes(16) % 16 == 0,
-              "per-warp smem must keep 16 B alignment");
+static_assert(WARP_SMEM_BYTES % 16 == 0, "per-warp smem must keep 16 B alignment");
 
 // ------------------------------------------------------------------------------------------------
 struct Block {
@@ -128,12 +127,10 @@ static void pool_free(Ctx *c, void *p) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// Debug / experiment switches (DESIGN.md 7a).  The environment is read ONCE per plan (gx_plan_create) or per streamed
-// batch call, never on the execute path; -1 = not set.
+// Test switches (DESIGN.md 7a): force a path the plan heuristics would not pick.  The environment is read ONCE per plan
+// (gx_plan_create) or per streamed batch call, never on the execute path; -1 = not set.
 struct Tunables {
-    int r = -1, batch = -1, code_band = -1, band_resident = 1;
-    int k = -1, chain1 = -1, tickets = -1, resident = -1, wpc = -1, grid_cap = -1, pad_keys = 0, poll_nap = 0, start_lead = 0,
-        fill_stats = 0, walk_stats = 0, walk_rows = 0, no_stream = 0, reads32 = 0, test_abort = 0;
+    int k = -1, chain1 = -1, tickets = -1, resident = -1, code_band = -1, walk_rows = 0, reads32 = 0, test_abort = 0;
 };
 static int env_int(const char *name, int dflt) {
     const char *e = getenv(name);
@@ -142,22 +139,11 @@ static int env_int(const char *name, int dflt) {
 static Tunables read_tunables() {
     Tunables t;
     t.k = env_int("GX_K", -1);
-    t.r = env_int("GX_R", -1);
-    t.batch = env_int("GX_BATCH", -1);
-    t.band_resident = env_int("GX_BAND_RESIDENT", 1);   // 0: resident-strips plans keep codes in every tile
     t.code_band = env_int("GX_CODE_BAND", -1);   // 0: codes in every tile; > 0: half-width of the code band in columns
     t.chain1 = env_int("GX_CHAIN1", -1);
     t.tickets = getenv("GX_TICKETS") ? 1 : -1;
     t.resident = env_int("GX_RESIDENT", -1);
-    t.wpc = env_int("GX_WPC", -1);
-    t.grid_cap = env_int("GX_GRID_CAP", -1);
-    t.pad_keys = getenv("GX_PAD_KEYS") ? 1 : 0;
-    t.poll_nap = env_int("GX_POLL_NAP", 0);
-    t.start_lead = env_int("GX_START_LEAD", 0);
-    t.fill_stats = env_int("GX_FILL_STATS", 0);
-    t.walk_stats = getenv("GX_WALK_STATS") ? 1 : 0;
     t.walk_rows = env_int("GX_WALK_ROWS", 0);          // 64..512, multiple of 64: rows of a code window of the walk
-    t.no_stream = getenv("GX_NO_STREAM") ? 1 : 0;
     t.reads32 = getenv("GX_READS32") ? 1 : 0;
     t.test_abort = getenv("GX_TEST_ABORT") ? 1 : 0;
     return t;
@@ -174,10 +160,10 @@ struct gx_plan {
     int kind = gx::KIND_WAVEFRONT;
     uint64_t n_pairs = 0;
     gx_scores sc{};
-    gx::Tunables tun;                  // debug switches as they were when the plan was created
+    gx::Tunables tun;                  // test switches as they were when the plan was created
     int is_local = 0, flags = 0;
-    int K = 8, R = 1;                  // register tile of the fill: K columns x R rows per lane per step
-    uint32_t cpb = 1;                  // code chunks per hand-off batch (batch = cpb * 64/(R*K) steps)
+    int K = 8;                         // columns per lane of the fill
+    uint32_t cpb = 1;                  // code chunks per hand-off batch (batch = cpb * 64/K steps)
     bool chain1 = false;               // latency-optimised recurrence (gx_fill.cuh, CHAIN1)
     int track = 0;
     bool traceback = false;
@@ -193,9 +179,6 @@ struct gx_plan {
     uint8_t *d_blob = nullptr;
     uint8_t *d_blob_sym = nullptr;     // blob re-encoded to symbols 0..3 when the batch uses <= 4 distinct bytes
     uint8_t *d_lut = nullptr;
-    unsigned long long *d_stats = nullptr;   // GX_FILL_STATS=1: wait/tile cycle counters of the last execute
-    unsigned long long h_stats[8] = {0};
-    unsigned long long *d_timeline = nullptr;   // GX_FILL_STATS=2: per-tile timestamps (debug)
     bool prof = false;
     gx::PairDesc *d_pairs = nullptr;
     gx::TileDesc *d_tiles = nullptr;
@@ -253,56 +236,54 @@ struct gx_band {
 
 namespace gx {
 
-// (K, R) register tiles the library is built with: K columns x R rows per lane per step (gx_fill.cuh).  R > 1 (several
-// rows per step) is supported by the kernels and was measured on every workload (profiles/r2a_sweep_kr_rowblock.jsonl):
-// the fill is bound by instructions issued per cell, which R does not lower, and the pipeline ramp of a pair grows with R
-// (31 steps of lane skew x R rows per strip), so only R = 1 is instantiated.  Add a pair here and in build.py to try one.
-#define GX_COMBOS(X) X(4, 1) X(8, 1) X(16, 1)
+// Columns per lane the library is built with (gx_fill.cuh).  A lane works on one row per step: several rows per step were
+// supported by the kernels and measured on every workload (profiles/r2a_sweep_kr_rowblock.jsonl), but the fill is bound by
+// instructions issued per cell, which they do not lower, and the pipeline ramp of a pair grows with them (31 steps of lane
+// skew x rows per step per strip).
+#define GX_COMBOS(X) X(4) X(8) X(16)
 
-// the fill kernels are instantiated in gx_fill_inst.cu, one translation unit per (K, R, CHAIN1) so that they build in parallel
-#define GX_DECL(K, R)                                                  \
-    FillKernel pick_fill_##K##_##R##_0(bool prof, bool L, bool C, int track); \
-    FillKernel pick_fill_##K##_##R##_1(bool prof, bool L, bool C, int track);
+// the fill kernels are instantiated in gx_fill_inst.cu, one translation unit per (K, CHAIN1) so that they build in parallel
+#define GX_DECL(K)                                                   \
+    FillKernel pick_fill_##K##_0(bool prof, bool L, bool C, int track); \
+    FillKernel pick_fill_##K##_1(bool prof, bool L, bool C, int track);
 GX_COMBOS(GX_DECL)
 #undef GX_DECL
 
-static bool combo_ok(int K, int R) {
-#define GX_CHK(k, r) if (K == k && R == r) return true;
+static bool combo_ok(int K) {
+#define GX_CHK(k) if (K == k) return true;
     GX_COMBOS(GX_CHK)
 #undef GX_CHK
     return false;
 }
 
-static FillKernel pick_fill(int K, int R, bool prof, bool chain1, bool L, bool C, int track) {
-#define GX_PICK(k, r) if (K == k && R == r) return chain1 ? pick_fill_##k##_##r##_1(prof, L, C, track) : pick_fill_##k##_##r##_0(prof, L, C, track);
+static FillKernel pick_fill(int K, bool prof, bool chain1, bool L, bool C, int track) {
+#define GX_PICK(k) if (K == k) return chain1 ? pick_fill_##k##_1(prof, L, C, track) : pick_fill_##k##_0(prof, L, C, track);
     GX_COMBOS(GX_PICK)
 #undef GX_PICK
     return nullptr;
 }
 
-static int launch_fill(gx_plan *pl, const FillParams &fp, int grid_cap, int track_override = -1) {
+static int launch_fill(gx_plan *pl, const FillParams &fp, int track_override = -1) {
     Ctx *c = pl->ctx;
     const int K = pl->K;
     const bool L = pl->is_local != 0, C = pl->traceback;
     const bool banded = pl->code_band && track_override < 0 && C && !L;   // two-variant kernel + per-tile flags
-    FillKernel kern = (track_override >= 0) ? pick_fill(K, pl->R, pl->prof, pl->chain1, L, false, track_override)
-                      : banded              ? pick_fill(K, pl->R, pl->prof, pl->chain1, false, true, 4)
-                                            : pick_fill(K, pl->R, pl->prof, pl->chain1, L, C, pl->track);
+    FillKernel kern = (track_override >= 0) ? pick_fill(K, pl->prof, pl->chain1, L, false, track_override)
+                      : banded              ? pick_fill(K, pl->prof, pl->chain1, false, true, 4)
+                                            : pick_fill(K, pl->prof, pl->chain1, L, C, pl->track);
     if (!kern) {
-        g_err = "no fill kernel for this (K, R)";
+        g_err = "no fill kernel for this K";
         return GX_ERR_INTERNAL;
     }
     // CTA shape: single-warp CTAs while the plan cannot fill half of the warp slots (see gx_common.cuh)
-    int wpc = (pl->n_strips * 2 >= (uint64_t)c->sm_count * warps_per_sm(K)) ? WARPS_PER_CTA : 1;
-    if (pl->tun.wpc >= 0) wpc = pl->tun.wpc == 1 ? 1 : WARPS_PER_CTA;
+    int wpc = (pl->n_strips * 2 >= (uint64_t)c->sm_count * WARPS_PER_SM) ? WARPS_PER_CTA : 1;
     if (pl->resident) wpc = 1;   // one strip per single-warp CTA, dealt round-robin over the SMs
-    const size_t smem = (size_t)wpc * warp_smem_bytes(K);
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(WARPS_PER_CTA * warp_smem_bytes(K))));
+    const size_t smem = (size_t)wpc * WARP_SMEM_BYTES;
+    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(WARPS_PER_CTA * WARP_SMEM_BYTES)));
     int occ = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, wpc * 32, smem));
     if (occ < 1) occ = 1;
-    const bool codes_kernel = C && track_override < 0;
-    occ = std::min(occ, (codes_kernel ? warps_per_sm(K) : GX_SCORE_CTAS * WARPS_PER_CTA) / wpc);
+    occ = std::min(occ, WARPS_PER_SM / wpc);
     uint64_t cap = (uint64_t)c->sm_count * occ;
     FillParams fq = fp;
     fq.tile_codes = banded ? pl->d_tile_codes : nullptr;
@@ -316,8 +297,6 @@ static int launch_fill(gx_plan *pl, const FillParams &fp, int grid_cap, int trac
         fq.n_tiles = (uint32_t)(pl->n_strips * pl->pmax);
     }
     uint64_t want = fq.pmax ? pl->n_strips : (pl->n_tiles + wpc - 1) / wpc;
-    if (pl->tun.grid_cap >= 0) grid_cap = pl->tun.grid_cap;
-    if (grid_cap > 0 && (uint64_t)grid_cap < cap) cap = grid_cap;
     int grid = (int)std::min<uint64_t>(want, cap);
     if (grid < 1) grid = 1;
     if (pl->resident) {
@@ -335,12 +314,12 @@ static int launch_fill(gx_plan *pl, const FillParams &fp, int grid_cap, int trac
 typedef void (*WalkKernel)(const WalkParams);
 static int launch_walk(gx_plan *pl, WalkParams wp) {
     WalkKernel kern = nullptr;
-#define GX_WALK(k, r) \
-    if (pl->K == k && pl->R == r) kern = gx_walk_kernel<k, r>;
+#define GX_WALK(k) \
+    if (pl->K == k) kern = gx_walk_kernel<k>;
     GX_COMBOS(GX_WALK)
 #undef GX_WALK
     if (!kern) {
-        g_err = "no walk kernel for this (K, R)";
+        g_err = "no walk kernel for this K";
         return GX_ERR_INTERNAL;
     }
     // rows of a code window: 512 lets a diagonal path cross a whole strip (32*K <= 256 columns for K <= 8) inside one window;
@@ -351,7 +330,7 @@ static int launch_walk(gx_plan *pl, WalkParams wp) {
     for (uint32_t cand : {512u, 384u, 256u, 192u, 128u, 64u}) {
         if (cand > 256u && pl->K > 8) continue;
         const uint32_t r_ = std::min(cand, row_cap);
-        const uint32_t per_sm = std::min<uint32_t>(2048u / WALK_THREADS, (227u * 1024u) / (walk_smem_bytes(pl->K, pl->R, r_) + 1024u));
+        const uint32_t per_sm = std::min<uint32_t>(2048u / WALK_THREADS, (227u * 1024u) / (walk_smem_bytes(pl->K, r_) + 1024u));
         if (pl->n_pairs <= (uint64_t)per_sm * (uint64_t)pl->ctx->sm_count) {
             rows = r_;
             break;
@@ -360,8 +339,8 @@ static int launch_walk(gx_plan *pl, WalkParams wp) {
     if (!rows) rows = pl->max_len <= 256 ? 64u : 128u;     // more pairs than fit at once: many CTAs per SM
     if (pl->tun.walk_rows >= 64 && pl->tun.walk_rows <= 512 && pl->tun.walk_rows % 64 == 0) rows = (uint32_t)pl->tun.walk_rows;
     wp.win_rows = rows;
-    const uint32_t smem = wp.traceback ? walk_smem_bytes(pl->K, pl->R, rows) : 0u;
-    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)walk_smem_bytes(pl->K, pl->R, 512u)));
+    const uint32_t smem = wp.traceback ? walk_smem_bytes(pl->K, rows) : 0u;
+    CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)walk_smem_bytes(pl->K, 512u)));
     // one CTA per pair: path warp, loader warp and two emit warps with traceback; a single warp (start cell and score only) without
     kern<<<(unsigned)pl->n_pairs, wp.traceback ? WALK_THREADS : 32, smem, pl->ctx->stream>>>(wp);
     CK(cudaGetLastError());
@@ -386,7 +365,7 @@ static int check_scores_impl(gx_scores sc, uint64_t m, uint64_t n, bool local) {
 
 static void plan_release(gx_plan *pl) {
     Ctx *c = pl->ctx;
-    void *ptrs[] = {pl->d_tile_codes, pl->d_blob, pl->d_blob_sym, pl->d_lut, pl->d_stats, pl->d_timeline, pl->d_pairs, pl->d_tiles, pl->d_strips, pl->d_ctrl, pl->d_colbuf, pl->d_top, pl->d_codes, pl->d_best, pl->d_first, pl->d_masks, pl->d_carry,
+    void *ptrs[] = {pl->d_tile_codes, pl->d_blob, pl->d_blob_sym, pl->d_lut, pl->d_pairs, pl->d_tiles, pl->d_strips, pl->d_ctrl, pl->d_colbuf, pl->d_top, pl->d_codes, pl->d_best, pl->d_first, pl->d_masks, pl->d_carry,
                     pl->d_results, pl->d_ops, pl->d_off1, pl->d_off2, pl->d_len1, pl->d_len2, pl->d_scores, pl->d_cells};
     for (void *p : ptrs) pool_free(c, p);
 }
@@ -476,7 +455,6 @@ int gx_init(int device) try {
         cudaGetDeviceCount(&ndev);
         const unsigned hw = std::thread::hardware_concurrency();
         c->host_threads = (int)std::max(1u, std::min(8u, hw / (unsigned)std::max(1, ndev)));
-        if (const char *e = getenv("GX_HOST_THREADS")) c->host_threads = std::max(1, atoi(e));
     }
     g_ctx = c;
     return GX_OK;
@@ -653,22 +631,16 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
     // ---- wavefront geometry: K columns per lane.  Larger K amortises the per-step hand-off over more cells,
     // smaller K gives more strips (warps) for batches that cannot fill the GPU otherwise.
     {
-        const uint64_t resident = (uint64_t)c->sm_count * warps_per_sm(16);   // thresholds below were tuned against 16 warps per SM
-        uint64_t strips16 = 0, strips8 = 0;
+        const uint64_t resident = (uint64_t)c->sm_count * WARPS_PER_SM;   // thresholds below were tuned against 16 warps per SM
+        uint64_t strips8 = 0;
         for (uint64_t q = 0; q < n_pairs; ++q)
-            if (len1[q] && len2[q]) {
-                strips16 += (len2[q] + 511) / 512;
-                strips8 += (len2[q] + 255) / 256;
-            }
+            if (len1[q] && len2[q]) strips8 += (len2[q] + 255) / 256;
         // measured on corona shards (tools/timeline_wl.py): 45 pairs K=16 ~ K=8; 23 pairs K=8 ~ K=4 << K=16;
         // 11 pairs K=4 6.1 ms vs K=8 8.5 ms; 6 pairs K=4 5.5 vs K=8 7.0 -- shorter strips win until the warp slots are full
         // round 2 (32-step batches in ticket mode, profiles/r2e_sweep_batch_b32.jsonl): K=8 beats K=16 wherever both fill the
         // warp slots (45 pairs 16.7 vs 17.3 ms, 1 Mbp x 1 Mbp 282 vs 340 ms), so K=16 is no longer picked by itself
-        (void)strips16;
         pl->K = (strips8 * 10 >= resident * 12 || max_len < 2048) ? 8 : 4;
-        if (combo_ok(pl->tun.k, 1)) pl->K = pl->tun.k;
-        pl->R = 1;
-        if (pl->tun.r > 0 && combo_ok(pl->K, pl->tun.r)) pl->R = pl->tun.r;
+        if (combo_ok(pl->tun.k)) pl->K = pl->tun.k;
         // latency-optimised recurrence (one more ALU op per cell, 1-op row chain) when warps are too few to hide the
         // classic 3-op chain: measured win below ~1/4 of the resident warps, loss at full occupancy
         {
@@ -686,30 +658,22 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
         const int kb = pl->K == 16 ? 4 : pl->K == 8 ? 3 : 2;
         if (pl->track == 2 && pl->chain1 && -((long long)sc.h + sc.g) >= (1ll << (31 - kb))) pl->chain1 = false;
     }
-    const int K = pl->K, R = pl->R, W = 32 * K;
+    const int K = pl->K, W = 32 * K;
     // resident-strips mode: every strip of the plan fits a warp slot of its own (single-warp CTAs, 16 per SM: the
     // launch bounds cap the registers at 128 and 16 x (per-warp shared memory + 1 KB) fits the SM for every K)
     {
         const uint64_t ns = pl->n_strips;
         // measured: 41 % of the warp slots (980 strips) 96 -> 76 ms, 60 % (6 corona pairs) 5.5 -> 4.6 ms, 83 % (1954 strips)
         // 352 -> 357 ms: with most slots busy the ticket order's interleaving of panels does as well, so stop at 70 %
-        pl->resident = ns > 0 && ns * 10 <= (uint64_t)c->sm_count * warps_per_sm(K) * 7 && pl->tun.tickets < 0;
-        if (pl->tun.resident >= 0 && ns <= (uint64_t)c->sm_count * warps_per_sm(K)) pl->resident = pl->tun.resident != 0;
+        pl->resident = ns > 0 && ns * 10 <= (uint64_t)c->sm_count * WARPS_PER_SM * 7 && pl->tun.tickets < 0;
+        if (pl->tun.resident >= 0 && ns <= (uint64_t)c->sm_count * WARPS_PER_SM) pl->resident = pl->tun.resident != 0;
     }
-    // hand-off batch length (gx_fill.cuh, Geo): 32 steps when the plan keeps every warp slot busy (ticket mode: the per-batch
-    // glue is what is left to amortise), short batches when the pipeline ramp of a pair -- strips x (31 + batch) steps --
-    // is where the time goes (resident strips).  profiles/r2e_sweep_batch_*.jsonl.
-    const uint32_t SPC = 64u / (uint32_t)(R * K), CPB_MAX = std::max(1u, 32u / (SPC * (uint32_t)R));
-    {
-        // (measured after the batch length became a run-time parameter, profiles/r2f_sweep_shards_batch.jsonl: 32 steps is
-        // also as good or better for resident strips -- BRCA2 1.08 -> 1.00 ms, one 30 kb pair 2.93 -> 2.74 ms, the 6-pair shard
-        // 4.74 -> 4.69 ms -- so every plan uses the longest batch; GX_BATCH forces another length)
-        uint32_t steps = 32u;
-        if (pl->tun.batch > 0) steps = (uint32_t)pl->tun.batch;
-        uint32_t cpb = std::max(1u, steps / SPC);
-        while (cpb & (cpb - 1)) cpb &= cpb - 1;          // power of two
-        pl->cpb = std::min(cpb, CPB_MAX);
-    }
+    // hand-off batch length (gx_fill.cuh, Geo): 32 steps, the longest the fill supports, for every plan.  Short batches
+    // shorten the pipeline ramp of a pair -- strips x (31 + batch) steps -- but measured no faster even for resident strips
+    // (profiles/r2f_sweep_shards_batch.jsonl: BRCA2 1.08 -> 1.00 ms, one 30 kb pair 2.93 -> 2.74 ms, the 6-pair shard
+    // 4.74 -> 4.69 ms at 32 steps).
+    const uint32_t SPC = 64u / (uint32_t)K;
+    pl->cpb = (uint32_t)K / 2u;                          // Geo<K>::CPB_MAX chunks = 32 steps
     const uint32_t CPB = pl->cpb, BATCH = CPB * SPC;
     pl->pairs.resize(n_pairs);
     std::vector<TileDesc> tiles;
@@ -733,7 +697,7 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
         pd.progress_off = (uint32_t)progress;
         pd.tile_base = (uint32_t)best;
         const uint32_t rows_max = (uint32_t)std::min<uint64_t>(m, PANEL_H);
-        pd.tile_code_bytes = interior ? tile_batches(rows_max, (uint32_t)R, BATCH) * CPB * 32 * 16 : 0;
+        pd.tile_code_bytes = interior ? tile_batches(rows_max, BATCH) * CPB * 32 * 16 : 0;
         pd.col0 = band_col0 ? (uint32_t)band_col0[q] : 0u;
         if (interior) {
             colbuf += (uint64_t)(pd.S - 1) * m;
@@ -802,7 +766,7 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
     // (6-pair shard, resident strips: fill 4.67 -> 4.07 ms; a single pair gains nothing -- its chain of strips runs at the
     // pace of the strips that do write codes -- and loses nothing.)
     std::vector<uint8_t> tile_codes;
-    if (pl->traceback && !is_local && !band_col0 && (!pl->resident || pl->tun.band_resident != 0) && pl->tun.code_band != 0 && best > 0) {
+    if (pl->traceback && !is_local && !band_col0 && pl->tun.code_band != 0 && best > 0) {
         tile_codes.assign(best, 1);
         double with = 0, all = 0;
         for (uint64_t q = 0; q < n_pairs; ++q) {
@@ -1296,26 +1260,7 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
     fp.blob = pl->d_blob;
     fp.blob_sym = pl->prof ? pl->d_blob_sym : nullptr;
     fp.one = 1u;
-    fp.stats = nullptr;
-    fp.timeline = nullptr;
-    fp.pad_keys = (sc.s_mismatch >= 0 || pl->tun.pad_keys) ? 1u : 0u;
-    fp.poll_nap = (uint32_t)pl->tun.poll_nap;
-    fp.start_lead = (uint32_t)pl->tun.start_lead;
-    if (pl->tun.fill_stats) {
-        if (!pl->d_stats) {
-            int rc = pool_alloc(c, 64, (void **)&pl->d_stats);
-            if (rc) return rc;
-        }
-        CK(cudaMemsetAsync(pl->d_stats, 0, 64, c->stream));
-        fp.stats = pl->d_stats;
-        if (pl->tun.fill_stats >= 2) {
-            if (!pl->d_timeline) {
-                int rc = pool_alloc(c, (std::max<uint64_t>(pl->n_tiles, pl->n_strips * pl->pmax) + 1) * 32, (void **)&pl->d_timeline);
-                if (rc) return rc;
-            }
-            fp.timeline = pl->d_timeline;
-        }
-    }
+    fp.pad_keys = sc.s_mismatch >= 0 ? 1u : 0u;
     fp.pairs = pl->d_pairs;
     fp.n_pairs = (uint32_t)pl->n_pairs;
     fp.code_bytes = pl->code_bytes;
@@ -1337,7 +1282,7 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
     fp.ap = sc.s_match - fp.hg;
     fp.bp = sc.s_mismatch - fp.hg;
     if (pl->n_tiles) {
-        int rc = launch_fill(pl, fp, 0);
+        int rc = launch_fill(pl, fp);
         if (rc) return rc;
         pl->launches++;
     }
@@ -1359,11 +1304,9 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
     wp.g = sc.g;
     wp.h = sc.h;
     wp.hg = fp.hg;
-    wp.kcols_log2 = pl->K == 16 ? 4 : pl->K == 4 ? 2 : 3;
     wp.is_local = pl->is_local;
     wp.traceback = pl->traceback ? 1 : 0;
     wp.have_best = pl->track == 2 ? 1 : 0;
-    wp.debug = pl->tun.walk_stats;
     wp.check = pl->d_ctrl + 2;
     wp.left_band = pl->d_ctrl + 3;
     wp.tile_codes = pl->code_band ? pl->d_tile_codes : nullptr;
@@ -1387,9 +1330,7 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
             fq.parity = pl->parity ^ 1u;
             fq.codes = nullptr;
             fq.tile_best = pl->d_first;
-            fq.stats = nullptr;
-            fq.timeline = nullptr;
-            int rc = launch_fill(pl, fq, 0, 3);
+            int rc = launch_fill(pl, fq, 3);
             if (rc) return rc;
             pl->launches++;
             CK(cudaMemcpyAsync(ctrl2, pl->d_ctrl + 1, 8, cudaMemcpyDeviceToHost, c->stream));
@@ -1408,7 +1349,6 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
         pl->launches++;
         CK(cudaEventRecord(c->ev[3], c->stream));
     }
-    if (fp.stats) CK(cudaMemcpyAsync(pl->h_stats, pl->d_stats, 64, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     uint32_t abort_word = ctrl_words[0];
     const uint32_t abort_word2 = ctrl2[0];
@@ -1480,10 +1420,9 @@ int gx_plan_fetch(gx_plan *pl, gx_result *out, uint8_t *ops_blob, const uint64_t
     }
     CK(cudaStreamSynchronize(c->stream));
     int rc = GX_OK;
-    const bool walk_dbg = pl->tun.walk_stats != 0;
     for (uint64_t q = 0; q < pl->n_pairs; ++q) {
-        if (!walk_dbg) out[q].fill_ms = pl->fill_ms;
-        if (!walk_dbg) out[q].walk_ms = pl->walk_ms;
+        out[q].fill_ms = pl->fill_ms;
+        out[q].walk_ms = pl->walk_ms;
         if (pl->traceback) {
             const uint64_t cap = ops_off[q + 1] - ops_off[q];
             if (out[q].n_ops > cap) {
@@ -1521,14 +1460,6 @@ int gx_plan_fetch_scores(gx_plan *pl, int64_t *scores) try {
     return GX_OK;
 }
 GX_GUARD_END
-
-int gx_plan_debug_timeline(gx_plan *pl, uint64_t *out, uint64_t cap_words) {
-    std::lock_guard<std::recursive_mutex> lk(g_mu);
-    if (!pl || !out || !pl->d_timeline || cap_words < pl->n_tiles * 4) return GX_ERR_ARG;
-    CK(cudaSetDevice(pl->ctx->device));
-    CK(cudaMemcpy(out, pl->d_timeline, pl->n_tiles * 32, cudaMemcpyDeviceToHost));
-    return GX_OK;
-}
 
 // Pure host arithmetic (no device): the ticket order plan_create would use for these pairs at register blocking K
 // (bands != 0: the pairs are consecutive column bands of one table).  out = {pair, panel, strip} triples.
@@ -1577,17 +1508,15 @@ double gx_plan_stat(const gx_plan *pl, int what) {
         case 8: return (double)pl->n_tiles;
         case 9: return (double)pl->kind;
         case 15: return (double)pl->K;
-        case 19: return (double)pl->R;
         case 20: return (double)pl->retries;
         case 23: return pl->code_cell_frac;
         case 24: return (double)pl->band_fallbacks;
-        case 22: return (double)(pl->cpb * (64u / (uint32_t)(pl->R * pl->K)));   // steps per hand-off batch
+        case 22: return (double)(pl->cpb * (64u / (uint32_t)pl->K));   // steps per hand-off batch
         case 21: return pl->resident ? 1.0 : 0.0;
         case 17: return pl->chain1 ? 1.0 : 0.0;
         case 18: return pl->lcs_ms;
         case 25: return pl->prof ? 1.0 : 0.0;
         case 26: return (double)pl->reads_bits;
-        case 10: case 11: case 12: case 13: case 14: return (double)pl->h_stats[what - 10];
         default: return -1.0;
     }
 }
@@ -1937,12 +1866,10 @@ GX_GUARD_END
 int gx_score_batch(const uint8_t *seq_blob, uint64_t blob_len, const uint64_t *off1, const uint64_t *len1, const uint64_t *off2,
                    const uint64_t *len2, uint64_t n_pairs, gx_scores sc, int is_local, int64_t *scores) try {
     if ((!seq_blob && blob_len) || ((!off1 || !len1 || !off2 || !len2 || !scores) && n_pairs)) return GX_ERR_ARG;
-    // large read sets stream through two copy/compute lanes; everything else goes through a plan
-    if (!getenv("GX_NO_STREAM")) {   // debug switch, read once per batch call
-        const int rcs = score_batch_streamed(seq_blob, blob_len, off1, len1, off2, len2, n_pairs, sc, is_local, scores,
-                                             nullptr, nullptr, getenv("GX_READS32") != nullptr);
-        if (rcs != GX_ERR_UNSUPPORTED) return rcs;
-    }
+    // large read sets stream through the copy/compute lanes; everything else goes through a plan
+    const int rcs = score_batch_streamed(seq_blob, blob_len, off1, len1, off2, len2, n_pairs, sc, is_local, scores, nullptr, nullptr,
+                                         getenv("GX_READS32") != nullptr);
+    if (rcs != GX_ERR_UNSUPPORTED) return rcs;
     std::lock_guard<std::recursive_mutex> lk(g_mu);
     gx_plan *pl = nullptr;
     int rc = cached_plan(len1, len2, n_pairs, sc, is_local, 0, &pl);
@@ -1960,11 +1887,9 @@ int gx_score_batch_cells(const uint8_t *seq_blob, uint64_t blob_len, const uint6
                          int64_t *scores, uint64_t *start_i, uint64_t *start_j) try {
     if ((!seq_blob && blob_len) || ((!off1 || !len1 || !off2 || !len2 || !scores || !start_i || !start_j) && n_pairs))
         return GX_ERR_ARG;
-    if (!getenv("GX_NO_STREAM")) {
-        const int rcs = score_batch_streamed(seq_blob, blob_len, off1, len1, off2, len2, n_pairs, sc, is_local, scores,
-                                             start_i, start_j, getenv("GX_READS32") != nullptr);
-        if (rcs != GX_ERR_UNSUPPORTED) return rcs;
-    }
+    const int rcs = score_batch_streamed(seq_blob, blob_len, off1, len1, off2, len2, n_pairs, sc, is_local, scores, start_i, start_j,
+                                         getenv("GX_READS32") != nullptr);
+    if (rcs != GX_ERR_UNSUPPORTED) return rcs;
     // everything the streamed path declines: a plan with start cells (read kernels when the batch qualifies, else the
     // wavefront fill and its start-cell reduction)
     std::lock_guard<std::recursive_mutex> lk(g_mu);

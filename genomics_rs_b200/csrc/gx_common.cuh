@@ -9,10 +9,7 @@ namespace gx {
 constexpr int NEG32 = -(1 << 30);
 
 // Rows of one panel: a tile is (panel p, strip s) = PANEL_H rows x 32*K columns, owned by one warp.
-#ifndef GX_PANEL_LOG2
-#define GX_PANEL_LOG2 12
-#endif
-constexpr int PANEL_H_LOG2 = GX_PANEL_LOG2;
+constexpr int PANEL_H_LOG2 = 12;
 constexpr int PANEL_H = 1 << PANEL_H_LOG2;
 // The fill kernel has no CTA-level cooperation (per-warp shared memory, no __syncthreads), so the same code runs as
 // 8-warp CTAs (2 per SM) or as single-warp CTAs (16 per SM).  Single-warp CTAs let the block scheduler spread a small
@@ -20,17 +17,16 @@ constexpr int PANEL_H = 1 << PANEL_H_LOG2;
 // with every warp slot busy the 8-warp shape is a few per cent faster.  gx_api.cu picks the shape per plan.
 constexpr int WARPS_PER_CTA = 8;
 constexpr int CTA_THREADS = WARPS_PER_CTA * 32;
-// 8-warp CTAs per SM: 2 (16 warps, 128 registers per thread) for every K.  Tried: 3 CTAs (24 warps, 80 registers)
-// for K <= 8 to have more warps covering the ones that wait for their left neighbour -- slower everywhere
+// 8-warp CTAs per SM: 2 (16 warps, 128 registers per thread) for every K and every instance.  Tried: 3 CTAs (24 warps,
+// 80 registers) for K <= 8 to have more warps covering the ones that wait for their left neighbour -- slower everywhere
 // (corona45 K=8 18.2 -> 20.9 ms, 1 Mbp x 1 Mbp 322 -> 373 ms): the register cap costs more than the occupancy gives.
-__host__ __device__ constexpr int ctas_per_sm(int K) { return K > 0 ? 2 : 2; }
-__host__ __device__ constexpr int warps_per_sm(int K) { return WARPS_PER_CTA * ctas_per_sm(K); }
+constexpr int CTAS_PER_SM = 2;
+constexpr int WARPS_PER_SM = WARPS_PER_CTA * CTAS_PER_SM;
 
 // per-warp shared memory: s1 panel segment (+32: 16 B alignment slack in front, 16 B over-read behind),
 // the left-boundary in-ring and right-boundary out-ring (2 x 32 rows x 8 B each) and one mbarrier.
 constexpr int WARP_SMEM_S1 = PANEL_H + 32;
 constexpr int WARP_SMEM_BYTES = WARP_SMEM_S1 + 512 + 512 + 16;
-__host__ __device__ constexpr int warp_smem_bytes(int /*K*/) { return WARP_SMEM_BYTES; }
 
 // Checked build (-DGX_CHECKED, `GX_BUILD_TAG=chk`): every shared-memory ring / staging index, code-chunk offset,
 // boundary-buffer row and op index the kernels form is range-checked on the device; a violation records its site number
@@ -112,10 +108,6 @@ struct FillParams {
     uint64_t code_bytes;             // size of `codes` (checked build)
     int4 *tile_best;
     uint32_t pad_keys;               // 1: padded columns of a pair's last strip could reach the maximum (s_mismatch >= 0): mask their keys
-    uint32_t poll_nap;               // ns a strip sleeps between two polls of its left boundary (0: poll back to back)
-    uint32_t start_lead;             // rows of extra lead a strip waits for before its first batch (slack against convoys)
-    unsigned long long *timeline;    // optional with stats: 4 words per tile (debug)
-    unsigned long long *stats;       // optional (null in production): [0] top-wait, [1] boundary-wait, [2] tile, [3] s1-wait cycles, [4] tiles
     int g, hg, ap, bp, h;            // ap = s_match - (h+g), bp = s_mismatch - (h+g): S is formed in E-space (E = V + h + g)
 };
 
@@ -129,9 +121,7 @@ struct WalkParams {
     DevResult *results;
     uint8_t *ops;
     int g, hg, h;
-    int kcols_log2;                  // log2(K) of the fill kernel that wrote the codes (informational; the walk is templated on K, R)
     int is_local, traceback, have_best;
-    int debug;                       // GX_WALK_STATS: iterations/reloads/cycles returned in spare result fields
     uint32_t *left_band;             // control block word 3: walks that needed a tile outside the code band
     const uint8_t *tile_codes;       // code band: one flag per tile, or null (every tile has codes)
     uint32_t *check;                 // checked build: where a failed bounds check records its site (control block word 2)
@@ -226,12 +216,6 @@ __device__ __forceinline__ uint2 lds_volatile_uint2(const uint2 *p) {
     uint2 v;
     asm volatile("ld.volatile.shared.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(smem_u32(p)) : "memory");
     return v;
-}
-
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
 }
 
 template <int N>

@@ -71,34 +71,25 @@ __device__ __forceinline__ void code_acc(uint32_t &cw, int S, int I, int V, uint
         : "r"(S), "r"(I), "r"(V), "r"(one), "n"(UNIT));
 }
 
-// geometry shared by fill, walk and host.  A lane owns K consecutive columns and works on R consecutive rows per
-// step (an R x K register tile); the 32 lanes of a warp run a systolic skew in units of row blocks: at step t lane l
-// updates row block t-l.  Steps are unrolled one 16-byte code chunk at a time (SPC steps = 64 cells per lane) and
-// the boundary hand-off between strips works in batches of BATCH steps = BATCH*R rows (<= 32: one row per lane).
-// A lane owns K consecutive columns and works on R consecutive rows per step (an R x K register tile); steps are unrolled
-// one 16-byte code chunk at a time (SPC steps = 64 cells per lane).  The boundary hand-off between strips works in batches
-// of `cpb` chunks = cpb*SPC steps, a RUN-TIME parameter of the plan (FillParams::cpb, 1..32/(SPC*R)): the per-batch glue
-// (publish the right boundary, settle the left one, two warp syncs) costs ~170 instructions, which 8 steps of K = 8 columns
-// cannot amortise (2.7 instructions per cell), while a strip trails its left neighbour by 31 + batch steps -- long batches
-// for plans that keep every warp slot busy, short ones where the pipeline ramp of a pair is what the time goes into
-// (profiles/r2e_sweep_batch_*.jsonl: 1 Mbp x 1 Mbp 322 -> 282 ms, 45 coronavirus pairs 17.9 -> 16.7 ms at 32 steps; one
-// BRCA2 pair 1.0 -> 1.4 ms).  At most 32 rows per batch: one boundary row per lane.
-// 8-warp CTAs per SM of the score-only instances (A/B switch: 3 = 24 warps at <= 85 registers)
-#ifndef GX_SCORE_CTAS
-#define GX_SCORE_CTAS 2
-#endif
-template <int K, int R>
+// geometry shared by fill, walk and host.  A lane owns K consecutive columns and works on one row per step; the 32 lanes
+// of a warp run a systolic skew: at step t lane l updates row t-l.  Steps are unrolled one 16-byte code chunk at a time
+// (SPC steps = 64 cells per lane).  The boundary hand-off between strips works in batches of `cpb` chunks = cpb*SPC steps,
+// a RUN-TIME parameter of the plan (FillParams::cpb, 1..CPB_MAX): the per-batch glue (publish the right boundary, settle
+// the left one, two warp syncs) costs ~170 instructions, which 8 steps of K = 8 columns cannot amortise (2.7 instructions
+// per cell), while a strip trails its left neighbour by 31 + batch steps (profiles/r2e_sweep_batch_*.jsonl: 1 Mbp x 1 Mbp
+// 322 -> 282 ms, 45 coronavirus pairs 17.9 -> 16.7 ms at 32 steps; one BRCA2 pair 1.0 -> 1.4 ms).  At most 32 rows per
+// batch: one boundary row per lane.
+template <int K>
 struct Geo {
-    static_assert(R * K <= 64 && (R & (R - 1)) == 0 && (K & (K - 1)) == 0, "R x K cells must fit one 16-byte code chunk");
+    static_assert(K >= 2 && K <= 64 && (K & (K - 1)) == 0, "K cells must fit one 16-byte code chunk");
     static constexpr int W = 32 * K;                       // columns per strip
-    static constexpr int SPC = 64 / (R * K);               // steps per 16-byte code chunk
-    static constexpr int CPB_MAX = 32 / (SPC * R) > 0 ? 32 / (SPC * R) : 1;   // chunks per batch: at most 32 rows per batch
+    static constexpr int SPC = 64 / K;                     // steps per 16-byte code chunk
+    static constexpr int CPB_MAX = K / 2;                  // chunks per batch: at most 32 rows per batch
     static constexpr int KB = Log2<K>::value;
-    static_assert(SPC * R <= 32, "one chunk must not exceed 32 rows");
 };
-// batches of one tile: row blocks (rows rounded up to R) + 31 steps of skew, in batches of `batch` steps
-__host__ __device__ __forceinline__ uint32_t tile_batches(uint32_t rows, uint32_t R, uint32_t batch) {
-    return ((rows + R - 1) / R + 31 + batch - 1) / batch;
+// batches of one tile: its rows + 31 steps of skew, in batches of `batch` steps
+__host__ __device__ __forceinline__ uint32_t tile_batches(uint32_t rows, uint32_t batch) {
+    return (rows + 31 + batch - 1) / batch;
 }
 
 // lane 0's left boundary comes from the in-ring, every other lane's from its left neighbour's registers: a predicated
@@ -127,10 +118,6 @@ __device__ __forceinline__ void lds_over_if(int &x, int &y, const uint2 *p, bool
 // (I' = max(I+g, E_left) = max(I+g, I+h+g, Mh_left) and h <= 0.)  One more ALU-pipe op per cell than the classic
 // form, a much shorter chain: chosen when there are too few strips to hide latency with warps.
 //
-// The R x K cells of a step are emitted anti-diagonal by anti-diagonal: cells of one anti-diagonal are independent,
-// so a single warp has min(R,K)-fold instruction-level parallelism and the dependent chain of a step is R+K-1 cells
-// for R rows (the step latency is what a lone strip, and the ramp of a pair's strip pipeline, run at).
-//
 // Match / mismatch score of a cell.  PROF (the batch uses at most 4 distinct symbols and the scores fit a byte): sequences
 // are staged as SHIFT AMOUNTS 8*symbol, a row's character becomes the one-hot word 1 << c1 (one SHF per row), a column's
 // four possible scores sit in the bytes of one register (prof4[k], built once per tile), and
@@ -138,20 +125,20 @@ __device__ __forceinline__ void lds_over_if(int &x, int &y, const uint2 *p, bool
 // is ONE instruction on the FMA pipe -- the add it replaces -- with no profile in shared memory (round 1 fetched a
 // profile row with K/4 LDS.128 + an address IMAD per step).  Otherwise: compare path (ISETP + SEL per cell).
 // The s1 character of the NEXT step is fetched while this one runs (`c1a` carries it from step to step, batch to batch).
-template <int K, int R, bool LOCAL, bool CODES, int TRACK, bool PROF, bool MASKED, bool PAD, bool CHAIN1, bool THRU = false>
-__device__ __forceinline__ void run_batch(int (&eu)[K], int (&du)[K], const int (&c2)[K], int (&eo)[R], int (&io)[R], int &vd,
+template <int K, bool LOCAL, bool CODES, int TRACK, bool PROF, bool MASKED, bool PAD, bool CHAIN1, bool THRU = false>
+__device__ __forceinline__ void run_batch(int (&eu)[K], int (&du)[K], const int (&c2)[K], int &eo, int &io, int &vd,
                                           int &best, int &best_r, const int g, const int hg, const int ap, const int bp,
                                           const uint32_t one, const uint8_t *s1base /* s1 row 0 of this tile */,
                                           const int (&prof4)[K] /* PROF: byte s = score of symbol s against column k */,
                                           const uint2 *inr /* left-boundary (E,I) of this batch's rows */, uint2 *outring, uint4 *code_dst,
                                           const int t0, const int rows, const int lane, const int kvalid,
-                                          int (&c1a)[R] /* s1 characters of the step about to run */, const int cpb /* chunks in this batch */,
+                                          int &c1a /* s1 character of the step about to run */, const int cpb /* chunks in this batch */,
                                           uint32_t *chk /* checked build: violation word */, const int s1lo, const int s1hi /* valid s1base indices */) {
-    using G = Geo<K, R>;
+    using G = Geo<K>;
     constexpr int KB = G::KB;
     const bool lane0 = lane == 0;
     // s1 character of tile row r; rows outside the tile are clamped only where they can occur (masked batches) --
-    // an unmasked batch looks at most R bytes past the tile's rows, which the staging buffer's slack covers
+    // an unmasked batch looks at most one byte past the tile's rows, which the staging buffer's slack covers
     auto s1char = [&](int r) __attribute__((always_inline)) -> int {
         if (MASKED) return (int)s1base[min(max(r, 0), rows - 1)];
         GX_CHECK(chk, r >= s1lo && r < s1hi, 11);
@@ -163,137 +150,103 @@ __device__ __forceinline__ void run_batch(int (&eu)[K], int (&du)[K], const int 
         // TRACK 2/3 (start cell / first maximum): the row maxima of this chunk's steps are kept in registers and folded into
         // (best, best_r) AFTER the chunk.  Updating per step put a compare + two selects on predicates between the cells of
         // consecutive steps and cost a lone strip 50 % (BRCA2 local fill 1.93 -> 1.30 ms, tools/mode_probe.py).
-        int rbk[(TRACK == 2 || TRACK == 3) ? G::SPC * R : 1];
+        int rbk[(TRACK == 2 || TRACK == 3) ? G::SPC : 1];
         static_for<G::SPC>([&](auto uc) {
             constexpr int uu = decltype(uc)::value;
             const int step = ch * G::SPC + uu;          // step inside the batch
-            const int rb = t0 + step - lane;            // row block of this lane at this step
-            const int r0 = rb * R;
-            // ---- left boundary of the R rows: neighbour lane's registers, lane 0: the in-ring
-            int el[R], il[R];
-#pragma unroll
-            for (int rr = 0; rr < R; ++rr) {
-                el[rr] = __shfl_up_sync(FULL, eo[rr], 1);
-                il[rr] = __shfl_up_sync(FULL, io[rr], 1);
-                GX_CHECK(chk, step * R + rr >= 0 && step * R + rr < 32, 12);
-#ifdef GX_LDS_SEL
-                {   // A/B: the round-1 form -- unconditional load issued independently of the shuffles, then two selects
-                    const uint2 bnd = inr[step * R + rr];
-                    el[rr] = lane0 ? (int)bnd.x : el[rr];
-                    il[rr] = lane0 ? (int)bnd.y : il[rr];
+            const int r0 = t0 + step - lane;            // row of this lane at this step
+            // ---- left boundary of the row: neighbour lane's registers, lane 0: the in-ring
+            int el = __shfl_up_sync(FULL, eo, 1);
+            int il = __shfl_up_sync(FULL, io, 1);
+            GX_CHECK(chk, step >= 0 && step < 32, 12);
+            lds_over_if(el, il, inr + step, lane0);
+            const bool act = MASKED ? ((r0 >= 0) && (r0 < rows)) : true;
+            // ---- this step's s1 character (fetched one step ago); fetch the next step's
+            const int c1 = PROF ? (int)(1u << c1a) : c1a;      // PROF: one-hot word of the symbol (shift amounts 0, 8, 16, 24)
+            c1a = s1char(r0 + 1);
+            // ---- the K cells of the row
+            int e_ = el, i_ = il, ed_ = vd;
+            int mh_ = el;   // CHAIN1: "max(D,S) of the cell to the left" -- for the lane's first column that is E_left itself
+            int rowbest = (CHAIN1 || TRACK == 3) ? INT32_MIN : -1;
+            static_for<K>([&](auto kc) {
+                constexpr int k = decltype(kc)::value;
+                int In, Dn, En, Skey, Ikey, Vkey;   // S/I/V keys: equal keys decide the direction code; Vkey orders the local maximum
+                if (CHAIN1) {
+                    In = LOCAL ? __viaddmax_s32_relu(i_, g, mh_) : __viaddmax_s32(i_, g, mh_);
+                    Dn = LOCAL ? __viaddmax_s32_relu(du[k], g, eu[k]) : __viaddmax_s32(du[k], g, eu[k]);
+                    const int Sh = PROF ? __dp4a(c1, prof4[k], ed_) : ed_ + ((c1 == c2[k]) ? ap : bp);
+                    const int Mh = __viaddmax_s32(Dn, hg, Sh);
+                    En = __viaddmax_s32(In, hg, Mh);   // local: I' >= 0 keeps E >= h+g, i.e. V >= 0
+                    if (THRU) mh_ = (k < kvalid) ? Mh : mh_;
+                    else mh_ = Mh;
+                    Skey = Sh;
+                    Ikey = CODES ? In + hg : 0;
+                    Vkey = En;     // E-space: same order, same equalities
+                } else {
+                    In = LOCAL ? __viaddmax_s32_relu(i_, g, e_) : __viaddmax_s32(i_, g, e_);
+                    Dn = LOCAL ? __viaddmax_s32_relu(du[k], g, eu[k]) : __viaddmax_s32(du[k], g, eu[k]);
+                    const int Sn = PROF ? __dp4a(c1, prof4[k], ed_) : ed_ + ((c1 == c2[k]) ? ap : bp);
+                    const int Vn = LOCAL ? __vimax3_s32_relu(In, Dn, Sn) : __vimax3_s32(In, Dn, Sn);
+                    En = Vn + hg;
+                    Skey = Sn;
+                    Ikey = In;
+                    Vkey = Vn;
                 }
-#else
-                lds_over_if(el[rr], il[rr], inr + step * R + rr, lane0);
-#endif
-            }
-            bool act[R];
-#pragma unroll
-            for (int rr = 0; rr < R; ++rr) act[rr] = MASKED ? ((r0 + rr >= 0) && (r0 + rr < rows)) : true;
-            // ---- this step's s1 characters (fetched one step ago); fetch the next step's
-            int c1[R];
-#pragma unroll
-            for (int rr = 0; rr < R; ++rr) {
-                c1[rr] = PROF ? (int)(1u << c1a[rr]) : c1a[rr];      // PROF: one-hot word of the symbol (shift amounts 0, 8, 16, 24)
-                c1a[rr] = s1char(r0 + R + rr);
-            }
-            // ---- the R x K cells, anti-diagonal by anti-diagonal
-            int e_[R], i_[R], ed_[R], mh_[R], rowbest[R];
-#pragma unroll
-            for (int rr = 0; rr < R; ++rr) {
-                e_[rr] = el[rr];
-                i_[rr] = il[rr];
-                ed_[rr] = (rr == 0) ? vd : el[rr > 0 ? rr - 1 : 0];
-                mh_[rr] = el[rr];   // CHAIN1: "max(D,S) of the cell to the left" -- for the lane's first column that is E_left itself
-                rowbest[rr] = (CHAIN1 || TRACK == 3) ? INT32_MIN : -1;
-            }
-            static_for<R + K - 1>([&](auto dc) {
-                constexpr int d = decltype(dc)::value;
-                static_for<R>([&](auto rc) {
-                    constexpr int rr = decltype(rc)::value;
-                    constexpr int k = d - rr;
-                    if constexpr (k >= 0 && k < K) {
-                        int In, Dn, En, Skey, Ikey, Vkey;   // S/I/V keys: equal keys decide the direction code; Vkey orders the local maximum
-                        if (CHAIN1) {
-                            In = LOCAL ? __viaddmax_s32_relu(i_[rr], g, mh_[rr]) : __viaddmax_s32(i_[rr], g, mh_[rr]);
-                            Dn = LOCAL ? __viaddmax_s32_relu(du[k], g, eu[k]) : __viaddmax_s32(du[k], g, eu[k]);
-                            const int Sh = PROF ? __dp4a(c1[rr], prof4[k], ed_[rr]) : ed_[rr] + ((c1[rr] == c2[k]) ? ap : bp);
-                            const int Mh = __viaddmax_s32(Dn, hg, Sh);
-                            En = __viaddmax_s32(In, hg, Mh);   // local: I' >= 0 keeps E >= h+g, i.e. V >= 0
-                            if (THRU) mh_[rr] = (k < kvalid) ? Mh : mh_[rr];
-                            else mh_[rr] = Mh;
-                            Skey = Sh;
-                            Ikey = CODES ? In + hg : 0;
-                            Vkey = En;     // E-space: same order, same equalities
-                        } else {
-                            In = LOCAL ? __viaddmax_s32_relu(i_[rr], g, e_[rr]) : __viaddmax_s32(i_[rr], g, e_[rr]);
-                            Dn = LOCAL ? __viaddmax_s32_relu(du[k], g, eu[k]) : __viaddmax_s32(du[k], g, eu[k]);
-                            const int Sn = PROF ? __dp4a(c1[rr], prof4[k], ed_[rr]) : ed_[rr] + ((c1[rr] == c2[k]) ? ap : bp);
-                            const int Vn = LOCAL ? __vimax3_s32_relu(In, Dn, Sn) : __vimax3_s32(In, Dn, Sn);
-                            En = Vn + hg;
-                            Skey = Sn;
-                            Ikey = In;
-                            Vkey = Vn;
-                        }
-                        if (CODES) {
-                            constexpr int bitpos = ((uu * R + rr) * K + k) * 2;
-                            code_acc<(1u << (bitpos & 31))>(cw[bitpos >> 5], Skey, Ikey, Vkey, one);
-                        }
-                        ed_[rr] = eu[k];
-                        if (MASKED) {
-                            eu[k] = act[rr] ? En : eu[k];
-                            du[k] = act[rr] ? Dn : du[k];
-                        } else {
-                            eu[k] = En;
-                            du[k] = Dn;
-                        }
-                        if (THRU) {
-                            e_[rr] = (k < kvalid) ? En : e_[rr];
-                            i_[rr] = (k < kvalid) ? In : i_[rr];
-                        } else {
-                            e_[rr] = En;
-                            i_[rr] = In;
-                        }
-                        if (TRACK == 2) {
-                            int key = (Vkey << KB) | k;
-                            if (PAD) key = (k < kvalid) ? key : (CHAIN1 ? INT32_MIN : -1);
-                            rowbest[rr] = max(rowbest[rr], key);
-                        } else if (TRACK == 1) {
-                            int key = Vkey;
-                            if (PAD) key = (k < kvalid) ? key : (CHAIN1 ? INT32_MIN : -1);
-                            rowbest[rr] = max(rowbest[rr], key);
-                        } else if (TRACK == 3) {
-                            // first maximum in row-major order (alignment_table's max_cell, algo.rs:258-262, strict `<`):
-                            // inside the row the key's low bits prefer the SMALLER column
-                            int key = (Vkey << KB) | (K - 1 - k);
-                            if (PAD) key = (k < kvalid) ? key : INT32_MIN;
-                            rowbest[rr] = max(rowbest[rr], key);
-                        }
-                    }
-                });
-            });
-            if (MASKED) vd = act[0] ? el[R - 1] : vd;
-            else vd = el[R - 1];
-#pragma unroll
-            for (int rr = 0; rr < R; ++rr) {
-                eo[rr] = e_[rr];
-                io[rr] = i_[rr];
-                if (TRACK == 2 || TRACK == 3) {
-                    rbk[uu * R + rr] = act[rr] ? rowbest[rr] : INT32_MIN;     // INT32_MIN: no row here
+                if (CODES) {
+                    constexpr int bitpos = (uu * K + k) * 2;
+                    code_acc<(1u << (bitpos & 31))>(cw[bitpos >> 5], Skey, Ikey, Vkey, one);
+                }
+                ed_ = eu[k];
+                if (MASKED) {
+                    eu[k] = act ? En : eu[k];
+                    du[k] = act ? Dn : du[k];
+                } else {
+                    eu[k] = En;
+                    du[k] = Dn;
+                }
+                if (THRU) {
+                    e_ = (k < kvalid) ? En : e_;
+                    i_ = (k < kvalid) ? In : i_;
+                } else {
+                    e_ = En;
+                    i_ = In;
+                }
+                if (TRACK == 2) {
+                    int key = (Vkey << KB) | k;
+                    if (PAD) key = (k < kvalid) ? key : (CHAIN1 ? INT32_MIN : -1);
+                    rowbest = max(rowbest, key);
                 } else if (TRACK == 1) {
-                    best = act[rr] ? max(best, rowbest[rr]) : best;
+                    int key = Vkey;
+                    if (PAD) key = (k < kvalid) ? key : (CHAIN1 ? INT32_MIN : -1);
+                    rowbest = max(rowbest, key);
+                } else if (TRACK == 3) {
+                    // first maximum in row-major order (alignment_table's max_cell, algo.rs:258-262, strict `<`):
+                    // inside the row the key's low bits prefer the SMALLER column
+                    int key = (Vkey << KB) | (K - 1 - k);
+                    if (PAD) key = (k < kvalid) ? key : INT32_MIN;
+                    rowbest = max(rowbest, key);
                 }
-                GX_CHECK(chk, step * R + rr < 32, 13);
-                if (lane == 31 && act[rr]) outring[step * R + rr] = make_uint2((uint32_t)e_[rr], (uint32_t)i_[rr]);   // row R*(t0+step-31)+rr
+            });
+            if (MASKED) vd = act ? el : vd;
+            else vd = el;
+            eo = e_;
+            io = i_;
+            if (TRACK == 2 || TRACK == 3) {
+                rbk[uu] = act ? rowbest : INT32_MIN;     // INT32_MIN: no row here
+            } else if (TRACK == 1) {
+                best = act ? max(best, rowbest) : best;
             }
+            GX_CHECK(chk, step < 32, 13);
+            if (lane == 31 && act) outring[step] = make_uint2((uint32_t)e_, (uint32_t)i_);   // row t0+step-31
         });
         if (TRACK == 2 || TRACK == 3) {
             // TRACK 2: the LAST maximum in row-major order wins (Iterator::max_by, algo.rs:311-322): a later row replaces an
             // equal value; inside the row the key's low bits prefer the larger column.  TRACK 3: the FIRST maximum
             // (alignment_table's max_cell, algo.rs:258-262): only a strictly larger value replaces (rows arrive in
             // increasing order).  A slot without a row (INT32_MIN) never replaces anything.
-            const int rbase = (t0 + ch * G::SPC - lane) * R;
+            const int rbase = t0 + ch * G::SPC - lane;
 #pragma unroll
-            for (int x = 0; x < G::SPC * R; ++x) {
+            for (int x = 0; x < G::SPC; ++x) {
                 const bool upd = (TRACK == 2) ? ((rbk[x] | (K - 1)) >= best && rbk[x] != INT32_MIN) : ((rbk[x] | (K - 1)) > (best | (K - 1)));
                 best = upd ? rbk[x] : best;
                 best_r = upd ? rbase + x : best_r;
@@ -307,25 +260,24 @@ __device__ __forceinline__ void run_batch(int (&eu)[K], int (&du)[K], const int 
 // tile's batch loops and picks one per tile (FillParams::tile_codes).  The choice is made once per tile, around two complete
 // copies of the loops: dispatching per batch inside shared loops slowed a resident strip's traceback variant by 8-40 %
 // (BRCA2 fill 0.99 -> 1.41 ms) even when the other variant never ran.
-template <int K, int R, bool LOCAL, bool CODES, int TRACK, bool PROF, bool CHAIN1, bool BAND = false>
-__global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE_CTAS) gx_fill_kernel(const FillParams P) {
-    using G = Geo<K, R>;
+template <int K, bool LOCAL, bool CODES, int TRACK, bool PROF, bool CHAIN1, bool BAND = false>
+__global__ void __launch_bounds__(CTA_THREADS, CTAS_PER_SM) gx_fill_kernel(const FillParams P) {
+    using G = Geo<K>;
     constexpr int W = G::W;
     const int cpb = (int)P.cpb;          // code chunks per hand-off batch (run-time: see Geo)
-    const int B = cpb * G::SPC;          // steps per batch
-    const int BR = B * R;                // rows per batch (<= 32)
+    const int B = cpb * G::SPC;          // steps (= rows) per batch, <= 32
     constexpr int KB = G::KB;
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31;
     const int wib = threadIdx.x >> 5;
-    uint8_t *wsm = smem + wib * warp_smem_bytes(K);
+    uint8_t *wsm = smem + wib * WARP_SMEM_BYTES;
     uint8_t *s1buf = wsm;
-    uint2 *inring = reinterpret_cast<uint2 *>(wsm + WARP_SMEM_S1);   // 2 x BR entries (double-buffered by batch)
+    uint2 *inring = reinterpret_cast<uint2 *>(wsm + WARP_SMEM_S1);   // 2 x B entries (double-buffered by batch)
     uint2 *outring = inring + 64;
     uint64_t *mbar = reinterpret_cast<uint64_t *>(outring + 64);
     static_assert(WARP_SMEM_S1 + 2 * 64 * 8 + 16 == WARP_SMEM_BYTES, "per-warp shared-memory layout");
 
-    // the s1 staging buffer starts out as valid symbols: unmasked batches prefetch up to 2R bytes past the rows the
+    // the s1 staging buffer starts out as valid symbols: unmasked batches prefetch up to 2 bytes past the rows the
     // TMA copy delivered (stale bytes of an earlier tile, or these zeros -- any symbol 0..3 indexes a real profile row)
     for (int x = lane; x < WARP_SMEM_S1 / 16; x += 32) reinterpret_cast<uint4 *>(s1buf)[x] = make_uint4(0u, 0u, 0u, 0u);
     if (lane == 0) {
@@ -368,10 +320,6 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
         const TileDesc td = P.tiles[tk];
         if (td.pair == 0xffffffffu) break;      // padding: this strip has fewer panels
         GX_CHECK(chk, td.pair < P.n_pairs, 1);
-        const long long st_t0 = P.stats ? clock64() : 0;
-        const unsigned long long tl_take = P.stats ? globaltimer_ns() : 0ull;
-        unsigned long long tl_dp0 = 0ull;
-        long long st_top = 0, st_bnd = 0, st_s1 = 0;
         const PairDesc *pd = P.pairs + td.pair;
         const int m = (int)pd->m, n = (int)pd->n, S = (int)pd->S;
         const int p = (int)td.p, s = (int)td.s;
@@ -382,7 +330,7 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
         const bool has_pad = (s + 1) * W > n;
         const int col0 = (int)pd->col0;
         GX_CHECK(chk, p >= 0 && p < (int)pd->P && s >= 0 && s < S && rows > 0 && rows <= PANEL_H, 2);
-        GX_CHECK(chk, BR >= 1 && BR <= 32 && cpb >= 1 && cpb <= G::CPB_MAX, 3);
+        GX_CHECK(chk, B >= 1 && B <= 32 && cpb >= 1 && cpb <= G::CPB_MAX, 3);
 
         // ---- stage s1[i0 .. i0+rows) with a TMA bulk copy (16-byte aligned window around it)
         const uint8_t *s1g = seq + pd->s1_off + i0;
@@ -425,7 +373,6 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
             // the previous panel of this strip must be complete (its `top` rows written)
             const uint32_t *pr = P.progress + pd->progress_off + s;
             uint32_t spins = 0;
-            const long long w0 = P.stats ? clock64() : 0;
             // poll with relaxed loads and a growing sleep (an acquire load is LDG + CCTL.IVALL: hundreds of waiting
             // warps invalidating their SM's L1 every microsecond slow the warps that do the work), acquire once at the end
             uint32_t nap = 100;
@@ -438,7 +385,6 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
                 nap = min(nap * 2u, 1000u);
             }
             (void)ld_acquire_u32(pr);
-            if (P.stats) st_top += clock64() - w0;
             if (dead) break;
             const int2 *tp = P.top + pd->top_off + jl;
 #pragma unroll
@@ -494,11 +440,9 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
         dead = __any_sync(FULL, dead);
         if (dead) break;
 
-        int eo[R], io[R];   // this lane's right edge (E, I) of the R rows of its last step: what the next lane shuffles in
-#pragma unroll
-        for (int rr = 0; rr < R; ++rr) eo[rr] = io[rr] = 0;
+        int eo = 0, io = 0;   // this lane's right edge (E, I) of the row of its last step: what the next lane shuffles in
         int best = (CHAIN1 || TRACK == 3) ? INT32_MIN : -1, best_r = 0;
-        const uint32_t nbat = tile_batches((uint32_t)rows, R, B);
+        const uint32_t nbat = tile_batches((uint32_t)rows, B);
         uint4 *code_base = nullptr;
         if (CODES)
             code_base = reinterpret_cast<uint4 *>(P.codes + pd->codes_off + (uint64_t)(p * S + s) * pd->tile_code_bytes) + lane;
@@ -506,35 +450,18 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
         bool tcodes = CODES;
         if constexpr (BAND) tcodes = P.tile_codes[pd->tile_base + p * S + s] != 0;
 
-        // ---- left boundary prefetch (LL protocol): lanes 0..BR-1 fetch the entries of local rows BR*bt + lane
+        // ---- left boundary prefetch (LL protocol): lanes 0..B-1 fetch the entries of local rows B*bt + lane
         unsigned long long nxt = 0;
         auto issue = [&](uint32_t bt) __attribute__((always_inline)) {
-            const int r = (int)(BR * bt) + lane;
-            GX_CHECK(chk, !(has_left && lane < BR && r < rows) || (i0 + r >= 0 && i0 + r < m), 4);
-            if (has_left && lane < BR && r < rows) nxt = ld_bnd(cb_in + r);
+            const int r = (int)(B * bt) + lane;
+            GX_CHECK(chk, !(has_left && lane < B && r < rows) || (i0 + r >= 0 && i0 + r < m), 4);
+            if (has_left && lane < B && r < rows) nxt = ld_bnd(cb_in + r);
         };
-        if (has_left && P.start_lead > 0) {
-            // slack: do not start before the left neighbour is start_lead rows into this panel
-            const int lead = min((int)P.start_lead, rows - 1);
-            uint32_t spins = 0;
-            const long long w0 = P.stats ? clock64() : 0;
-            while ((((uint32_t)(ld_bnd(cb_in + lead) >> 32)) & 1u) != parity) {
-                if (spin_check(spins, abort_word)) {
-                    dead = true;
-                    break;
-                }
-                __nanosleep(500);
-            }
-            if (P.stats) st_bnd += clock64() - w0;
-            dead = __any_sync(FULL, dead);
-            if (dead) break;
-        }
         issue(0);
 
         // wait for the s1 segment
         {
             uint32_t tries = 0;
-            const long long w0 = P.stats ? clock64() : 0;
             while (!mbar_try_wait(mbar, phase)) {
                 if (++tries > (1u << 24)) {
                     atomicExch(abort_word, 1u);
@@ -543,30 +470,26 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
                 }
             }
             dead = __any_sync(FULL, dead);
-            if (P.stats) st_s1 += clock64() - w0;
             if (dead) break;
         }
         phase ^= 1u;
         const uint8_t *s1base = s1buf + delta;
         __syncwarp();
-        // the s1 characters of step 0 (run_batch fetches one step ahead)
-        int c1a[R];
-#pragma unroll
-        for (int rr = 0; rr < R; ++rr) c1a[rr] = s1base[min(max(-lane * R + rr, 0), rows - 1)];
+        // the s1 character of step 0 (run_batch fetches one step ahead)
+        int c1a = s1base[min(max(-lane, 0), rows - 1)];
 
         // ---- batch loop.  The hand-off rings are double-buffered (the global load of batch bt+2's left boundary is in
         //      flight while batch bt computes), and every batch ends with: publish its finished right-boundary rows,
         //      then settle the in-ring of the next batch (post() below).
         // settle(b): lanes 0..B-1 turn the prefetched word of local row B*b+lane into an in-ring entry.
         // The common case (data already there) is branch-free apart from one vote.
-        const bool lane_b = lane < BR;
+        const bool lane_b = lane < B;
         auto settle = [&](uint32_t b) __attribute__((always_inline)) -> bool {
-            const int rb = (int)(BR * b) + lane;
+            const int rb = (int)(B * b) + lane;
             const bool need = has_left && lane_b && (rb < rows);
             bool ok = !need || ((((uint32_t)(nxt >> 32)) & 1u) == parity);
             if (!__all_sync(FULL, ok)) {
                 uint32_t spins = 0;
-                const long long w0 = P.stats ? clock64() : 0;
                 bool lost = false;
                 do {
                     if (__any_sync(FULL, spin_check(spins, abort_word))) {
@@ -576,24 +499,21 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
                     // not there yet: poll again at once.  The L2 round trip (~500 clk) paces the loop, a polling warp
                     // issues ~3 % of its scheduler's slots, and every nap here would be added to the lag of this strip
                     // behind its left neighbour -- strips x lag is the pipeline ramp of a pair.
-                    if (P.poll_nap) __nanosleep(P.poll_nap);
                     if (!ok) nxt = ld_bnd(cb_in + rb);
                     ok = !need || ((((uint32_t)(nxt >> 32)) & 1u) == parity);
                 } while (!__all_sync(FULL, ok));
-                if (P.stats) st_bnd += clock64() - w0;
                 if (lost) return false;
             }
             uint2 cur;
             cur.x = has_left ? (uint32_t)nxt : (uint32_t)((LOCAL ? 0 : h + (i0 + rb + 1) * g) + hg);  // algo.rs:204-211: V = delete_score
             cur.y = has_left ? (uint32_t)(((int)(uint32_t)(nxt >> 32)) >> 1) : (uint32_t)NEG32;
-            GX_CHECK(chk, !lane_b || (b & 1u) * BR + lane < 64, 5);
-            if (lane_b) inring[(b & 1u) * BR + lane] = cur;
+            GX_CHECK(chk, !lane_b || (b & 1u) * B + lane < 64, 5);
+            if (lane_b) inring[(b & 1u) * B + lane] = cur;
             return true;
         };
         if (!settle(0)) dead = true;
         if (nbat > 1) issue(1);
         __syncwarp();
-        if (P.stats) tl_dp0 = globaltimer_ns();
         uint2 pub = make_uint2(0u, 0u);   // out-ring entry read back after the previous batch
         int pub_row = -1;
         auto flush_pub = [&]() __attribute__((always_inline)) {
@@ -610,8 +530,8 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
         // and the rows finished in batch bt are published before anything else can block.
         const bool has_out = cb_out != nullptr;
         auto post = [&](uint32_t bt, uint2 *outr) __attribute__((always_inline)) -> bool {
-            // rows lane 31 finished in this batch: row blocks t0-31 .. t0+B-32
-            const int ro = ((int)(B * bt) - 31) * R + lane;
+            // rows lane 31 finished in this batch: rows t0-31 .. t0+B-32
+            const int ro = (int)(B * bt) - 31 + lane;
             const bool take = has_out && lane_b && ro >= 0 && ro < rows;
             __syncwarp();                                    // out-ring stores of this batch -> visible
             if (take) pub = lds_volatile_uint2(outr + lane);
@@ -628,7 +548,7 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
         // batches [0, nb_head) and [nb_body, nbat) touch rows outside the tile (skew) and run the masked steps;
         // the body runs unmasked steps with straight-line glue.
         const uint32_t nb_head = (30 + B) / B;                              // first batch with t0 >= 31
-        const uint32_t nb_body = max(nb_head, ((uint32_t)rows / R) / B);    // first batch that reaches past the last full row block
+        const uint32_t nb_body = max(nb_head, (uint32_t)rows / B);          // first batch that reaches past the last row
         bool thru = false;
         if constexpr (!LOCAL && !CODES && TRACK == 0) thru = right_band && has_pad;
         // phase 0: masked head batches (all batches of a THRU tile), then the unmasked body; phase 1: masked tail.
@@ -643,19 +563,19 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
             for (int ph = 0; ph < 2 && !dead; ++ph) {
                 const uint32_t m_end = (ph == 0 && !thru) ? min(nb_head, nbat) : nbat;
                 for (; bt < m_end && !dead; ++bt) {
-                    uint2 *outr = outring + (bt & 1u) * BR;
+                    uint2 *outr = outring + (bt & 1u) * B;
                     uint4 *cdst = WC ? code_base + (size_t)bt * cpb * 32 : nullptr;
                     GX_CHECK(chk, !WC || ((size_t)(bt + 1) * cpb * 512 <= pd->tile_code_bytes &&
                                           pd->codes_off + (uint64_t)(p * S + s + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
                     if constexpr (!LOCAL && !CODES && TRACK == 0) {
                         if (thru)
-                            run_batch<K, R, LOCAL, WC, TRACK, PROF, true, false, CHAIN1, true>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
-                                                                                            one, s1base, prof4, inring + (bt & 1u) * BR, outr, cdst,
+                            run_batch<K, LOCAL, WC, TRACK, PROF, true, false, CHAIN1, true>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
+                                                                                            one, s1base, prof4, inring + (bt & 1u) * B, outr, cdst,
                                                                                             (int)(B * bt), rows, lane, kvalid, c1a, cpb, chk, -(int)delta, WARP_SMEM_S1 - (int)delta);
                     }
                     if (!thru)
-                        run_batch<K, R, LOCAL, WC, TRACK, PROF, true, (TRACK != 0), CHAIN1>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
-                                                                                         one, s1base, prof4, inring + (bt & 1u) * BR, outr, cdst,
+                        run_batch<K, LOCAL, WC, TRACK, PROF, true, (TRACK != 0), CHAIN1>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
+                                                                                         one, s1base, prof4, inring + (bt & 1u) * B, outr, cdst,
                                                                                          (int)(B * bt), rows, lane, kvalid, c1a, cpb, chk, -(int)delta, WARP_SMEM_S1 - (int)delta);
                     if (!post(bt, outr)) dead = true;
                 }
@@ -665,23 +585,23 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
                 // cell it derives from, so the plain body is exact -- the tile reductions ignore winners with j > n.
                 if ((TRACK != 0) && has_pad && P.pad_keys != 0u) {
                     for (; bt < nb_body && !dead; ++bt) {
-                        uint2 *outr = outring + (bt & 1u) * BR;
+                        uint2 *outr = outring + (bt & 1u) * B;
                         uint4 *cdst = WC ? code_base + (size_t)bt * cpb * 32 : nullptr;
                         GX_CHECK(chk, !WC || ((size_t)(bt + 1) * cpb * 512 <= pd->tile_code_bytes &&
                                               pd->codes_off + (uint64_t)(p * S + s + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
-                        run_batch<K, R, LOCAL, WC, TRACK, PROF, false, true, CHAIN1>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
-                                                                                  one, s1base, prof4, inring + (bt & 1u) * BR, outr, cdst,
+                        run_batch<K, LOCAL, WC, TRACK, PROF, false, true, CHAIN1>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
+                                                                                  one, s1base, prof4, inring + (bt & 1u) * B, outr, cdst,
                                                                                   (int)(B * bt), rows, lane, kvalid, c1a, cpb, chk, -(int)delta, WARP_SMEM_S1 - (int)delta);
                         if (!post(bt, outr)) dead = true;
                     }
                 } else {
                     for (; bt < nb_body && !dead; ++bt) {
-                        uint2 *outr = outring + (bt & 1u) * BR;
+                        uint2 *outr = outring + (bt & 1u) * B;
                         uint4 *cdst = WC ? code_base + (size_t)bt * cpb * 32 : nullptr;
                         GX_CHECK(chk, !WC || ((size_t)(bt + 1) * cpb * 512 <= pd->tile_code_bytes &&
                                               pd->codes_off + (uint64_t)(p * S + s + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
-                        run_batch<K, R, LOCAL, WC, TRACK, PROF, false, false, CHAIN1>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
-                                                                                   one, s1base, prof4, inring + (bt & 1u) * BR, outr, cdst,
+                        run_batch<K, LOCAL, WC, TRACK, PROF, false, false, CHAIN1>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
+                                                                                   one, s1base, prof4, inring + (bt & 1u) * B, outr, cdst,
                                                                                    (int)(B * bt), rows, lane, kvalid, c1a, cpb, chk, -(int)delta, WARP_SMEM_S1 - (int)delta);
                         if (!post(bt, outr)) dead = true;
                     }
@@ -739,22 +659,6 @@ __global__ void __launch_bounds__(CTA_THREADS, CODES ? ctas_per_sm(K) : GX_SCORE
                 bj = take ? oj : bj;
             }
             if (lane == 0) P.tile_best[pd->tile_base + p * S + s] = make_int4(bv, bi, bj, 0);
-        }
-        if (P.stats && lane == 0) {
-            atomicAdd(P.stats + 0, (unsigned long long)st_top);
-            atomicAdd(P.stats + 1, (unsigned long long)st_bnd);
-            atomicAdd(P.stats + 2, (unsigned long long)(clock64() - st_t0));
-            atomicAdd(P.stats + 3, (unsigned long long)st_s1);
-            atomicAdd(P.stats + 4, 1ull);
-            if (P.timeline) {   // per tile: ticket taken, first DP step, end (ns), pair/p/s and SM
-                unsigned long long *tl = P.timeline + 4ull * tk;
-                uint32_t smid;
-                asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-                tl[0] = tl_take;
-                tl[1] = tl_dp0;
-                tl[2] = globaltimer_ns();
-                tl[3] = ((unsigned long long)td.pair << 48) | ((unsigned long long)p << 32) | ((unsigned long long)s << 12) | smid;
-            }
         }
     }
 }

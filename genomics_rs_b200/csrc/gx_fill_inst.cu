@@ -1,9 +1,9 @@
-// gx_fill_inst.cu -- instantiates gx_fill_kernel for one (K, R, CHAIN1) combination: compiled once per combination
-// with -DGX_INST_K=4|8|16 -DGX_INST_R=1|2|4|8 -DGX_INST_CHAIN=0|1 (genomics_rs_b200/build.py builds the objects in parallel).
+// gx_fill_inst.cu -- instantiates gx_fill_kernel for one (K, CHAIN1) combination: compiled once per combination
+// with -DGX_INST_K=4|8|16 -DGX_INST_CHAIN=0|1 (genomics_rs_b200/build.py builds the objects in parallel).
 #include "gx_fill.cuh"
 
-#if !defined(GX_INST_K) || !defined(GX_INST_R) || !defined(GX_INST_CHAIN)
-#error "compile with -DGX_INST_K=4|8|16 -DGX_INST_R=1|2|4|8 -DGX_INST_CHAIN=0|1"
+#if !defined(GX_INST_K) || !defined(GX_INST_CHAIN)
+#error "compile with -DGX_INST_K=4|8|16 -DGX_INST_CHAIN=0|1"
 #endif
 
 namespace gx {
@@ -13,23 +13,22 @@ typedef void (*FillKernel)(const FillParams);
 template <bool PROF>
 static FillKernel pick_mode(bool L, bool C, int track) {
     constexpr int K = GX_INST_K;
-    constexpr int R = GX_INST_R;
     constexpr bool CH = GX_INST_CHAIN != 0;
-    if (track == 4) return gx_fill_kernel<K, R, false, true, 0, PROF, CH, true>;   // global traceback with a code band
+    if (track == 4) return gx_fill_kernel<K, false, true, 0, PROF, CH, true>;   // global traceback with a code band
     if (track == 3) {   // first-maximum pass of GX_FLAG_LCS_AT_MAX: score only
-        if (L) return gx_fill_kernel<K, R, true, false, 3, PROF, CH>;
-        return gx_fill_kernel<K, R, false, false, 3, PROF, CH>;
+        if (L) return gx_fill_kernel<K, true, false, 3, PROF, CH>;
+        return gx_fill_kernel<K, false, false, 3, PROF, CH>;
     }
-    if (!L && !C) return gx_fill_kernel<K, R, false, false, 0, PROF, CH>;
-    if (!L && C) return gx_fill_kernel<K, R, false, true, 0, PROF, CH>;
-    if (L && !C && track == 1) return gx_fill_kernel<K, R, true, false, 1, PROF, CH>;
-    if (L && !C) return gx_fill_kernel<K, R, true, false, 2, PROF, CH>;
-    return gx_fill_kernel<K, R, true, true, 2, PROF, CH>;
+    if (!L && !C) return gx_fill_kernel<K, false, false, 0, PROF, CH>;
+    if (!L && C) return gx_fill_kernel<K, false, true, 0, PROF, CH>;
+    if (L && !C && track == 1) return gx_fill_kernel<K, true, false, 1, PROF, CH>;
+    if (L && !C) return gx_fill_kernel<K, true, false, 2, PROF, CH>;
+    return gx_fill_kernel<K, true, true, 2, PROF, CH>;
 }
 
-#define GX_CAT_(a, b, c, d, e, f) a##b##c##d##e##f
-#define GX_CAT(a, b, c, d, e, f) GX_CAT_(a, b, c, d, e, f)
-FillKernel GX_CAT(pick_fill_, GX_INST_K, _, GX_INST_R, _, GX_INST_CHAIN)(bool prof, bool L, bool C, int track) {
+#define GX_CAT_(a, b, c, d) a##b##c##d
+#define GX_CAT(a, b, c, d) GX_CAT_(a, b, c, d)
+FillKernel GX_CAT(pick_fill_, GX_INST_K, _, GX_INST_CHAIN)(bool prof, bool L, bool C, int track) {
     return prof ? pick_mode<true>(L, C, track) : pick_mode<false>(L, C, track);
 }
 

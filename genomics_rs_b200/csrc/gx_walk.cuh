@@ -28,20 +28,20 @@
 namespace gx {
 
 // dynamic shared memory of one walk CTA: a 2 KB control block (descriptor ring, request ring, tails, ready words, partial
-// results, debug counters) and three code-window buffers.
-// A window is `rows` rows of one strip = rows/R (+1) row blocks + 31 steps of lane skew, 64/(R*K) steps per code chunk.
-__host__ __device__ constexpr uint32_t walk_chunks(int K, int R, uint32_t rows) {
-    return (uint32_t)((rows / R + 1 + 31 + 64 / (R * K) - 1) / (64 / (R * K)) + 1);
+// results) and three code-window buffers.
+// A window is `rows` rows of one strip = rows (+1) steps + 31 steps of lane skew, 64/K steps per code chunk.
+__host__ __device__ constexpr uint32_t walk_chunks(int K, uint32_t rows) {
+    return (uint32_t)((rows + 1 + 31 + 64 / K - 1) / (64 / K) + 1);
 }
-__host__ __device__ constexpr uint32_t walk_buf_bytes(int K, int R, uint32_t rows) { return walk_chunks(K, R, rows) * 32 * 16; }
+__host__ __device__ constexpr uint32_t walk_buf_bytes(int K, uint32_t rows) { return walk_chunks(K, rows) * 32 * 16; }
 constexpr uint32_t WALK_CTRL_BYTES = 2048;
 constexpr uint32_t WALK_RING = 64;          // run descriptors in flight between the path warp and the emit warps
 constexpr uint32_t WALK_REQ = 8;            // window requests in flight between the path warp and the loader warp (<= 3 used)
 constexpr uint32_t WALK_NBUF = 3;           // window buffers: the current one and two prefetch targets
 constexpr uint32_t WALK_EMIT = 2;            // emit warps (<= 4: their tails are read with one 16-byte load)
 constexpr uint32_t WALK_THREADS = 64 + 32 * WALK_EMIT;   // path warp, emit warp 0, loader warp, emit warps 1..
-__host__ __device__ constexpr uint32_t walk_smem_bytes(int K, int R, uint32_t rows) {
-    return WALK_CTRL_BYTES + WALK_NBUF * walk_buf_bytes(K, R, rows);
+__host__ __device__ constexpr uint32_t walk_smem_bytes(int K, uint32_t rows) {
+    return WALK_CTRL_BYTES + WALK_NBUF * walk_buf_bytes(K, rows);
 }
 static_assert(PANEL_H_LOG2 <= 12, "window requests carry panel rows in 12 bits");
 
@@ -68,7 +68,7 @@ __device__ __forceinline__ uint32_t lds_code_word(uint32_t addr) {
     return v;
 }
 
-template <int K, int R>
+template <int K>
 __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams P) {
     const uint32_t q = blockIdx.x;
     if (q >= P.n_pairs) return;
@@ -158,10 +158,10 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
         return;
     }
 
-    using G = Geo<K, R>;
+    using G = Geo<K>;
     constexpr uint32_t SPC = G::SPC;
     const uint32_t WR = P.win_rows;                          // rows per window (64..512, chosen per launch); a window spans the strip's width
-    const uint32_t BUF_BYTES = walk_buf_bytes(K, R, WR);
+    const uint32_t BUF_BYTES = walk_buf_bytes(K, WR);
     extern __shared__ __align__(16) uint8_t walk_smem[];
     // descriptor ring, LL style: {i | tag, j, direction | previous direction << 2 | run << 4 | tag, ops emitted before}.  The path warp
     // writes a descriptor with ONE 16-byte shared-memory store and the emit warp it belongs to (sequence number mod WALK_EMIT) polls
@@ -172,12 +172,11 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
     uint32_t *tail = reinterpret_cast<uint32_t *>(walk_smem + WALK_RING * 16 + WALK_REQ * 16);
     uint32_t *ready = tail + 4;                                                        // per buffer: last request finished | no-codes << 31
     uint32_t *part = tail + 8;                                                         // per emit warp: 8 words of partial results
-    unsigned long long *dbg = reinterpret_cast<unsigned long long *>(tail + 8 + 8 * WALK_EMIT);
     uint32_t *scratch = tail + 16 + 8 * WALK_EMIT;                                     // 64 words
     uint8_t *bufs = walk_smem + WALK_CTRL_BYTES;
     if (threadIdx.x < WALK_RING) ring[threadIdx.x] = make_uint4(0u, 0u, 0u, 0u);       // lap tags start at 1
     if (threadIdx.x < WALK_REQ) req[threadIdx.x] = make_uint4(0u, 0u, 0u, 0u);         // request numbers start at 1
-    if (threadIdx.x < 16 + 8 * WALK_EMIT) tail[threadIdx.x] = 0u;                       // tails, ready words, partial results, debug counters
+    if (threadIdx.x < 8 + 8 * WALK_EMIT) tail[threadIdx.x] = 0u;                        // tails, ready words, partial results
     __syncthreads();
 
     if (wid == 0) {
@@ -194,10 +193,8 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
         }
         uint32_t pushed = 0, safe = WALK_RING;               // descriptors pushed; pushes below `safe` find their slot free
         uint32_t nops = 0, prevc = 0;                        // ops pushed so far; direction of the previous run (Match, algo.rs:338)
-        uint32_t dbg_ringwait = 0;
         auto push = [&](uint32_t pi, uint32_t pj, uint32_t meta, uint32_t before) __attribute__((always_inline)) {
             if (pushed >= safe) {           // slot reuse: its previous descriptor (RING back) must have been consumed
-                dbg_ringwait++;
                 do {                        // tail[e] = 1 + the last descriptor emit warp e is done with: everything below all of them is consumed
                     const uint4 tl = lds_volatile_uint4(reinterpret_cast<const uint4 *>(tail));
                     uint32_t lo = tl.x;
@@ -235,23 +232,15 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
         };
         // code of the window cell (row rr relative to the buffer's first chunk, column jc of the strip): 0 S / 1 I / 2 D / 3 stop
         auto code_at = [&](uint32_t rr, uint32_t jc) __attribute__((always_inline)) -> uint32_t {
-            uint32_t off, sh;
-            if constexpr (R == 1 && K >= 4) {
-                // 64 cells (SPC steps x K columns) per 16-byte unit [chunk][fill-lane]; with u = t * K the cell is entry
-                // (u & 63) | k of unit (u >> 6, l).  Written out so that the chain from (rr, jc) to the address is five
-                // instructions deep (t, v, two masks, multiply-add, add)
-                constexpr uint32_t LK = (K == 4) ? 2u : (K == 8) ? 3u : 4u;
-                static_assert(K == 4 || K == 8 || K == 16, "code_at: K");
-                const uint32_t l = jc >> LK, t = rr + l;          // the step at which fill-lane l worked on this row
-                const uint32_t v = t << (LK - 2u);                // u >> 2
-                off = (v & ~15u) * 32u + (v & 12u) + (l << 4);    // (u >> 6) * 512 + l * 16 + (entry >> 4) * 4
-                sh = ((((t << LK) | (jc & (K - 1u))) & 15u)) * 2u;
-            } else {
-                const uint32_t l = jc / K, t = rr / R + l;        // the step at which fill-lane l worked on this row's block
-                const uint32_t idx2 = ((t / SPC) * 32u + l) * 64u + ((t % SPC) * R + rr % R) * K + jc % K;
-                off = (idx2 >> 4) * 4u;
-                sh = (idx2 & 15u) * 2u;
-            }
+            // 64 cells (SPC steps x K columns) per 16-byte unit [chunk][fill-lane]; with u = t * K the cell is entry
+            // (u & 63) | k of unit (u >> 6, l).  Written out so that the chain from (rr, jc) to the address is five
+            // instructions deep (t, v, two masks, multiply-add, add)
+            constexpr uint32_t LK = (K == 4) ? 2u : (K == 8) ? 3u : 4u;
+            static_assert(K == 4 || K == 8 || K == 16, "code_at: K");
+            const uint32_t l = jc >> LK, t = rr + l;              // the step at which fill-lane l worked on this row
+            const uint32_t v = t << (LK - 2u);                    // u >> 2
+            const uint32_t off = (v & ~15u) * 32u + (v & 12u) + (l << 4);   // (u >> 6) * 512 + l * 16 + (entry >> 4) * 4
+            const uint32_t sh = ((((t << LK) | (jc & (K - 1u))) & 15u)) * 2u;
             GX_CHECK(P.check, off < BUF_BYTES, 21);
             const uint32_t word = lds_code_word(cbase + off);
             return (word >> sh) & 3u;
@@ -260,17 +249,12 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
         // first row of the window that ends at panel row r1: WR rows, rounded down to a code chunk's first row, so that the
         // row inside the buffer is the row inside the window (no offset on the chain)
         auto win_r0 = [&](uint32_t r1) __attribute__((always_inline)) -> uint32_t {
-            return ((r1 >= WR - 1u) ? r1 - (WR - 1u) : 0u) / (SPC * R) * (SPC * R);
+            return ((r1 >= WR - 1u) ? r1 - (WR - 1u) : 0u) / SPC * SPC;
         };
-        uint32_t dbg_reloads = 0, dbg_miss = 0;
-        long long dbg_reload_cyc = 0;
         bool left_band = false;
-        const long long dbg_t0 = clock64();
         bool walking = (i != 0 && j != 0);
         while (walking) {
             // ---------------- (i, j) is an interior cell outside the current window: change windows
-            dbg_reloads++;
-            const long long dbg_r0 = P.debug ? clock64() : 0;
             const uint32_t jj = j - 1u, ii = i - 1u;
             const uint32_t tp = ii >> PANEL_H_LOG2, ts = jj / G::W, tr = ii & (PANEL_H - 1);
             uint32_t hit = WALK_NBUF;
@@ -279,7 +263,6 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
                 if (b != cb && bp[b] == tp && bs[b] == ts && tr >= br0[b] && tr <= br1[b]) hit = b;
             if (hit == WALK_NBUF) {
                 // neither prediction holds this cell: load the window that ends at this row into the buffer just left
-                dbg_miss++;
                 hit = cb;
                 const uint32_t r0 = win_r0(tr);
                 const uint32_t sq = post(hit, tp, ts, r0, tr);
@@ -365,7 +348,6 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
                     }
                 }
             }
-            if (P.debug) dbg_reload_cyc += clock64() - dbg_r0;
             if (c0 == 3u) break;                          // local alignment ends here; the cell is not emitted (algo.rs:401-405)
 
             // ---------------- run following inside the window
@@ -426,13 +408,6 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
             }
         }
         if (left_band && lane == 0) atomicAdd(P.left_band, 1u);
-        if (lane == 0) {
-            dbg[0] = (unsigned long long)pushed | ((unsigned long long)min(dbg_reloads, 0xffffu) << 32) |
-                     ((unsigned long long)min(dbg_miss, 0xffffu) << 48);
-            dbg[1] = (unsigned long long)(clock64() - dbg_t0);
-            dbg[2] = (unsigned long long)dbg_reload_cyc;
-            dbg[3] = dbg_ringwait;
-        }
         for (uint32_t e = 0; e < WALK_EMIT; ++e) push(0u, 0u, 3u, nops);   // end of path, one marker per emit warp
         nreq++;
         sts_volatile_uint4(req + nreq % WALK_REQ, make_uint4(0u, 0u, 0x80000000u, nreq));   // the loader warp may leave
@@ -448,8 +423,8 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
             const uint32_t p = d.x, s_ = d.y, r0 = d.z & 0xfffu, r1 = (d.z >> 12) & 0xfffu, b = (d.z >> 24) & 3u;
             uint32_t flag = 1u;
             if (P.tile_codes) flag = P.tile_codes[pd->tile_base + p * pd->S + s_];
-            const uint32_t c0w = (r0 / R) / SPC;
-            const uint32_t nch = (r1 / R + 31u) / SPC - c0w + 1u;
+            const uint32_t c0w = r0 / SPC;
+            const uint32_t nch = (r1 + 31u) / SPC - c0w + 1u;
             GX_CHECK(P.check, b < WALK_NBUF && nch * 512u <= BUF_BYTES && (uint64_t)(c0w + nch) * 512 <= pd->tile_code_bytes &&
                                   pd->codes_off + (uint64_t)(p * pd->S + s_ + 1) * pd->tile_code_bytes <= P.code_bytes, 23);
             const uint4 *tile = reinterpret_cast<const uint4 *>(P.codes + pd->codes_off + (uint64_t)(p * pd->S + s_) * pd->tile_code_bytes) +
@@ -544,12 +519,6 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
         res.mismatches = nx;
         res.gap_extensions = ne;
         res.opening_gaps = no;
-        if (P.debug) {
-            res.lcs_at_first_max = dbg[0];
-            res.fill_ms = (double)dbg[1];
-            res.walk_ms = (double)dbg[2];
-            res.start_i |= dbg[3] << 32;                       // ring-full waits of the path warp
-        }
         P.results[q] = res;
     }
 }

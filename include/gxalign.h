@@ -142,13 +142,12 @@ void gx_plan_destroy(gx_plan *plan);
 /* introspection for benchmarks: what==0 fill ms, 1 walk ms, 2 kernels launched by the last execute,
  * 3 cells (sum (m+1)(n+1)), 4 traceback bytes written per execute, 5 device bytes held by the plan,
  * 6 h2d bytes per upload, 7 d2h bytes per fetch, 8 tiles, 9 kernel family (0 wavefront, 1 read batch),
- * 15 K, 17 recurrence form (1 = CHAIN1), 18 ms of the GX_FLAG_LCS_AT_MAX passes, 19 R, 20 ticket-mode retries,
+ * 15 K, 17 recurrence form (1 = CHAIN1), 18 ms of the GX_FLAG_LCS_AT_MAX passes, 20 ticket-mode retries,
  * 21 resident strips (1) or tickets (0), 22 steps per hand-off batch, 23 share of the cells in code-writing tiles,
  * 24 executes repeated because a path left the code band, 25 fill scores through the one-hot IDP.4A path (1; set at upload),
- * 26 read plans: lane width of the read kernel the last execute ran (16 = s16x2, 32; 0 before) */
+ * 26 read plans: lane width of the read kernel the last execute ran (16 = s16x2, 32; 0 before).
+ * Any other number returns -1. */
 double gx_plan_stat(const gx_plan *plan, int what);
-/* debug (GX_FILL_STATS=2): per tile {ticket ns, first DP step ns, end ns, pair<<48|panel<<32|strip<<12|sm}; cap_words >= 4 * tiles */
-int gx_plan_debug_timeline(gx_plan *plan, uint64_t *out, uint64_t cap_words);
 
 /* ---- one very long pair, global, score only, cut into column bands (BASELINE config 5; SURVEY.md 8e).
  * Replaces alignment_table (algo.rs:151-282) for tables whose 48-byte cells could never exist (1 Mbp x 1 Mbp).

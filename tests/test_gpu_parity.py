@@ -162,7 +162,7 @@ _RAGGED_ORACLE = {}
 @pytest.mark.parametrize("k,r", KR_COMBOS)
 def test_random_medium_ragged_vs_linear(gx, oracle, k, r, chain1, monkeypatch):
     """sizes that cross strip (32*K columns), batch (up to 32 rows) and panel (4096 rows) boundaries, for every
-    K x R register tile the library can pick (GX_K / GX_R force it) and both forms of the recurrence"""
+    K the library can pick (GX_K forces it) and both forms of the recurrence"""
     force_kr(monkeypatch, k, r)
     monkeypatch.setenv("GX_CHAIN1", str(chain1))
     rng = np.random.default_rng(11)

@@ -5,7 +5,7 @@ for band in 0 ""; do
   python tools/mode_probe.py brca2 | grep "local=0 traceback=1"
   python tools/mode_probe.py corona1 | grep "local=0 traceback=1"
   rm -f gpurun_out/sweep_band.jsonl
-  python tools/sweep_kr.py --workloads corona6,corona11,corona23 --combos 4x1,8x1 --chain 0 --steps 4 --out gpurun_out/sweep_band.jsonl > /dev/null 2>&1
+  python tools/sweep_kr.py --workloads corona6,corona11,corona23 --k 4,8 --chain 0 --steps 4 --out sweep_band.jsonl > /dev/null 2>&1
   python - <<'PY'
 import json
 for l in open('gpurun_out/sweep_band.jsonl'):

@@ -4,7 +4,7 @@ mkdir -p gpurun_out
 for tag in r1 ""; do
   lib=genomics_rs_b200/libgxalign${tag:+_$tag}.so
   out=gpurun_out/sweep_r1cmp_${tag:-cur}.jsonl; rm -f $out
-  GX_LIB_PATH=$PWD/$lib timeout 600 python tools/sweep_kr.py --workloads brca2_global,brca2_local,corona1,corona6,corona11,corona23,corona45,nw200k --combos 4x1 --chain 0,1 --steps 5 --out $out > gpurun_out/sweep_r1cmp_${tag:-cur}.log 2>&1
+  GX_LIB_PATH=$PWD/$lib timeout 600 python tools/sweep_kr.py --workloads brca2_global,brca2_local,corona1,corona6,corona11,corona23,corona45,nw200k --k 4 --chain 0,1 --steps 5 --out $out > ${out%.jsonl}.log 2>&1
   echo "== ${tag:-current}"; python - $out <<'PY'
 import json, sys
 for l in open(sys.argv[1]):

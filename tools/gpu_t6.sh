@@ -1,6 +1,6 @@
 #!/bin/bash
 rm -f gpurun_out/sweep_t6.jsonl
-GX_TICKETS=1 python tools/sweep_kr.py --workloads corona6,corona11 --combos 4x1,8x1 --chain 0 --steps 4 --out gpurun_out/sweep_t6.jsonl > /dev/null 2>&1
+GX_TICKETS=1 python tools/sweep_kr.py --workloads corona6,corona11 --k 4,8 --chain 0 --steps 4 --out sweep_t6.jsonl > /dev/null 2>&1
 python - <<'PY'
 import json
 for l in open('gpurun_out/sweep_t6.jsonl'):

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Fill / walk time of every (K, R, recurrence form) register tile on the wavefront workloads, in ONE process
-(the debug switches are read per plan).  Results: one JSON line per run in gpurun_out/sweep_kr.jsonl.
+"""Fill / walk time of every K (columns per lane) and recurrence form on the wavefront workloads, in ONE process
+(GX_K / GX_CHAIN1 are read per plan).  Results: one JSON line per run in the --out file.
 
-    python tools/sweep_kr.py [--workloads brca2_global,brca2_local,corona45,corona6,nw200k,nw1m] [--combos 4x4,8x4] [--steps 5]
+    python tools/sweep_kr.py [--workloads brca2_global,brca2_local,corona45,corona6,nw200k,nw1m] [--k 4,8,16] [--steps 5]
 """
 import argparse
 import json
@@ -20,7 +20,7 @@ import genomics_rs_b200 as gx  # noqa: E402
 from genomics_rs_b200 import _lib, workloads as wl  # noqa: E402
 
 SCORES = wl.CONFIG_TOML
-ALL = [(4, 1), (8, 1), (16, 1)]
+ALL = [4, 8, 16]
 
 
 def workload(name):
@@ -47,14 +47,15 @@ def workload(name):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--workloads", default="brca2_global,brca2_local,corona6,corona45,nw200k")
-    ap.add_argument("--combos", default="")
+    ap.add_argument("--k", default="", help="comma list of K values to force (default: 4,8,16)")
     ap.add_argument("--chain", default="0,1")
     ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--batch", default="", help="comma list of GX_BATCH values (steps per hand-off batch) to force, e.g. 8,16,32")
     ap.add_argument("--auto-only", action="store_true", help="only the configuration the library picks itself")
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "sweep_kr.jsonl"))
     args = ap.parse_args()
-    combos = [tuple(int(x) for x in c.split("x")) for c in args.combos.split(",") if c] or ALL
+    if not os.path.dirname(args.out):   # a bare file name goes next to the default output file
+        args.out = os.path.join(os.path.dirname(ap.get_default("out")), args.out)
+    ks = [int(k) for k in args.k.split(",") if k] or ALL
     chains = [int(c) for c in args.chain.split(",")]
     _lib.ensure_init(0)
     os.makedirs(os.path.dirname(args.out), exist_ok=True)
@@ -63,15 +64,12 @@ def main():
         (blob, off1, len1, off2, len2), is_local, tb = workload(name)
         cells = int(((len1 + 1) * (len2 + 1)).sum())
         ref = None
-        batches = [int(b) for b in args.batch.split(",") if b] or [0]
-        for k, r, bsteps in [(0, 0, 0)] + ([] if args.auto_only else [(k, r, b) for k, r in combos for b in batches]):
+        for k in [0] + ([] if args.auto_only else ks):
             for c in ([-1] if k == 0 else chains):
-                for var in ("GX_K", "GX_R", "GX_CHAIN1", "GX_BATCH"):
+                for var in ("GX_K", "GX_CHAIN1"):
                     os.environ.pop(var, None)
                 if k:
-                    os.environ["GX_K"], os.environ["GX_R"], os.environ["GX_CHAIN1"] = str(k), str(r), str(c)
-                if bsteps:
-                    os.environ["GX_BATCH"] = str(bsteps)
+                    os.environ["GX_K"], os.environ["GX_CHAIN1"] = str(k), str(c)
                 try:
                     plan = gx.Plan(len1, len2, SCORES, is_local, traceback=tb)
                     plan.upload(blob, off1, off2)
@@ -85,7 +83,7 @@ def main():
                         walks.append(plan.walk_ms)
                     wall = (time.perf_counter() - t0) / args.steps * 1e3
                     scores = plan.fetch_scores().tolist() if not tb else plan.fetch()[0]["score"].tolist()
-                    rec = dict(workload=name, K=int(plan.stat(15)), R=int(plan.stat(19)), chain1=int(plan.stat(17)), forced=bool(k),
+                    rec = dict(workload=name, K=int(plan.stat(15)), chain1=int(plan.stat(17)), forced=bool(k),
                                batch=int(plan.stat(22)), resident=int(plan.stat(21)),
                                fill_ms=float(np.median(fills)), fill_min=float(min(fills)), walk_ms=float(np.median(walks)), wall_ms=wall,
                                gcups_fill=cells / (np.median(fills) * 1e-3) / 1e9, cells=cells)
@@ -94,7 +92,7 @@ def main():
                     rec["scores_agree"] = scores == ref
                     plan.close()
                 except Exception as e:   # keep sweeping: one broken tile shape must not hide the others
-                    rec = dict(workload=name, K=k, R=r, chain1=c, error=str(e)[:300])
+                    rec = dict(workload=name, K=k, chain1=c, error=str(e)[:300])
                 print(json.dumps(rec), flush=True)
                 fh.write(json.dumps(rec) + "\n")
                 fh.flush()
