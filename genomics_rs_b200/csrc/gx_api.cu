@@ -131,6 +131,8 @@ static void pool_free(Ctx *c, void *p) {
 // (gx_plan_create) or per streamed batch call, never on the execute path; -1 = not set.
 struct Tunables {
     int k = -1, chain1 = -1, tickets = -1, resident = -1, code_band = -1, walk_rows = 0, reads32 = 0, test_abort = 0;
+    int code_compact = 0, pad_ = 0;    // (pad_: no padding bytes, the plan cache compares Tunables with memcmp)
+    uint64_t code_budget = 0;          // cap on the bytes of a plan's codes buffer, 0 = none
 };
 static int env_int(const char *name, int dflt) {
     const char *e = getenv(name);
@@ -146,6 +148,9 @@ static Tunables read_tunables() {
     t.walk_rows = env_int("GX_WALK_ROWS", 0);          // 64..512, multiple of 64: rows of a code window of the walk
     t.reads32 = getenv("GX_READS32") ? 1 : 0;
     t.test_abort = getenv("GX_TEST_ABORT") ? 1 : 0;
+    t.code_compact = env_int("GX_CODE_COMPACT", 0);   // 1: compact code storage for every global traceback plan with a code band
+    const char *b = getenv("GX_CODE_BUDGET");
+    t.code_budget = b ? strtoull(b, nullptr, 10) : 0;
     return t;
 }
 
@@ -211,7 +216,11 @@ struct gx_plan {
     int reads_bits = 0;                // read plans: lane width of the kernel the last execute ran (16: s16x2, 32)
     bool code_band = false;            // global traceback plan in ticket mode: only tiles near the diagonal write direction codes
     uint8_t *d_tile_codes = nullptr;   // one flag per tile (indexed like tile_best)
-    int band_fallbacks = 0;            // executes repeated with codes everywhere because a path left the band
+    bool compact = false;              // compact code storage: only tiles in the code band have codes (gx_common.cuh)
+    uint32_t *d_tile_slot = nullptr;   // compact: slot of each tile's codes (indexed like tile_best)
+    uint2 *d_left_cell = nullptr;      // compact: per pair, the cell where a walk left the band (0,0 = it did not)
+    std::vector<uint64_t> code_w;      // code band: half-width of each pair's band in columns
+    int band_fallbacks = 0;            // executes repeated (codes everywhere, or a wider compact band) because a path left the band
     uint32_t left_band = 0;            // walks of the last execute that needed a tile outside the band
     double code_cell_frac = 1.0;       // share of the cells that lie in code-writing tiles
     uint64_t h2d_bytes = 0, d2h_bytes = 0, dev_bytes = 0;
@@ -269,7 +278,7 @@ static int launch_fill(gx_plan *pl, const FillParams &fp, int track_override = -
     const bool L = pl->is_local != 0, C = pl->traceback;
     const bool banded = pl->code_band && track_override < 0 && C && !L;   // two-variant kernel + per-tile flags
     FillKernel kern = (track_override >= 0) ? pick_fill(K, pl->prof, pl->chain1, L, false, track_override)
-                      : banded              ? pick_fill(K, pl->prof, pl->chain1, false, true, 4)
+                      : banded              ? pick_fill(K, pl->prof, pl->chain1, false, true, pl->compact ? 5 : 4)
                                             : pick_fill(K, pl->prof, pl->chain1, L, C, pl->track);
     if (!kern) {
         g_err = "no fill kernel for this K";
@@ -287,6 +296,7 @@ static int launch_fill(gx_plan *pl, const FillParams &fp, int track_override = -
     uint64_t cap = (uint64_t)c->sm_count * occ;
     FillParams fq = fp;
     fq.tile_codes = banded ? pl->d_tile_codes : nullptr;
+    fq.tile_slot = banded && pl->compact ? pl->d_tile_slot : nullptr;
     if (pl->resident && pl->n_strips > cap) {
         g_err = "resident-strips plan does not fit the device (fewer than 16 single-warp CTAs per SM)";
         return GX_ERR_INTERNAL;
@@ -365,9 +375,67 @@ static int check_scores_impl(gx_scores sc, uint64_t m, uint64_t n, bool local) {
 
 static void plan_release(gx_plan *pl) {
     Ctx *c = pl->ctx;
-    void *ptrs[] = {pl->d_tile_codes, pl->d_blob, pl->d_blob_sym, pl->d_lut, pl->d_pairs, pl->d_tiles, pl->d_strips, pl->d_ctrl, pl->d_colbuf, pl->d_top, pl->d_codes, pl->d_best, pl->d_first, pl->d_masks, pl->d_carry,
+    void *ptrs[] = {pl->d_tile_codes, pl->d_tile_slot, pl->d_left_cell, pl->d_blob, pl->d_blob_sym, pl->d_lut, pl->d_pairs, pl->d_tiles, pl->d_strips, pl->d_ctrl, pl->d_colbuf, pl->d_top, pl->d_codes, pl->d_best, pl->d_first, pl->d_masks, pl->d_carry,
                     pl->d_results, pl->d_ops, pl->d_off1, pl->d_off2, pl->d_len1, pl->d_len2, pl->d_scores, pl->d_cells};
     for (void *p : ptrs) pool_free(c, p);
+}
+
+// Code band of a global traceback plan (gx_common.cuh) from each pair's half-width pl->code_w[q]: the flag of every tile
+// and the share of the cells in code-writing tiles.  With `slots` (compact storage) also the slot of every in-band tile,
+// each pair's codes_off and the plan's code_bytes.
+static double code_band_layout(gx_plan *pl, std::vector<uint8_t> &flags, std::vector<uint32_t> *slots) {
+    const uint32_t W = 32u * (uint32_t)pl->K;
+    flags.assign(pl->best_entries, 1);
+    if (slots) slots->assign(pl->best_entries, 0u);
+    double with = 0, all = 0;
+    uint64_t codes = 0;
+    for (uint64_t q = 0; q < pl->n_pairs; ++q) {
+        PairDesc &pd = pl->pairs[q];
+        uint32_t used = 0;
+        for (uint32_t p2 = 0; p2 < pd.P; ++p2) {
+            const double rows = (double)std::min<uint64_t>(PANEL_H, pd.m - (uint64_t)p2 * PANEL_H);
+            for (uint32_t s2 = 0; s2 < pd.S; ++s2) {
+                const double cols = (double)std::min<uint64_t>((uint64_t)W, pd.n - (uint64_t)s2 * W);
+                const uint64_t t = pd.tile_base + (uint64_t)p2 * pd.S + s2;
+                const bool in = tile_in_code_band(pd.m, pd.n, p2, s2, W, pl->code_w[q]);
+                flags[t] = in ? 1 : 0;
+                if (slots && in) (*slots)[t] = used++;
+                all += rows * cols;
+                if (in) with += rows * cols;
+            }
+        }
+        if (slots) {
+            pd.codes_off = codes;
+            codes += (uint64_t)used * pd.tile_code_bytes;
+        }
+    }
+    if (slots) pl->code_bytes = codes;
+    return all > 0 ? with / all : 1.0;
+}
+
+// (Re)allocates the codes buffer of a compact plan at pl->code_bytes.  Pair q is the one named when it does not fit.
+static int alloc_compact_codes(gx_plan *pl, uint64_t q) {
+    Ctx *c = pl->ctx;
+    pool_free(c, pl->d_codes);
+    pl->d_codes = nullptr;
+    const bool over = pl->tun.code_budget != 0 && pl->code_bytes > pl->tun.code_budget;
+    const int rc = over ? GX_ERR_NOMEM : pool_alloc(c, pl->code_bytes, (void **)&pl->d_codes);
+    if (rc == GX_ERR_NOMEM)
+        g_err = "traceback codes do not fit: pair " + std::to_string(q) + " needs a code band of half-width " +
+                std::to_string(pl->code_w[q]) + " columns, which makes " + std::to_string(pl->code_bytes) + " bytes of codes (" +
+                (over ? "GX_CODE_BUDGET is " + std::to_string(pl->tun.code_budget) + " bytes" : std::string("device allocation failed")) + ")";
+    return rc;
+}
+
+// Copies a compact plan's tile flags, slot table and (once uploaded) pair descriptors to the device.
+static int upload_compact_layout(gx_plan *pl, const std::vector<uint8_t> &flags, const std::vector<uint32_t> &slots) {
+    Ctx *c = pl->ctx;
+    CK(cudaMemcpyAsync(pl->d_tile_codes, flags.data(), flags.size(), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(pl->d_tile_slot, slots.data(), slots.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    if (pl->uploaded)
+        CK(cudaMemcpyAsync(pl->d_pairs, pl->pairs.data(), pl->n_pairs * sizeof(PairDesc), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return GX_OK;
 }
 
 }  // namespace gx
@@ -752,7 +820,29 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
     A((16 + progress) * 4, (void **)&pl->d_ctrl);
     A(colbuf * 8, (void **)&pl->d_colbuf);
     A(top * 8, (void **)&pl->d_top);
-    if (pl->traceback) A(codes, (void **)&pl->d_codes);
+    // Direction codes.  Dense: every tile has its codes at its position in the table.  A global traceback plan with a code
+    // band whose dense codes do not fit (the device, or GX_CODE_BUDGET) keeps codes for the tiles of the band only (compact
+    // storage, allocated below); every plan that fits keeps dense codes.  A local alignment's path is not known before
+    // the fill, so its codes cannot be limited to a band.
+    const bool band_ok = pl->traceback && !is_local && !band_col0 && pl->tun.code_band != 0 && best > 0;
+    if (pl->traceback && rc == GX_OK) {
+        const bool over = pl->tun.code_budget != 0 && codes > pl->tun.code_budget;
+        if (band_ok && (pl->tun.code_compact > 0 || over)) {
+            pl->compact = true;
+        } else {
+            if (over) rc = GX_ERR_NOMEM;
+            else A(codes, (void **)&pl->d_codes);
+            if (rc == GX_ERR_NOMEM && band_ok) {
+                rc = GX_OK;
+                pl->compact = true;
+            } else if (rc == GX_ERR_NOMEM) {
+                g_err = "traceback codes: " + std::to_string(codes) + " bytes do not fit (" +
+                        (over ? "GX_CODE_BUDGET is " + std::to_string(pl->tun.code_budget) + " bytes" : std::string("device allocation failed")) + "); " +
+                        (is_local ? "a local alignment's path is not known before the fill, so its codes cannot be limited to a band"
+                                  : "the code band is off (GX_CODE_BAND=0)");
+            }
+        }
+    }
     if (pl->is_local) A(best * 16, (void **)&pl->d_best);
     if (pl->lcs) {
         pl->carry_words = (uint32_t)((max_len + 31) / 32 + 1);
@@ -766,31 +856,31 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
     // (6-pair shard, resident strips: fill 4.67 -> 4.07 ms; a single pair gains nothing -- its chain of strips runs at the
     // pace of the strips that do write codes -- and loses nothing.)
     std::vector<uint8_t> tile_codes;
-    if (pl->traceback && !is_local && !band_col0 && pl->tun.code_band != 0 && best > 0) {
-        tile_codes.assign(best, 1);
-        double with = 0, all = 0;
+    std::vector<uint32_t> tile_slot;
+    if (band_ok) {
+        pl->code_w.resize(n_pairs);
         for (uint64_t q = 0; q < n_pairs; ++q) {
             const PairDesc &pd = pl->pairs[q];
             const uint64_t dmn = pd.m > pd.n ? pd.m - pd.n : pd.n - pd.m;
-            const uint64_t cw = pl->tun.code_band > 0 ? (uint64_t)pl->tun.code_band : 1024 + dmn;
-            for (uint32_t p2 = 0; p2 < pd.P; ++p2) {
-                const double rows = (double)std::min<uint64_t>(PANEL_H, pd.m - (uint64_t)p2 * PANEL_H);
-                for (uint32_t s2 = 0; s2 < pd.S; ++s2) {
-                    const double cols = (double)std::min<uint64_t>((uint64_t)W, pd.n - (uint64_t)s2 * W);
-                    const bool in = tile_in_code_band(pd.m, pd.n, p2, s2, (uint32_t)W, cw);
-                    tile_codes[pd.tile_base + (uint64_t)p2 * pd.S + s2] = in ? 1 : 0;
-                    all += rows * cols;
-                    if (in) with += rows * cols;
-                }
-            }
+            pl->code_w[q] = pl->tun.code_band > 0 ? (uint64_t)pl->tun.code_band : 1024 + dmn;
         }
-        pl->code_cell_frac = all > 0 ? with / all : 1.0;
-        pl->code_band = pl->code_cell_frac < 0.9;     // not worth a second kernel variant otherwise
+        pl->code_cell_frac = code_band_layout(pl, tile_codes, pl->compact ? &tile_slot : nullptr);
+        pl->code_band = pl->compact || pl->code_cell_frac < 0.9;     // dense: not worth a second kernel variant otherwise
         if (!pl->code_band) pl->code_cell_frac = 1.0;
         if (pl->code_band) A(best, (void **)&pl->d_tile_codes);
+        if (pl->compact) {
+            A(best * 4, (void **)&pl->d_tile_slot);
+            A(n_pairs * sizeof(uint2), (void **)&pl->d_left_cell);
+            if (rc == GX_OK) {
+                const uint64_t qw = (uint64_t)(std::max_element(pl->code_w.begin(), pl->code_w.end()) - pl->code_w.begin());
+                rc = alloc_compact_codes(pl, qw);
+                if (rc == GX_OK) pl->dev_bytes += (pl->code_bytes + 511) & ~uint64_t(511);
+            }
+            if (rc == GX_OK) rc = upload_compact_layout(pl, tile_codes, tile_slot);
+        }
     }
     if (pl->traceback) A(ops, (void **)&pl->d_ops);
-    if (rc == GX_OK && pl->code_band) {
+    if (rc == GX_OK && pl->code_band && !pl->compact) {
         cudaError_t e = cudaMemcpyAsync(pl->d_tile_codes, tile_codes.data(), best, cudaMemcpyHostToDevice, c->stream);
         if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
         if (e != cudaSuccess) rc = fail_cuda(e, "upload tile code flags");
@@ -1136,6 +1226,36 @@ GX_GUARD_END
 
 static int plan_execute_once(gx_plan *pl, bool *aborted);
 
+// Compact storage, after an execute in which walks left the code band: widens the band of every pair whose walk left
+// (at least doubled, and wide enough to hold the tile of the cell where the walk stopped), then lays out and allocates
+// the codes again.  Pairs that stayed inside keep their width.
+static int widen_code_band(gx_plan *pl) {
+    Ctx *c = pl->ctx;
+    std::vector<uint2> cells(pl->n_pairs);
+    CK(cudaMemcpyAsync(cells.data(), pl->d_left_cell, pl->n_pairs * sizeof(uint2), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    const uint32_t W = 32u * (uint32_t)pl->K;
+    uint64_t named = 0;
+    for (uint64_t q = 0; q < pl->n_pairs; ++q) {
+        if (cells[q].x == 0u || cells[q].y == 0u) continue;    // this pair's walk stayed inside
+        const PairDesc &pd = pl->pairs[q];
+        const uint32_t p = (cells[q].x - 1u) >> PANEL_H_LOG2, s = (cells[q].y - 1u) / W;
+        uint64_t w = 2 * pl->code_w[q];
+        while (!tile_in_code_band(pd.m, pd.n, p, s, W, w)) w *= 2;
+        pl->code_w[q] = w;
+        named = q;
+    }
+    const uint64_t old_bytes = (pl->code_bytes + 511) & ~uint64_t(511);
+    std::vector<uint8_t> flags;
+    std::vector<uint32_t> slots;
+    pl->code_cell_frac = code_band_layout(pl, flags, &slots);
+    pl->dev_bytes -= old_bytes;
+    int rc = alloc_compact_codes(pl, named);
+    if (rc) return rc;
+    pl->dev_bytes += (pl->code_bytes + 511) & ~uint64_t(511);
+    return upload_compact_layout(pl, flags, slots);
+}
+
 // Ticket-ordered tile list of a plan (built at creation for ticket plans, on demand when a resident-strips plan falls back)
 static int plan_build_tickets(gx_plan *pl) {
     Ctx *c = pl->ctx;
@@ -1167,6 +1287,10 @@ int gx_plan_execute(gx_plan *pl) try {
     std::lock_guard<std::recursive_mutex> lk(g_mu);
     if (!pl) return GX_ERR_ARG;
     if (!pl->uploaded) return GX_ERR_ARG;
+    if (pl->compact && !pl->d_codes) {   // an earlier execute could not allocate its widened codes
+        g_err = "the traceback codes of this plan do not fit (see the execute that failed): create it again";
+        return GX_ERR_NOMEM;
+    }
     bool aborted = false;
     int rc = plan_execute_once(pl, &aborted);
     // A resident-strips fill that gave up waiting (SPIN_LIMIT: the device was shared with something that kept its strips
@@ -1183,7 +1307,24 @@ int gx_plan_execute(gx_plan *pl) try {
     // A path left the code band (a walk needed a tile that wrote no codes): repeat with codes in every tile.  The band is
     // an optimisation of where traceback pointers are STORED, never of what is computed, so this keeps every result exact;
     // the time of the discarded attempt stays in fill_ms / walk_ms.
-    if (rc == GX_OK && pl->code_band && pl->left_band != 0) {
+    // Compact storage has no memory for codes everywhere: the pairs whose walk left get a band at least twice as wide that
+    // holds the cell where it stopped, and the execute repeats until no walk leaves.  Every round at least doubles a
+    // pair's width, which the table bounds; the widths stay for the plan's life.
+    if (rc == GX_OK && pl->compact && pl->left_band != 0) {
+        float f0 = 0, w0 = 0;
+        int l0 = 0;
+        while (rc == GX_OK && pl->left_band != 0) {
+            f0 += pl->fill_ms;
+            w0 += pl->walk_ms;
+            l0 += pl->launches;
+            pl->band_fallbacks++;
+            rc = widen_code_band(pl);
+            if (rc == GX_OK) rc = plan_execute_once(pl, &aborted);
+        }
+        pl->fill_ms += f0;
+        pl->walk_ms += w0;
+        pl->launches += l0;
+    } else if (rc == GX_OK && pl->code_band && pl->left_band != 0) {
         const float f0 = pl->fill_ms, w0 = pl->walk_ms;
         const int l0 = pl->launches;
         pl->code_band = false;
@@ -1256,6 +1397,7 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
     }
     pl->colbuf_dirty = true;  // until this execute completes
     CK(cudaMemsetAsync(pl->d_ctrl, 0, (16 + pl->progress_entries) * 4, c->stream));
+    if (pl->d_left_cell) CK(cudaMemsetAsync(pl->d_left_cell, 0, pl->n_pairs * sizeof(uint2), c->stream));
     FillParams fp;
     fp.blob = pl->d_blob;
     fp.blob_sym = pl->prof ? pl->d_blob_sym : nullptr;
@@ -1310,6 +1452,8 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
     wp.check = pl->d_ctrl + 2;
     wp.left_band = pl->d_ctrl + 3;
     wp.tile_codes = pl->code_band ? pl->d_tile_codes : nullptr;
+    wp.tile_slot = pl->compact ? pl->d_tile_slot : nullptr;
+    wp.left_cell = pl->compact ? pl->d_left_cell : nullptr;
     wp.code_bytes = pl->code_bytes;
     wp.ops_bytes = pl->ops_bytes;
     {
@@ -1517,6 +1661,8 @@ double gx_plan_stat(const gx_plan *pl, int what) {
         case 18: return pl->lcs_ms;
         case 25: return pl->prof ? 1.0 : 0.0;
         case 26: return (double)pl->reads_bits;
+        case 27: return pl->compact ? 2.0 : pl->code_band ? 1.0 : 0.0;
+        case 28: return pl->code_band ? (double)*std::max_element(pl->code_w.begin(), pl->code_w.end()) : 0.0;
         default: return -1.0;
     }
 }

@@ -66,8 +66,12 @@ struct PairDesc {
 // the table's scaled diagonal j = i*n/m -- where the path of a global alignment runs; every other tile runs the score-only
 // cell (5 instead of 9 instructions).  One flag byte per tile (FillParams / WalkParams::tile_codes, indexed like tile_best;
 // null = every tile has codes), written by the host, read by the fill (which variant to run) and by the walk, which
-// verifies that every tile it enters has codes; if a path ever leaves the band the execute is repeated with codes
-// everywhere (gx_plan_execute), so results stay exact.
+// verifies that every tile it enters has codes; if a path ever leaves the band the execute is repeated (gx_plan_execute),
+// so results stay exact: with codes everywhere, or -- compact storage -- with a wider band for the pairs that left it.
+// Compact storage (pairs whose codes would not fit the device for every tile): only in-band tiles have memory for codes.
+// A slot table (FillParams / WalkParams::tile_slot, indexed like tile_best) maps tile (p,s) to its slot, its codes are at
+// codes_off + slot * tile_code_bytes; an out-of-band tile maps to slot 0 of its pair (tile (0,0) is always in the band),
+// so that every address the kernels form lies inside the codes buffer although nothing is read or written there.
 __host__ inline bool tile_in_code_band(uint64_t m, uint64_t n, uint32_t p, uint32_t s, uint32_t W, uint64_t code_w) {
     const uint64_t i0 = (uint64_t)p << PANEL_H_LOG2;
     const uint64_t i1 = (i0 + PANEL_H < m) ? i0 + PANEL_H : m;
@@ -109,6 +113,7 @@ struct FillParams {
     int4 *tile_best;
     uint32_t pad_keys;               // 1: padded columns of a pair's last strip could reach the maximum (s_mismatch >= 0): mask their keys
     int g, hg, ap, bp, h;            // ap = s_match - (h+g), bp = s_mismatch - (h+g): S is formed in E-space (E = V + h + g)
+    const uint32_t *tile_slot;       // compact code storage: slot of each tile's codes (code band, above), or null (dense)
 };
 
 struct WalkParams {
@@ -127,6 +132,8 @@ struct WalkParams {
     uint32_t *check;                 // checked build: where a failed bounds check records its site (control block word 2)
     uint64_t code_bytes, ops_bytes;  // sizes of the codes / ops buffers (checked build)
     uint32_t win_rows;               // rows of a code window of the walk (256 or 512)
+    const uint32_t *tile_slot;       // compact code storage: slot of each tile's codes, or null (tile (p,s) at p*S+s)
+    uint2 *left_cell;                // compact code storage: per pair, the cell whose tile was outside the band, or null
 };
 
 // ---------------------------------------------------------------------------------------------

@@ -259,8 +259,10 @@ __device__ __forceinline__ void run_batch(int (&eu)[K], int (&du)[K], const int 
 // BAND (global traceback plans with a code band): the kernel carries BOTH the traceback and the score-only variant of the
 // tile's batch loops and picks one per tile (FillParams::tile_codes).  The choice is made once per tile, around two complete
 // copies of the loops: dispatching per batch inside shared loops slowed a resident strip's traceback variant by 8-40 %
-// (BRCA2 fill 0.99 -> 1.41 ms) even when the other variant never ran.
-template <int K, bool LOCAL, bool CODES, int TRACK, bool PROF, bool CHAIN1, bool BAND = false>
+// (BRCA2 fill 0.99 -> 1.41 ms) even when the other variant never ran.  BAND_COMPACT also takes the tile's code address
+// from its slot (FillParams::tile_slot, gx_common.cuh) instead of from its position in the table.
+constexpr int BAND_NONE = 0, BAND_DENSE = 1, BAND_COMPACT = 2;
+template <int K, bool LOCAL, bool CODES, int TRACK, bool PROF, bool CHAIN1, int BAND = BAND_NONE>
 __global__ void __launch_bounds__(CTA_THREADS, CTAS_PER_SM) gx_fill_kernel(const FillParams P) {
     using G = Geo<K>;
     constexpr int W = G::W;
@@ -444,11 +446,13 @@ __global__ void __launch_bounds__(CTA_THREADS, CTAS_PER_SM) gx_fill_kernel(const
         int best = (CHAIN1 || TRACK == 3) ? INT32_MIN : -1, best_r = 0;
         const uint32_t nbat = tile_batches((uint32_t)rows, B);
         uint4 *code_base = nullptr;
+        int code_tile = p * S + s;       // where this tile's codes are, in tiles from the pair's codes_off
+        if constexpr (BAND == BAND_COMPACT) code_tile = (int)P.tile_slot[pd->tile_base + p * S + s];
         if (CODES)
-            code_base = reinterpret_cast<uint4 *>(P.codes + pd->codes_off + (uint64_t)(p * S + s) * pd->tile_code_bytes) + lane;
+            code_base = reinterpret_cast<uint4 *>(P.codes + pd->codes_off + (uint64_t)code_tile * pd->tile_code_bytes) + lane;
         // code band (global plans): tiles away from the table's diagonal run the score-only cell and write no codes
         bool tcodes = CODES;
-        if constexpr (BAND) tcodes = P.tile_codes[pd->tile_base + p * S + s] != 0;
+        if constexpr (BAND != BAND_NONE) tcodes = P.tile_codes[pd->tile_base + p * S + s] != 0;
 
         // ---- left boundary prefetch (LL protocol): lanes 0..B-1 fetch the entries of local rows B*bt + lane
         unsigned long long nxt = 0;
@@ -566,7 +570,7 @@ __global__ void __launch_bounds__(CTA_THREADS, CTAS_PER_SM) gx_fill_kernel(const
                     uint2 *outr = outring + (bt & 1u) * B;
                     uint4 *cdst = WC ? code_base + (size_t)bt * cpb * 32 : nullptr;
                     GX_CHECK(chk, !WC || ((size_t)(bt + 1) * cpb * 512 <= pd->tile_code_bytes &&
-                                          pd->codes_off + (uint64_t)(p * S + s + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
+                                          pd->codes_off + (uint64_t)(code_tile + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
                     if constexpr (!LOCAL && !CODES && TRACK == 0) {
                         if (thru)
                             run_batch<K, LOCAL, WC, TRACK, PROF, true, false, CHAIN1, true>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
@@ -588,7 +592,7 @@ __global__ void __launch_bounds__(CTA_THREADS, CTAS_PER_SM) gx_fill_kernel(const
                         uint2 *outr = outring + (bt & 1u) * B;
                         uint4 *cdst = WC ? code_base + (size_t)bt * cpb * 32 : nullptr;
                         GX_CHECK(chk, !WC || ((size_t)(bt + 1) * cpb * 512 <= pd->tile_code_bytes &&
-                                              pd->codes_off + (uint64_t)(p * S + s + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
+                                              pd->codes_off + (uint64_t)(code_tile + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
                         run_batch<K, LOCAL, WC, TRACK, PROF, false, true, CHAIN1>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
                                                                                   one, s1base, prof4, inring + (bt & 1u) * B, outr, cdst,
                                                                                   (int)(B * bt), rows, lane, kvalid, c1a, cpb, chk, -(int)delta, WARP_SMEM_S1 - (int)delta);
@@ -599,7 +603,7 @@ __global__ void __launch_bounds__(CTA_THREADS, CTAS_PER_SM) gx_fill_kernel(const
                         uint2 *outr = outring + (bt & 1u) * B;
                         uint4 *cdst = WC ? code_base + (size_t)bt * cpb * 32 : nullptr;
                         GX_CHECK(chk, !WC || ((size_t)(bt + 1) * cpb * 512 <= pd->tile_code_bytes &&
-                                              pd->codes_off + (uint64_t)(p * S + s + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
+                                              pd->codes_off + (uint64_t)(code_tile + 1) * pd->tile_code_bytes <= P.code_bytes), 7);
                         run_batch<K, LOCAL, WC, TRACK, PROF, false, false, CHAIN1>(eu, du, c2, eo, io, vd, best, best_r, g, hg, ap, bp,
                                                                                    one, s1base, prof4, inring + (bt & 1u) * B, outr, cdst,
                                                                                    (int)(B * bt), rows, lane, kvalid, c1a, cpb, chk, -(int)delta, WARP_SMEM_S1 - (int)delta);
@@ -608,7 +612,7 @@ __global__ void __launch_bounds__(CTA_THREADS, CTAS_PER_SM) gx_fill_kernel(const
                 }
             }
         };
-        if constexpr (BAND) {
+        if constexpr (BAND != BAND_NONE) {
             if (tcodes) run_tile(std::true_type{});
             else run_tile(std::false_type{});
         } else {

@@ -14,7 +14,8 @@ template <bool PROF>
 static FillKernel pick_mode(bool L, bool C, int track) {
     constexpr int K = GX_INST_K;
     constexpr bool CH = GX_INST_CHAIN != 0;
-    if (track == 4) return gx_fill_kernel<K, false, true, 0, PROF, CH, true>;   // global traceback with a code band
+    if (track == 4) return gx_fill_kernel<K, false, true, 0, PROF, CH, BAND_DENSE>;     // global traceback with a code band
+    if (track == 5) return gx_fill_kernel<K, false, true, 0, PROF, CH, BAND_COMPACT>;   // ... and compact code storage
     if (track == 3) {   // first-maximum pass of GX_FLAG_LCS_AT_MAX: score only
         if (L) return gx_fill_kernel<K, true, false, 3, PROF, CH>;
         return gx_fill_kernel<K, false, false, 3, PROF, CH>;

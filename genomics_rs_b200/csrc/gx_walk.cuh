@@ -14,7 +14,8 @@
 //                           length, the look-ahead lane that already read the turn cell supplies the next direction.
 //                           One self-contained 16-byte descriptor per run goes into a shared-memory ring.
 //   loader warp (warp 2)    owns the code windows: on request it copies the chunks of (tile, row range) into one of three
-//                           window buffers (cp.async, 16 B each) and checks the tile's code-band flag.  The path warp asks
+//                           window buffers (cp.async, 16 B each) and checks the tile's code-band flag (a tile outside
+//                           the band is not copied: with compact code storage it has no codes of its own).  The path warp asks
 //                           for the windows it will probably need next (left neighbour strip at the rows where a
 //                           diagonal path leaves this one; the rows above) when it enters a window, so a window change
 //                           normally costs a few shared-memory reads.
@@ -407,7 +408,10 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
                 left -= run;
             }
         }
-        if (left_band && lane == 0) atomicAdd(P.left_band, 1u);
+        if (left_band && lane == 0) {
+            atomicAdd(P.left_band, 1u);
+            if (P.left_cell) P.left_cell[q] = make_uint2(i, j);   // compact storage: the host widens this pair's band to hold it
+        }
         for (uint32_t e = 0; e < WALK_EMIT; ++e) push(0u, 0u, 3u, nops);   // end of path, one marker per emit warp
         nreq++;
         sts_volatile_uint4(req + nreq % WALK_REQ, make_uint4(0u, 0u, 0x80000000u, nreq));   // the loader warp may leave
@@ -423,14 +427,18 @@ __global__ void __launch_bounds__(WALK_THREADS) gx_walk_kernel(const WalkParams 
             const uint32_t p = d.x, s_ = d.y, r0 = d.z & 0xfffu, r1 = (d.z >> 12) & 0xfffu, b = (d.z >> 24) & 3u;
             uint32_t flag = 1u;
             if (P.tile_codes) flag = P.tile_codes[pd->tile_base + p * pd->S + s_];
+            // the tile's codes: at its position in the table, or (compact storage) at its slot
+            uint32_t ct = p * pd->S + s_;
+            if (P.tile_slot) ct = P.tile_slot[pd->tile_base + ct];
             const uint32_t c0w = r0 / SPC;
             const uint32_t nch = (r1 + 31u) / SPC - c0w + 1u;
             GX_CHECK(P.check, b < WALK_NBUF && nch * 512u <= BUF_BYTES && (uint64_t)(c0w + nch) * 512 <= pd->tile_code_bytes &&
-                                  pd->codes_off + (uint64_t)(p * pd->S + s_ + 1) * pd->tile_code_bytes <= P.code_bytes, 23);
-            const uint4 *tile = reinterpret_cast<const uint4 *>(P.codes + pd->codes_off + (uint64_t)(p * pd->S + s_) * pd->tile_code_bytes) +
+                                  pd->codes_off + (uint64_t)(ct + 1u) * pd->tile_code_bytes <= P.code_bytes, 23);
+            const uint4 *tile = reinterpret_cast<const uint4 *>(P.codes + pd->codes_off + (uint64_t)ct * pd->tile_code_bytes) +
                                 (size_t)c0w * 32 + lane;
             uint32_t dst = smem_u32(bufs + b * BUF_BYTES) + (uint32_t)lane * 16u;
-            for (uint32_t q2 = 0; q2 < nch; ++q2) {
+            // a tile outside the code band holds no codes: post its flag only (the path warp gives up if it enters it)
+            for (uint32_t q2 = 0; flag && q2 < nch; ++q2) {
                 asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(tile + (size_t)q2 * 32) : "memory");
                 dst += 32 * 16;
             }

@@ -37,7 +37,11 @@ enum {
     GX_ERR_OPS_CAP = 4,       /* ops buffer too small (need >= m+n+1) */
     GX_ERR_NO_DEVICE = 5,     /* no CUDA device of compute capability 10.x; there is no CPU path */
     GX_ERR_CUDA = 6,          /* CUDA runtime error, see gx_last_error() */
-    GX_ERR_NOMEM = 7,         /* device or host allocation failed / traceback storage would not fit */
+    GX_ERR_NOMEM = 7,         /* device or host allocation failed / traceback storage would not fit.  A global traceback
+                               * plan whose direction codes do not fit for every tile keeps them for the tiles of the
+                               * code band only (DESIGN.md 2); it fails when even those do not fit, also after the band
+                               * was widened for a path that left it (gx_last_error names the pair, the half-width
+                               * and the bytes).  Local traceback has no band: its codes must fit for every tile. */
     GX_ERR_NOT_INIT = 8,      /* gx_init() has not been called */
     GX_ERR_UNSUPPORTED = 9,   /* flag or mode not implemented */
     GX_ERR_INTERNAL = 10      /* impossible traceback state (the reference panics: algo.rs:407-408) */
@@ -128,8 +132,11 @@ int gx_score_batch_cells(const uint8_t *seq_blob, uint64_t blob_len,
 /* ---- the same, split into phases so that callers can keep inputs resident in HBM, overlap
  * copies, and time the kernels alone.  gx_align_batch == create + upload + execute + fetch (+ destroy, deferred).
  * gx_plan_execute never returns a wrong result for speed's sake: a resident-strips fill that gives up waiting is
- * repeated in ticket mode, and a global traceback plan that stores direction codes only near the table's diagonal
- * (the "code band", DESIGN.md 2) is repeated with codes everywhere if any path leaves the band. */
+ * repeated in ticket mode, and a global traceback plan that writes direction codes only near the table's diagonal
+ * (the "code band", DESIGN.md 2) is repeated if any path leaves the band: with codes everywhere, or -- when the plan
+ * keeps codes for the band's tiles only (compact storage, stat 27 = 2) -- with the band of each pair whose path left
+ * at least doubled and wide enough for where it left, until no path leaves.  The widths stay for the plan's life.  If
+ * the widened codes do not fit it returns GX_ERR_NOMEM. */
 typedef struct gx_plan gx_plan;
 int gx_plan_create(const uint64_t *len1, const uint64_t *len2, uint64_t n_pairs,
                    gx_scores sc, int is_local, int flags, gx_plan **plan);
@@ -140,12 +147,14 @@ int gx_plan_fetch(gx_plan *plan, gx_result *out, uint8_t *ops_blob, const uint64
 int gx_plan_fetch_scores(gx_plan *plan, int64_t *scores);   /* scores only: 4 B per pair on the wire for read batches */
 void gx_plan_destroy(gx_plan *plan);
 /* introspection for benchmarks: what==0 fill ms, 1 walk ms, 2 kernels launched by the last execute,
- * 3 cells (sum (m+1)(n+1)), 4 traceback bytes written per execute, 5 device bytes held by the plan,
+ * 3 cells (sum (m+1)(n+1)), 4 bytes of the traceback codes buffer, 5 device bytes held by the plan,
  * 6 h2d bytes per upload, 7 d2h bytes per fetch, 8 tiles, 9 kernel family (0 wavefront, 1 read batch),
  * 15 K, 17 recurrence form (1 = CHAIN1), 18 ms of the GX_FLAG_LCS_AT_MAX passes, 20 ticket-mode retries,
  * 21 resident strips (1) or tickets (0), 22 steps per hand-off batch, 23 share of the cells in code-writing tiles,
  * 24 executes repeated because a path left the code band, 25 fill scores through the one-hot IDP.4A path (1; set at upload),
- * 26 read plans: lane width of the read kernel the last execute ran (16 = s16x2, 32; 0 before).
+ * 26 read plans: lane width of the read kernel the last execute ran (16 = s16x2, 32; 0 before),
+ * 27 code storage (0 codes in every tile or none, 1 dense with a code band, 2 compact: codes for the band's tiles only),
+ * 28 widest code-band half-width in columns of the last execute (0 without a code band).
  * Any other number returns -1. */
 double gx_plan_stat(const gx_plan *plan, int what);
 
