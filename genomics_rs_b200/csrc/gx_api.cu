@@ -148,7 +148,7 @@ static Tunables read_tunables() {
     t.walk_rows = env_int("GX_WALK_ROWS", 0);          // 64..512, multiple of 64: rows of a code window of the walk
     t.reads32 = getenv("GX_READS32") ? 1 : 0;
     t.test_abort = getenv("GX_TEST_ABORT") ? 1 : 0;
-    t.code_compact = env_int("GX_CODE_COMPACT", 0);   // 1: compact code storage for every global traceback plan with a code band
+    t.code_compact = env_int("GX_CODE_COMPACT", 0);   // 1: compact code storage for every traceback plan that can have a code band
     const char *b = getenv("GX_CODE_BUDGET");
     t.code_budget = b ? strtoull(b, nullptr, 10) : 0;
     return t;
@@ -220,6 +220,8 @@ struct gx_plan {
     uint32_t *d_tile_slot = nullptr;   // compact: slot of each tile's codes (indexed like tile_best)
     uint2 *d_left_cell = nullptr;      // compact: per pair, the cell where a walk left the band (0,0 = it did not)
     std::vector<uint64_t> code_w;      // code band: half-width of each pair's band in columns
+    std::vector<uint2> code_end;       // code band: the cell each pair's band line ends at, (m, n) or the local start cell
+    float start_ms = 0;                // compact local plans: ms of the start-cell pass of the last execute
     int band_fallbacks = 0;            // executes repeated (codes everywhere, or a wider compact band) because a path left the band
     uint32_t left_band = 0;            // walks of the last execute that needed a tile outside the band
     double code_cell_frac = 1.0;       // share of the cells that lie in code-writing tiles
@@ -252,9 +254,9 @@ namespace gx {
 #define GX_COMBOS(X) X(4) X(8) X(16)
 
 // the fill kernels are instantiated in gx_fill_inst.cu, one translation unit per (K, CHAIN1) so that they build in parallel
-#define GX_DECL(K)                                                   \
-    FillKernel pick_fill_##K##_0(bool prof, bool L, bool C, int track); \
-    FillKernel pick_fill_##K##_1(bool prof, bool L, bool C, int track);
+#define GX_DECL(K)                                                             \
+    FillKernel pick_fill_##K##_0(bool prof, bool L, bool C, int track, int band); \
+    FillKernel pick_fill_##K##_1(bool prof, bool L, bool C, int track, int band);
 GX_COMBOS(GX_DECL)
 #undef GX_DECL
 
@@ -265,8 +267,9 @@ static bool combo_ok(int K) {
     return false;
 }
 
-static FillKernel pick_fill(int K, bool prof, bool chain1, bool L, bool C, int track) {
-#define GX_PICK(k) if (K == k) return chain1 ? pick_fill_##k##_1(prof, L, C, track) : pick_fill_##k##_0(prof, L, C, track);
+// band: BAND_NONE, or the code-band instance of a traceback plan (BAND_DENSE / BAND_COMPACT, gx_fill.cuh)
+static FillKernel pick_fill(int K, bool prof, bool chain1, bool L, bool C, int track, int band) {
+#define GX_PICK(k) if (K == k) return chain1 ? pick_fill_##k##_1(prof, L, C, track, band) : pick_fill_##k##_0(prof, L, C, track, band);
     GX_COMBOS(GX_PICK)
 #undef GX_PICK
     return nullptr;
@@ -276,10 +279,11 @@ static int launch_fill(gx_plan *pl, const FillParams &fp, int track_override = -
     Ctx *c = pl->ctx;
     const int K = pl->K;
     const bool L = pl->is_local != 0, C = pl->traceback;
-    const bool banded = pl->code_band && track_override < 0 && C && !L;   // two-variant kernel + per-tile flags
-    FillKernel kern = (track_override >= 0) ? pick_fill(K, pl->prof, pl->chain1, L, false, track_override)
-                      : banded              ? pick_fill(K, pl->prof, pl->chain1, false, true, pl->compact ? 5 : 4)
-                                            : pick_fill(K, pl->prof, pl->chain1, L, C, pl->track);
+    // two-variant kernel + per-tile flags: global traceback plans with a code band, local ones with compact storage
+    const bool banded = pl->code_band && track_override < 0 && C && (!L || pl->compact);
+    FillKernel kern = (track_override >= 0) ? pick_fill(K, pl->prof, pl->chain1, L, false, track_override, BAND_NONE)
+                      : banded              ? pick_fill(K, pl->prof, pl->chain1, L, true, 0, pl->compact ? BAND_COMPACT : BAND_DENSE)
+                                            : pick_fill(K, pl->prof, pl->chain1, L, C, pl->track, BAND_NONE);
     if (!kern) {
         g_err = "no fill kernel for this K";
         return GX_ERR_INTERNAL;
@@ -380,7 +384,24 @@ static void plan_release(gx_plan *pl) {
     for (void *p : ptrs) pool_free(c, p);
 }
 
-// Code band of a global traceback plan (gx_common.cuh) from each pair's half-width pl->code_w[q]: the flag of every tile
+// Half-width a pair's code band starts with: GX_CODE_BAND=w, else 1024 columns (+ |m - n| for a global plan, whose line
+// is the scaled diagonal; a local plan's line has slope 1 and ends at the start cell)
+static uint64_t default_code_w(const gx_plan *pl, const PairDesc &pd) {
+    if (pl->tun.code_band > 0) return (uint64_t)pl->tun.code_band;
+    if (pl->is_local) return 1024;
+    return 1024 + (pd.m > pd.n ? pd.m - pd.n : pd.n - pd.m);
+}
+
+// Tile (p, s) of pair q in its code band of half-width w (gx_common.cuh): global plans around the diagonal (0,0)-(m,n),
+// local plans around the slope-1 line that ends at the pair's start cell code_end[q]
+static bool pair_tile_in_band(const gx_plan *pl, uint64_t q, uint32_t p, uint32_t s, uint32_t W, uint64_t w) {
+    const PairDesc &pd = pl->pairs[q];
+    const uint64_t a1 = pl->code_end[q].x, b1 = pl->code_end[q].y, d = pl->is_local ? std::min(a1, b1) : 0;
+    const uint64_t a0 = pl->is_local ? a1 - d : 0, b0 = pl->is_local ? b1 - d : 0;
+    return tile_in_code_band(a0, b0, a1, b1, pd.m, p, s, W, w);
+}
+
+// Code band of a traceback plan (gx_common.cuh) from each pair's half-width pl->code_w[q]: the flag of every tile
 // and the share of the cells in code-writing tiles.  With `slots` (compact storage) also the slot of every in-band tile,
 // each pair's codes_off and the plan's code_bytes.
 static double code_band_layout(gx_plan *pl, std::vector<uint8_t> &flags, std::vector<uint32_t> *slots) {
@@ -397,7 +418,7 @@ static double code_band_layout(gx_plan *pl, std::vector<uint8_t> &flags, std::ve
             for (uint32_t s2 = 0; s2 < pd.S; ++s2) {
                 const double cols = (double)std::min<uint64_t>((uint64_t)W, pd.n - (uint64_t)s2 * W);
                 const uint64_t t = pd.tile_base + (uint64_t)p2 * pd.S + s2;
-                const bool in = tile_in_code_band(pd.m, pd.n, p2, s2, W, pl->code_w[q]);
+                const bool in = pair_tile_in_band(pl, q, p2, s2, W, pl->code_w[q]);
                 flags[t] = in ? 1 : 0;
                 if (slots && in) (*slots)[t] = used++;
                 all += rows * cols;
@@ -421,7 +442,7 @@ static int alloc_compact_codes(gx_plan *pl, uint64_t q) {
     const bool over = pl->tun.code_budget != 0 && pl->code_bytes > pl->tun.code_budget;
     const int rc = over ? GX_ERR_NOMEM : pool_alloc(c, pl->code_bytes, (void **)&pl->d_codes);
     if (rc == GX_ERR_NOMEM)
-        g_err = "traceback codes do not fit: pair " + std::to_string(q) + " needs a code band of half-width " +
+        g_err = std::string("traceback codes do not fit: ") + (pl->is_local ? "local pair " : "pair ") + std::to_string(q) + " needs a code band of half-width " +
                 std::to_string(pl->code_w[q]) + " columns, which makes " + std::to_string(pl->code_bytes) + " bytes of codes (" +
                 (over ? "GX_CODE_BUDGET is " + std::to_string(pl->tun.code_budget) + " bytes" : std::string("device allocation failed")) + ")";
     return rc;
@@ -436,6 +457,20 @@ static int upload_compact_layout(gx_plan *pl, const std::vector<uint8_t> &flags,
         CK(cudaMemcpyAsync(pl->d_pairs, pl->pairs.data(), pl->n_pairs * sizeof(PairDesc), cudaMemcpyHostToDevice, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     return GX_OK;
+}
+
+// A compact plan whose pairs' half-widths or end cells changed: lays out the band again, reallocates the codes (pair q is
+// the one named when they do not fit) and uploads the layout.
+static int relayout_compact(gx_plan *pl, uint64_t q) {
+    const uint64_t old_bytes = (pl->code_bytes + 511) & ~uint64_t(511);
+    std::vector<uint8_t> flags;
+    std::vector<uint32_t> slots;
+    pl->code_cell_frac = code_band_layout(pl, flags, &slots);
+    pl->dev_bytes -= old_bytes;
+    int rc = alloc_compact_codes(pl, q);
+    if (rc) return rc;
+    pl->dev_bytes += (pl->code_bytes + 511) & ~uint64_t(511);
+    return upload_compact_layout(pl, flags, slots);
 }
 
 }  // namespace gx
@@ -820,11 +855,11 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
     A((16 + progress) * 4, (void **)&pl->d_ctrl);
     A(colbuf * 8, (void **)&pl->d_colbuf);
     A(top * 8, (void **)&pl->d_top);
-    // Direction codes.  Dense: every tile has its codes at its position in the table.  A global traceback plan with a code
-    // band whose dense codes do not fit (the device, or GX_CODE_BUDGET) keeps codes for the tiles of the band only (compact
-    // storage, allocated below); every plan that fits keeps dense codes.  A local alignment's path is not known before
-    // the fill, so its codes cannot be limited to a band.
-    const bool band_ok = pl->traceback && !is_local && !band_col0 && pl->tun.code_band != 0 && best > 0;
+    // Direction codes.  Dense: every tile has its codes at its position in the table.  A traceback plan with a code band
+    // whose dense codes do not fit (the device, or GX_CODE_BUDGET) keeps codes for the tiles of the band only (compact
+    // storage, allocated below); every plan that fits keeps dense codes.  A local plan's band needs its start cell, which
+    // each execute finds first with a score-only pass (gx_plan_execute), so only compact local plans have a band.
+    const bool band_ok = pl->traceback && !band_col0 && pl->tun.code_band != 0 && best > 0;
     if (pl->traceback && rc == GX_OK) {
         const bool over = pl->tun.code_budget != 0 && codes > pl->tun.code_budget;
         if (band_ok && (pl->tun.code_compact > 0 || over)) {
@@ -836,10 +871,9 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
                 rc = GX_OK;
                 pl->compact = true;
             } else if (rc == GX_ERR_NOMEM) {
-                g_err = "traceback codes: " + std::to_string(codes) + " bytes do not fit (" +
-                        (over ? "GX_CODE_BUDGET is " + std::to_string(pl->tun.code_budget) + " bytes" : std::string("device allocation failed")) + "); " +
-                        (is_local ? "a local alignment's path is not known before the fill, so its codes cannot be limited to a band"
-                                  : "the code band is off (GX_CODE_BAND=0)");
+                g_err = std::string("traceback codes") + (is_local ? " of a local plan: " : ": ") + std::to_string(codes) + " bytes do not fit (" +
+                        (over ? "GX_CODE_BUDGET is " + std::to_string(pl->tun.code_budget) + " bytes" : std::string("device allocation failed")) +
+                        "); the code band is off (GX_CODE_BAND=0)";
             }
         }
     }
@@ -851,18 +885,21 @@ static int plan_create_locked(const uint64_t *len1, const uint64_t *len2, uint64
         A((size_t)n_pairs * 2 * pl->carry_words * 4 + 16, (void **)&pl->d_carry);
     }
     A(n_pairs * sizeof(DevResult), (void **)&pl->d_results);
-    // code band (see gx_common.cuh): global traceback plans.  A global alignment's path runs along the scaled diagonal
-    // j = i*n/m (all 45 coronavirus pairs stay within 316 columns of it): default half-width 1024 + |m - n| columns.
+    // code band (see gx_common.cuh): global traceback plans, and local ones with compact storage.  A global alignment's path
+    // runs along the scaled diagonal j = i*n/m (all 45 coronavirus pairs stay within 316 columns of it): default half-width
+    // 1024 + |m - n| columns.  A local plan's band is laid out here for the provisional start cell (m, n), so that its codes
+    // size is known and a budget that cannot hold even that fails now; each execute moves it to the real start cell.
     // (6-pair shard, resident strips: fill 4.67 -> 4.07 ms; a single pair gains nothing -- its chain of strips runs at the
     // pace of the strips that do write codes -- and loses nothing.)
     std::vector<uint8_t> tile_codes;
     std::vector<uint32_t> tile_slot;
-    if (band_ok) {
+    if (band_ok && (!is_local || pl->compact)) {
         pl->code_w.resize(n_pairs);
+        pl->code_end.resize(n_pairs);
         for (uint64_t q = 0; q < n_pairs; ++q) {
             const PairDesc &pd = pl->pairs[q];
-            const uint64_t dmn = pd.m > pd.n ? pd.m - pd.n : pd.n - pd.m;
-            pl->code_w[q] = pl->tun.code_band > 0 ? (uint64_t)pl->tun.code_band : 1024 + dmn;
+            pl->code_w[q] = default_code_w(pl, pd);
+            pl->code_end[q] = make_uint2(pd.m, pd.n);
         }
         pl->code_cell_frac = code_band_layout(pl, tile_codes, pl->compact ? &tile_slot : nullptr);
         pl->code_band = pl->compact || pl->code_cell_frac < 0.9;     // dense: not worth a second kernel variant otherwise
@@ -1225,6 +1262,8 @@ int gx_plan_upload(gx_plan *pl, const uint8_t *blob, uint64_t blob_len, const ui
 GX_GUARD_END
 
 static int plan_execute_once(gx_plan *pl, bool *aborted);
+static FillParams make_fill_params(const gx_plan *pl);
+static WalkParams make_walk_params(const gx_plan *pl);
 
 // Compact storage, after an execute in which walks left the code band: widens the band of every pair whose walk left
 // (at least doubled, and wide enough to hold the tile of the cell where the walk stopped), then lays out and allocates
@@ -1238,22 +1277,67 @@ static int widen_code_band(gx_plan *pl) {
     uint64_t named = 0;
     for (uint64_t q = 0; q < pl->n_pairs; ++q) {
         if (cells[q].x == 0u || cells[q].y == 0u) continue;    // this pair's walk stayed inside
-        const PairDesc &pd = pl->pairs[q];
         const uint32_t p = (cells[q].x - 1u) >> PANEL_H_LOG2, s = (cells[q].y - 1u) / W;
+        // terminates: the walk only moves up and left from the band's end cell, so this tile starts before it
         uint64_t w = 2 * pl->code_w[q];
-        while (!tile_in_code_band(pd.m, pd.n, p, s, W, w)) w *= 2;
+        while (!pair_tile_in_band(pl, q, p, s, W, w)) w *= 2;
         pl->code_w[q] = w;
         named = q;
     }
-    const uint64_t old_bytes = (pl->code_bytes + 511) & ~uint64_t(511);
-    std::vector<uint8_t> flags;
-    std::vector<uint32_t> slots;
-    pl->code_cell_frac = code_band_layout(pl, flags, &slots);
-    pl->dev_bytes -= old_bytes;
-    int rc = alloc_compact_codes(pl, named);
+    return relayout_compact(pl, named);
+}
+
+// First phase of an execute of a compact local plan: a score-only fill that tracks the start cell (TRACK 2), and the
+// walk's reduction of tile_best into the results, without traceback.  Every pair whose start cell differs from the end
+// cell of its code band gets a band of the default half-width that ends there; the others keep band and width.  The
+// traceback fill (plan_execute_once) tracks nothing, so its walk reduces the tile_best left here: the same start cell.
+static int local_start_pass(gx_plan *pl, bool *aborted, int *launches) {
+    Ctx *c = pl->ctx;
+    CK(cudaSetDevice(c->device));
+    pl->start_ms = 0;
+    CK(cudaEventRecord(c->ev[0], c->stream));
+    if (pl->colbuf_dirty) {
+        if (pl->colbuf_entries) CK(cudaMemsetAsync(pl->d_colbuf, 0xff, pl->colbuf_entries * 8, c->stream));  // parity bit 1 everywhere
+        pl->parity = 0;
+    }
+    pl->colbuf_dirty = true;  // until this pass completes
+    CK(cudaMemsetAsync(pl->d_ctrl, 0, (16 + pl->progress_entries) * 4, c->stream));
+    int rc = launch_fill(pl, make_fill_params(pl), 2);
     if (rc) return rc;
-    pl->dev_bytes += (pl->code_bytes + 511) & ~uint64_t(511);
-    return upload_compact_layout(pl, flags, slots);
+    WalkParams wp = make_walk_params(pl);
+    wp.traceback = 0;
+    rc = launch_walk(pl, wp);
+    if (rc) return rc;
+    *launches = 2;
+    CK(cudaEventRecord(c->ev[1], c->stream));
+    uint32_t ctrl_words[2] = {0, 0};   // [0] abort word, [1] checked build: site of a failed bounds check
+    CK(cudaMemcpyAsync(ctrl_words, pl->d_ctrl + 1, 8, cudaMemcpyDeviceToHost, c->stream));
+    std::vector<DevResult> res(pl->n_pairs);
+    CK(cudaMemcpyAsync(res.data(), pl->d_results, pl->n_pairs * sizeof(DevResult), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    if (ctrl_words[1]) {
+        g_err = "checked build: device bounds check failed at site " + std::to_string(ctrl_words[1]);
+        return GX_ERR_INTERNAL;
+    }
+    if (ctrl_words[0]) {
+        g_err = "fill kernel aborted: a tile waited > SPIN_LIMIT polls for a dependency";
+        *aborted = true;
+        return GX_ERR_INTERNAL;
+    }
+    CK(cudaEventElapsedTime(&pl->start_ms, c->ev[0], c->ev[1]));
+    pl->parity ^= 1u;
+    pl->colbuf_dirty = false;
+    bool moved = false;
+    for (uint64_t q = 0; q < pl->n_pairs; ++q) {
+        if (pl->pairs[q].P == 0) continue;    // no tiles, no band
+        const uint2 e = make_uint2((uint32_t)res[q].start_i, (uint32_t)res[q].start_j);
+        if (e.x == pl->code_end[q].x && e.y == pl->code_end[q].y) continue;
+        pl->code_end[q] = e;
+        pl->code_w[q] = default_code_w(pl, pl->pairs[q]);
+        moved = true;
+    }
+    if (!moved) return GX_OK;
+    return relayout_compact(pl, (uint64_t)(std::max_element(pl->code_w.begin(), pl->code_w.end()) - pl->code_w.begin()));
 }
 
 // Ticket-ordered tile list of a plan (built at creation for ticket plans, on demand when a resident-strips plan falls back)
@@ -1292,7 +1376,15 @@ int gx_plan_execute(gx_plan *pl) try {
         return GX_ERR_NOMEM;
     }
     bool aborted = false;
-    int rc = plan_execute_once(pl, &aborted);
+    // A compact local plan finds its start cells first and moves the code bands there (local_start_pass); the widening
+    // rounds below repeat only the traceback fill and walk, the start cells cannot change between them.
+    const bool start_pass = pl->compact && pl->is_local;
+    int start_launches = 0;
+    auto run = [&]() {
+        int r = start_pass ? local_start_pass(pl, &aborted, &start_launches) : GX_OK;
+        return r ? r : plan_execute_once(pl, &aborted);
+    };
+    int rc = run();
     // A resident-strips fill that gave up waiting (SPIN_LIMIT: the device was shared with something that kept its strips
     // from running together, or was lost) is repeated ONCE in ticket mode, where a waiting warp only ever waits for
     // warps that hold earlier tickets.  Band plans that span processes cannot be rewound: they stay failed (poisoned).
@@ -1302,7 +1394,7 @@ int gx_plan_execute(gx_plan *pl) try {
         int rb = plan_build_tickets(pl);
         if (rb) return rb;
         pl->colbuf_dirty = true;     // the aborted execute left the LL parity words in an unknown state
-        rc = plan_execute_once(pl, &aborted);
+        rc = run();
     }
     // A path left the code band (a walk needed a tile that wrote no codes): repeat with codes in every tile.  The band is
     // an optimisation of where traceback pointers are STORED, never of what is computed, so this keeps every result exact;
@@ -1335,9 +1427,71 @@ int gx_plan_execute(gx_plan *pl) try {
         pl->walk_ms += w0;
         pl->launches += l0;
     }
+    if (rc == GX_OK && start_pass) {
+        pl->fill_ms += pl->start_ms;
+        pl->launches += start_launches;
+    }
     return rc;
 }
 GX_GUARD_END
+
+// Kernel parameters of an execute of a wavefront plan
+static FillParams make_fill_params(const gx_plan *pl) {
+    FillParams fp;
+    const gx_scores sc = pl->sc;
+    gx_band *bd = pl->band;
+    fp.blob = pl->d_blob;
+    fp.blob_sym = pl->prof ? pl->d_blob_sym : nullptr;
+    fp.one = 1u;
+    fp.pad_keys = sc.s_mismatch >= 0 ? 1u : 0u;
+    fp.pairs = pl->d_pairs;
+    fp.n_pairs = (uint32_t)pl->n_pairs;
+    fp.code_bytes = pl->code_bytes;
+    fp.tiles = pl->d_tiles;
+    fp.n_tiles = (uint32_t)pl->n_tiles;
+    fp.pmax = 0;   // launch_fill switches to the [strip][panel] list when every strip gets a warp
+    fp.parity = pl->parity;
+    fp.cpb = pl->cpb;
+    fp.epoch = bd ? bd->epoch + 1 : 0;
+    fp.ticket = pl->d_ctrl;
+    fp.progress = pl->d_ctrl + 16;
+    fp.colbuf = pl->d_colbuf;
+    fp.top = pl->d_top;
+    fp.codes = pl->d_codes;
+    fp.tile_best = pl->d_best;
+    fp.g = sc.g;
+    fp.h = sc.h;
+    fp.hg = sc.h + sc.g;
+    fp.ap = sc.s_match - fp.hg;
+    fp.bp = sc.s_mismatch - fp.hg;
+    return fp;
+}
+
+static WalkParams make_walk_params(const gx_plan *pl) {
+    WalkParams wp;
+    wp.blob = pl->d_blob;
+    wp.pairs = pl->d_pairs;
+    wp.n_pairs = (uint32_t)pl->n_pairs;
+    wp.top = pl->d_top;
+    wp.codes = pl->d_codes;
+    wp.tile_best = pl->d_best;
+    wp.results = pl->d_results;
+    wp.ops = pl->d_ops;
+    wp.g = pl->sc.g;
+    wp.h = pl->sc.h;
+    wp.hg = pl->sc.h + pl->sc.g;
+    wp.is_local = pl->is_local;
+    wp.traceback = pl->traceback ? 1 : 0;
+    wp.have_best = pl->track == 2 ? 1 : 0;
+    wp.check = pl->d_ctrl + 2;
+    wp.left_band = pl->d_ctrl + 3;
+    wp.tile_codes = pl->code_band ? pl->d_tile_codes : nullptr;
+    wp.tile_slot = pl->compact ? pl->d_tile_slot : nullptr;
+    wp.left_cell = pl->compact ? pl->d_left_cell : nullptr;
+    wp.code_bytes = pl->code_bytes;
+    wp.ops_bytes = pl->ops_bytes;
+    return wp;
+}
 
 static int plan_execute_once(gx_plan *pl, bool *aborted) {
     Ctx *c = pl->ctx;
@@ -1398,31 +1552,7 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
     pl->colbuf_dirty = true;  // until this execute completes
     CK(cudaMemsetAsync(pl->d_ctrl, 0, (16 + pl->progress_entries) * 4, c->stream));
     if (pl->d_left_cell) CK(cudaMemsetAsync(pl->d_left_cell, 0, pl->n_pairs * sizeof(uint2), c->stream));
-    FillParams fp;
-    fp.blob = pl->d_blob;
-    fp.blob_sym = pl->prof ? pl->d_blob_sym : nullptr;
-    fp.one = 1u;
-    fp.pad_keys = sc.s_mismatch >= 0 ? 1u : 0u;
-    fp.pairs = pl->d_pairs;
-    fp.n_pairs = (uint32_t)pl->n_pairs;
-    fp.code_bytes = pl->code_bytes;
-    fp.tiles = pl->d_tiles;
-    fp.n_tiles = (uint32_t)pl->n_tiles;
-    fp.pmax = 0;   // launch_fill switches to the [strip][panel] list when every strip gets a warp
-    fp.parity = pl->parity;
-    fp.cpb = pl->cpb;
-    fp.epoch = bd ? bd->epoch + 1 : 0;
-    fp.ticket = pl->d_ctrl;
-    fp.progress = pl->d_ctrl + 16;
-    fp.colbuf = pl->d_colbuf;
-    fp.top = pl->d_top;
-    fp.codes = pl->d_codes;
-    fp.tile_best = pl->d_best;
-    fp.g = sc.g;
-    fp.h = sc.h;
-    fp.hg = sc.h + sc.g;
-    fp.ap = sc.s_match - fp.hg;
-    fp.bp = sc.s_mismatch - fp.hg;
+    FillParams fp = make_fill_params(pl);
     if (pl->n_tiles) {
         int rc = launch_fill(pl, fp);
         if (rc) return rc;
@@ -1434,28 +1564,7 @@ static int plan_execute_once(gx_plan *pl, bool *aborted) {
         CK(cudaGetLastError());
         pl->launches++;
     }
-    WalkParams wp;
-    wp.blob = pl->d_blob;
-    wp.pairs = pl->d_pairs;
-    wp.n_pairs = (uint32_t)pl->n_pairs;
-    wp.top = pl->d_top;
-    wp.codes = pl->d_codes;
-    wp.tile_best = pl->d_best;
-    wp.results = pl->d_results;
-    wp.ops = pl->d_ops;
-    wp.g = sc.g;
-    wp.h = sc.h;
-    wp.hg = fp.hg;
-    wp.is_local = pl->is_local;
-    wp.traceback = pl->traceback ? 1 : 0;
-    wp.have_best = pl->track == 2 ? 1 : 0;
-    wp.check = pl->d_ctrl + 2;
-    wp.left_band = pl->d_ctrl + 3;
-    wp.tile_codes = pl->code_band ? pl->d_tile_codes : nullptr;
-    wp.tile_slot = pl->compact ? pl->d_tile_slot : nullptr;
-    wp.left_cell = pl->compact ? pl->d_left_cell : nullptr;
-    wp.code_bytes = pl->code_bytes;
-    wp.ops_bytes = pl->ops_bytes;
+    WalkParams wp = make_walk_params(pl);
     {
         int rc = launch_walk(pl, wp);
         if (rc) return rc;
@@ -1663,6 +1772,7 @@ double gx_plan_stat(const gx_plan *pl, int what) {
         case 26: return (double)pl->reads_bits;
         case 27: return pl->compact ? 2.0 : pl->code_band ? 1.0 : 0.0;
         case 28: return pl->code_band ? (double)*std::max_element(pl->code_w.begin(), pl->code_w.end()) : 0.0;
+        case 29: return pl->start_ms;
         default: return -1.0;
     }
 }

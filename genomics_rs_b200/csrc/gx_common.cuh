@@ -62,9 +62,12 @@ struct PairDesc {
     const uint32_t *ack;
 };
 
-// Code band (global traceback plans): direction codes are only WRITTEN by tiles within `code_w` columns of
-// the table's scaled diagonal j = i*n/m -- where the path of a global alignment runs; every other tile runs the score-only
-// cell (5 instead of 9 instructions).  One flag byte per tile (FillParams / WalkParams::tile_codes, indexed like tile_best;
+// Code band (global traceback plans, and local ones with compact storage): direction codes are only WRITTEN by tiles
+// within `code_w` columns of a line from (a0,b0) to the path's end cell (a1,b1) -- for a global alignment the table's
+// scaled diagonal (0,0)-(m,n); for a local one the slope-1 line back from its start cell (i*,j*) to the table's edge,
+// (i*-d, j*-d) with d = min(i*,j*), found by a score-only pass first.  Above row a0 the line's column is b0; tiles
+// that start at or beyond the end cell are out (the path moves only up and left from it); tile (0,0) is always in.
+// Every other tile runs the score-only cell (5 instead of 9 instructions).  One flag byte per tile (FillParams / WalkParams::tile_codes, indexed like tile_best;
 // null = every tile has codes), written by the host, read by the fill (which variant to run) and by the walk, which
 // verifies that every tile it enters has codes; if a path ever leaves the band the execute is repeated (gx_plan_execute),
 // so results stay exact: with codes everywhere, or -- compact storage -- with a wider band for the pairs that left it.
@@ -72,11 +75,15 @@ struct PairDesc {
 // A slot table (FillParams / WalkParams::tile_slot, indexed like tile_best) maps tile (p,s) to its slot, its codes are at
 // codes_off + slot * tile_code_bytes; an out-of-band tile maps to slot 0 of its pair (tile (0,0) is always in the band),
 // so that every address the kernels form lies inside the codes buffer although nothing is read or written there.
-__host__ inline bool tile_in_code_band(uint64_t m, uint64_t n, uint32_t p, uint32_t s, uint32_t W, uint64_t code_w) {
+__host__ inline bool tile_in_code_band(uint64_t a0, uint64_t b0, uint64_t a1, uint64_t b1, uint64_t m, uint32_t p, uint32_t s,
+                                       uint32_t W, uint64_t code_w) {
     const uint64_t i0 = (uint64_t)p << PANEL_H_LOG2;
     const uint64_t i1 = (i0 + PANEL_H < m) ? i0 + PANEL_H : m;
-    const uint64_t lo = i0 * n / m, hi = i1 * n / m;     // diagonal columns at the tile's first / last row
     const uint64_t c0 = (uint64_t)s * W, c1 = c0 + W;   // the tile's columns [c0, c1)
+    if (p == 0 && s == 0) return true;
+    if (i0 >= a1 || c0 >= b1) return false;
+    auto col = [&](uint64_t i) { return (i <= a0 || a1 == a0) ? b0 : b0 + (i - a0) * (b1 - b0) / (a1 - a0); };
+    const uint64_t lo = col(i0), hi = col(i1);          // the line's columns at the tile's first / last row
     return c1 + code_w > lo && c0 < hi + code_w + 1;
 }
 

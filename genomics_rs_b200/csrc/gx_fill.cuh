@@ -260,7 +260,8 @@ __device__ __forceinline__ void run_batch(int (&eu)[K], int (&du)[K], const int 
 // tile's batch loops and picks one per tile (FillParams::tile_codes).  The choice is made once per tile, around two complete
 // copies of the loops: dispatching per batch inside shared loops slowed a resident strip's traceback variant by 8-40 %
 // (BRCA2 fill 0.99 -> 1.41 ms) even when the other variant never ran.  BAND_COMPACT also takes the tile's code address
-// from its slot (FillParams::tile_slot, gx_common.cuh) instead of from its position in the table.
+// from its slot (FillParams::tile_slot, gx_common.cuh) instead of from its position in the table; its LOCAL instance runs
+// with TRACK 0, after a score-only start-cell pass (TRACK 2) whose tile_best it leaves to the walk.
 constexpr int BAND_NONE = 0, BAND_DENSE = 1, BAND_COMPACT = 2;
 template <int K, bool LOCAL, bool CODES, int TRACK, bool PROF, bool CHAIN1, int BAND = BAND_NONE>
 __global__ void __launch_bounds__(CTA_THREADS, CTAS_PER_SM) gx_fill_kernel(const FillParams P) {

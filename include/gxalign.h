@@ -37,11 +37,13 @@ enum {
     GX_ERR_OPS_CAP = 4,       /* ops buffer too small (need >= m+n+1) */
     GX_ERR_NO_DEVICE = 5,     /* no CUDA device of compute capability 10.x; there is no CPU path */
     GX_ERR_CUDA = 6,          /* CUDA runtime error, see gx_last_error() */
-    GX_ERR_NOMEM = 7,         /* device or host allocation failed / traceback storage would not fit.  A global traceback
-                               * plan whose direction codes do not fit for every tile keeps them for the tiles of the
-                               * code band only (DESIGN.md 2); it fails when even those do not fit, also after the band
-                               * was widened for a path that left it (gx_last_error names the pair, the half-width
-                               * and the bytes).  Local traceback has no band: its codes must fit for every tile. */
+    GX_ERR_NOMEM = 7,         /* device or host allocation failed / traceback storage would not fit.  A traceback plan
+                               * whose direction codes do not fit for every tile keeps them for the tiles of the code
+                               * band only (DESIGN.md 2: global plans around the table's diagonal, local plans around
+                               * the slope-1 line that ends at the start cell); it fails when even those do not fit,
+                               * also after the band was moved to a new start cell or widened for a path that left it
+                               * (gx_last_error names the pair -- "local pair" for a local plan --, the half-width and
+                               * the bytes).  With GX_CODE_BAND=0 there is no band: codes must fit for every tile. */
     GX_ERR_NOT_INIT = 8,      /* gx_init() has not been called */
     GX_ERR_UNSUPPORTED = 9,   /* flag or mode not implemented */
     GX_ERR_INTERNAL = 10      /* impossible traceback state (the reference panics: algo.rs:407-408) */
@@ -135,8 +137,11 @@ int gx_score_batch_cells(const uint8_t *seq_blob, uint64_t blob_len,
  * repeated in ticket mode, and a global traceback plan that writes direction codes only near the table's diagonal
  * (the "code band", DESIGN.md 2) is repeated if any path leaves the band: with codes everywhere, or -- when the plan
  * keeps codes for the band's tiles only (compact storage, stat 27 = 2) -- with the band of each pair whose path left
- * at least doubled and wide enough for where it left, until no path leaves.  The widths stay for the plan's life.  If
- * the widened codes do not fit it returns GX_ERR_NOMEM. */
+ * at least doubled and wide enough for where it left, until no path leaves.  The widths stay for the plan's life.
+ * A local traceback plan with compact storage runs in two phases: a score-only pass finds every pair's start cell
+ * (stat 29), each pair whose start cell moved gets a band of the default half-width around the slope-1 line that ends
+ * there, then the traceback fill and walk run, repeated as above while a path leaves its band.  If the moved or
+ * widened codes do not fit it returns GX_ERR_NOMEM, and so does every later execute of that plan. */
 typedef struct gx_plan gx_plan;
 int gx_plan_create(const uint64_t *len1, const uint64_t *len2, uint64_t n_pairs,
                    gx_scores sc, int is_local, int flags, gx_plan **plan);
@@ -154,7 +159,8 @@ void gx_plan_destroy(gx_plan *plan);
  * 24 executes repeated because a path left the code band, 25 fill scores through the one-hot IDP.4A path (1; set at upload),
  * 26 read plans: lane width of the read kernel the last execute ran (16 = s16x2, 32; 0 before),
  * 27 code storage (0 codes in every tile or none, 1 dense with a code band, 2 compact: codes for the band's tiles only),
- * 28 widest code-band half-width in columns of the last execute (0 without a code band).
+ * 28 widest code-band half-width in columns of the last execute (0 without a code band),
+ * 29 ms of the start-cell pass of the last execute of a compact local plan (0 for other plans; included in stat 0).
  * Any other number returns -1. */
 double gx_plan_stat(const gx_plan *plan, int what);
 
