@@ -4,11 +4,11 @@ this package is the host-side mirror of the reference's interface around it.  No
 from .config import Config, Scores, get_config, parse_config
 from .sequence import Sequence, SequenceContainer
 from .alignment import (AlignedSequences, AlignmentChoice, DeviceTable, Plan, RESULT_DTYPE, align, align_all, align_batch,
-                        alignment_table, k0_measure, pack_pairs, retrace, score_batch, score_planes)
+                        align_reads, alignment_table, k0_measure, pack_pairs, retrace, score_batch, score_planes)
 from .banded import Band, band_range, nw_score_banded, nw_score_banded_local
 from . import _lib
 
 __all__ = ["Config", "Scores", "get_config", "parse_config", "Sequence", "SequenceContainer", "AlignedSequences",
-           "AlignmentChoice", "DeviceTable", "Plan", "RESULT_DTYPE", "align", "align_all", "align_batch", "alignment_table",
-           "k0_measure", "pack_pairs", "retrace", "score_batch", "score_planes",
+           "AlignmentChoice", "DeviceTable", "Plan", "RESULT_DTYPE", "align", "align_all", "align_batch", "align_reads",
+           "alignment_table", "k0_measure", "pack_pairs", "retrace", "score_batch", "score_planes",
            "Band", "band_range", "nw_score_banded", "nw_score_banded_local"]

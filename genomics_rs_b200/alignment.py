@@ -348,6 +348,33 @@ def score_batch(blob: np.ndarray, off1, len1, off2, len2, scores, is_local: bool
     return out
 
 
+def align_reads(blob: np.ndarray, off1, len1, off2, len2, scores, is_local: bool, ops: Optional[np.ndarray] = None,
+                ops_off: Optional[np.ndarray] = None):
+    """gx_align_reads: the whole alignment of every pair of a short-read set (pairs of <= 640 bp), streamed through the
+    read kernel.  -> (results, ops, ops_off): results in RESULT_DTYPE (lcs_at_first_max 0, fill_ms the call's kernel
+    time, walk_ms 0), pair q's ops at ops[ops_off[q] : ops_off[q] + results["n_ops"][q]].  ops_off (n_pairs + 1 entries,
+    ops_off[q+1] - ops_off[q] >= len1[q] + len2[q] + 1) defaults to the packed prefix sums; `ops` (uint8, at least
+    ops_off[-1] bytes) may be supplied to keep the buffer across calls.  Arrays in, arrays out: no per-pair objects."""
+    lib = _lib.ensure_init()
+    blob = np.ascontiguousarray(blob, np.uint8)
+    off1, len1, off2, len2 = [np.ascontiguousarray(x, np.uint64) for x in (off1, len1, off2, len2)]
+    n = int(off1.size)
+    assert len1.size == n and off2.size == n and len2.size == n
+    if ops_off is None:
+        ops_off = np.zeros(n + 1, np.uint64)
+        np.cumsum(len1 + len2 + np.uint64(1), out=ops_off[1:])
+    ops_off = np.ascontiguousarray(ops_off, np.uint64)
+    assert ops_off.size == n + 1
+    if ops is None:
+        ops = np.zeros(max(int(ops_off[-1]), 1), np.uint8)
+    assert ops.dtype == np.uint8 and ops.flags.c_contiguous and ops.size >= int(ops_off[-1])
+    res = np.zeros(n, dtype=RESULT_DTYPE)
+    _lib.check(lib.gx_align_reads(blob.ctypes.data if blob.size else None, blob.size, off1.ctypes.data, len1.ctypes.data,
+                                  off2.ctypes.data, len2.ctypes.data, n, _scores_struct(scores), int(bool(is_local)),
+                                  res.ctypes.data, ops.ctypes.data, ops_off.ctypes.data))
+    return res, ops, ops_off
+
+
 def k0_measure() -> dict:
     """INT32/DPX issue rates measured on this GPU, CUDA-event timed (warp-instructions per clock per SM):
     the ALU pipe (VIADDMNMX, VIMNMX3), the FMA pipe (IMAD, IDP.4A), both together, and the dependency-free instruction

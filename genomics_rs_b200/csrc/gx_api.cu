@@ -1,6 +1,7 @@
 // gx_api.cu -- C ABI of libgxalign (include/gxalign.h): context, plans, kernel dispatch.
 // No CPU compute path exists in this file: every entry point needs a live sm_100 device.
 #include <algorithm>
+#include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -44,6 +45,14 @@ struct Ctx {
     size_t lane_scores_cap = 0;
     uint32_t *lane_cells_host[NLANES] = {nullptr, nullptr, nullptr};   // pinned: start cells (gx_score_batch_cells, local)
     size_t lane_cells_cap = 0;
+    // gx_align_reads, pinned: per-pair traceback records and op offsets, and the op bytes of the chunk in flight
+    ReadTb *lane_tb_host[NLANES] = {nullptr, nullptr, nullptr};
+    uint32_t *lane_opoff_host[NLANES] = {nullptr, nullptr, nullptr};
+    size_t lane_tb_cap = 0;
+    uint8_t *lane_ops_host[NLANES] = {nullptr, nullptr, nullptr};
+    size_t lane_ops_cap[NLANES] = {0, 0, 0};
+    cudaEvent_t lane_k0[NLANES] = {nullptr, nullptr, nullptr};   // around each lane's read kernel (fill_ms)
+    cudaEvent_t lane_k1[NLANES] = {nullptr, nullptr, nullptr};
     int host_threads = 1;                             // worker threads for the host passes over a chunk
     uint8_t *ops_stage = nullptr;                     // pinned D2H staging of op lists (grown on demand)
     size_t ops_stage_cap = 0;
@@ -551,6 +560,8 @@ int gx_init(int device) try {
     for (int k = 0; k < Ctx::NLANES; ++k) {
         CK(cudaStreamCreateWithFlags(&c->lane_stream[k], cudaStreamNonBlocking));
         CK(cudaEventCreateWithFlags(&c->lane_done[k], cudaEventDisableTiming));
+        CK(cudaEventCreate(&c->lane_k0[k]));
+        CK(cudaEventCreate(&c->lane_k1[k]));
     }
     {
         // host passes of the streamed read path: a few threads per process (one process per GPU shares the host)
@@ -582,6 +593,11 @@ void gx_shutdown(void) {
         if (g_ctx->lane_scores_host[k]) cudaFreeHost(g_ctx->lane_scores_host[k]);
         if (g_ctx->lane_rec_host[k]) cudaFreeHost(g_ctx->lane_rec_host[k]);
         if (g_ctx->lane_cells_host[k]) cudaFreeHost(g_ctx->lane_cells_host[k]);
+        if (g_ctx->lane_k0[k]) cudaEventDestroy(g_ctx->lane_k0[k]);
+        if (g_ctx->lane_k1[k]) cudaEventDestroy(g_ctx->lane_k1[k]);
+        if (g_ctx->lane_tb_host[k]) cudaFreeHost(g_ctx->lane_tb_host[k]);
+        if (g_ctx->lane_opoff_host[k]) cudaFreeHost(g_ctx->lane_opoff_host[k]);
+        if (g_ctx->lane_ops_host[k]) cudaFreeHost(g_ctx->lane_ops_host[k]);
     }
     if (g_ctx->ops_stage) cudaFreeHost(g_ctx->ops_stage);
     cudaStreamDestroy(g_ctx->stream);
@@ -963,14 +979,26 @@ static void host_parallel(int threads, uint64_t n, F &&f) {   // f(tid, lo, hi) 
     for (auto &t : th) t.join();
 }
 
+// gx_align_reads: the caller's outputs (gx_align_batch's traceback arguments)
+struct ReadsTrace {
+    gx_result *out;
+    uint8_t *ops_blob;
+    const uint64_t *ops_off;
+};
+
 // start_i / start_j (both or neither): also each pair's start cell -- the read kernels' for local batches, (m, n) for global.
+// tr (traceback, gx_align_reads): instead of scores, each pair's whole alignment from the 32-bit kernel's traceback
+// instances, for any n_pairs.  Op bytes go to a per-chunk device buffer at prefix offsets of len1 + len2 + 1 (one more
+// array on the wire, 4 B per pair), and come back with a 20-byte record per pair.  The chunks' kernels run one after
+// another (each fills the device and owns the one code scratch buffer); their copies still overlap.
 static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const uint64_t *off1, const uint64_t *len1,
                                 const uint64_t *off2, const uint64_t *len2, uint64_t n_pairs, gx_scores sc, int is_local,
-                                int64_t *scores, uint64_t *start_i, uint64_t *start_j, bool force32) {
+                                int64_t *scores, uint64_t *start_i, uint64_t *start_j, bool force32,
+                                const ReadsTrace *tr = nullptr) {
     std::lock_guard<std::recursive_mutex> lk(g_mu);
     if (!g_ctx) return GX_ERR_NOT_INIT;
     Ctx *c = g_ctx;
-    if (n_pairs < (1u << 18) || (is_local && sc.s_mismatch >= 0)) return GX_ERR_UNSUPPORTED;
+    if ((!tr && n_pairs < (1u << 18)) || (is_local && sc.s_mismatch >= 0)) return GX_ERR_UNSUPPORTED;
     int rc = check_scores_impl(sc, READS_MAX_LEN, READS_MAX_LEN, is_local != 0);
     if (rc) return rc;
     CK(cudaSetDevice(c->device));
@@ -1005,26 +1033,93 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
         }
         c->lane_cells_cap = CH;
     }
+    if (tr && c->lane_tb_cap < CH) {
+        for (int k = 0; k < NL; ++k) {
+            if (c->lane_tb_host[k]) cudaFreeHost(c->lane_tb_host[k]);
+            c->lane_tb_host[k] = nullptr;
+            if (c->lane_opoff_host[k]) cudaFreeHost(c->lane_opoff_host[k]);
+            c->lane_opoff_host[k] = nullptr;
+            if (cudaHostAlloc((void **)&c->lane_tb_host[k], CH * sizeof(ReadTb), cudaHostAllocDefault) != cudaSuccess ||
+                cudaHostAlloc((void **)&c->lane_opoff_host[k], CH * sizeof(uint32_t), cudaHostAllocDefault) != cudaSuccess) {
+                cudaGetLastError();
+                c->lane_tb_cap = 0;
+                return GX_ERR_NOMEM;
+            }
+        }
+        c->lane_tb_cap = CH;
+    }
     struct Lane {
         uint8_t *blob = nullptr;
         size_t blob_cap = 0;
         uint4 *rec = nullptr;
         int *scores = nullptr;
         uint32_t *cells = nullptr;
+        uint32_t *opoff = nullptr;   // traceback: per pair, its first op byte in `ops`
+        ReadTb *tb = nullptr;
+        uint8_t *ops = nullptr;
+        size_t ops_cap = 0;
         uint64_t first = 0, count = 0;
         bool busy = false;
     } lane[NL];
+    unsigned long long *codes = nullptr;   // traceback: code scratch of the running kernel (one slot per resident warp)
+    size_t codes_cap = 0;
+    uint32_t *check = nullptr;             // traceback: checked build's bounds-check site
+    int prev_lane = -1;                    // traceback: lane of the previous chunk's kernel
+    double kernel_ms = 0.0;
     auto release = [&]() {
         for (auto &L : lane) {
-            void *ptrs[] = {L.blob, L.rec, L.scores, L.cells};
+            void *ptrs[] = {L.blob, L.rec, L.scores, L.cells, L.opoff, L.tb, L.ops};
             for (void *p : ptrs) pool_free(c, p);
         }
+        pool_free(c, codes);
+        pool_free(c, check);
     };
     auto drain = [&](int k) -> int {   // scores (and start cells) of the chunk that ran on lane k -> caller's arrays
         Lane &L = lane[k];
         if (!L.busy) return GX_OK;
         cudaError_t e = cudaEventSynchronize(c->lane_done[k]);
         if (e != cudaSuccess) return fail_cuda(e, "cudaEventSynchronize(lane_done)");
+        if (tr) {
+            float ms = 0.f;
+            e = cudaEventElapsedTime(&ms, c->lane_k0[k], c->lane_k1[k]);
+            if (e != cudaSuccess) return fail_cuda(e, "cudaEventElapsedTime(lane kernel)");
+            kernel_ms += ms;
+            const ReadTb *tb = c->lane_tb_host[k];
+            const uint32_t *oo = c->lane_opoff_host[k];
+            const uint8_t *ob = c->lane_ops_host[k];
+            std::atomic<bool> bad{false};
+            host_parallel(T, L.count, [&](int, uint64_t a, uint64_t b) {
+                for (uint64_t q = a; q < b; ++q) {
+                    const ReadTb &t = tb[q];
+                    const uint64_t p = L.first + q;
+                    gx_result r;
+                    r.score = t.score;
+                    r.start_i = t.start >> 16;
+                    r.start_j = t.start & 0xffffu;
+                    r.end_i = t.end >> 16;
+                    r.end_j = t.end & 0xffffu;
+                    r.matches = t.match_mis & 0xffffu;
+                    r.mismatches = t.match_mis >> 16;
+                    r.gap_extensions = t.ext_open & 0xffffu;
+                    r.opening_gaps = t.ext_open >> 16;
+                    r.n_ops = r.matches + r.mismatches + r.gap_extensions + r.opening_gaps;
+                    r.lcs_at_first_max = 0;
+                    r.fill_ms = r.walk_ms = 0.0;   // fill_ms: the whole call's, once every chunk is back
+                    tr->out[p] = r;
+                    if (r.n_ops > len1[p] + len2[p] + 1) {   // the device would have written past the pair's op range
+                        bad = true;
+                        continue;
+                    }
+                    memcpy(tr->ops_blob + tr->ops_off[p], ob + oo[q], r.n_ops);
+                }
+            });
+            L.busy = false;
+            if (bad) {
+                g_err = "read traceback: an op count exceeds m + n + 1";
+                return GX_ERR_INTERNAL;
+            }
+            return GX_OK;
+        }
         const int *src = c->lane_scores_host[k];
         int64_t *dst = scores + L.first;
         for (uint64_t q = 0; q < L.count; ++q) dst[q] = src[q];
@@ -1046,11 +1141,19 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
     for (int k = 0; k < NL && rc == GX_OK; ++k) {
         Lane &L = lane[k];
         rc = pool_alloc(c, CH * sizeof(uint4), (void **)&L.rec);
-        if (!rc) rc = pool_alloc(c, CH * 4, (void **)&L.scores);
+        if (!rc && !tr) rc = pool_alloc(c, CH * 4, (void **)&L.scores);
         if (!rc && cells) rc = pool_alloc(c, CH * 4, (void **)&L.cells);
+        if (!rc && tr) rc = pool_alloc(c, CH * sizeof(uint32_t), (void **)&L.opoff);
+        if (!rc && tr) rc = pool_alloc(c, CH * sizeof(ReadTb), (void **)&L.tb);
+    }
+    if (!rc && tr) rc = pool_alloc(c, sizeof(uint32_t), (void **)&check);
+    if (!rc && tr) {   // before the first kernel, which runs on lane 0; every later one waits for the one before it
+        const cudaError_t e = cudaMemsetAsync(check, 0, sizeof(uint32_t), c->lane_stream[0]);
+        if (e != cudaSuccess) rc = fail_cuda(e, "cudaMemsetAsync(check)");
     }
     struct Part {
         uint64_t lo = UINT64_MAX, hi = 0, maxlen = 0, sum = 0, bad = 0;
+        uint64_t ops = 0, ops_bad = 0;   // traceback: op bytes of the slice; an ops_off gap below len1 + len2 + 1
     };
     std::vector<Part> parts((size_t)std::max(T, 1));
     // errors inside the chunk loop leave through `break`: the lanes are drained and their pool blocks released below
@@ -1079,15 +1182,25 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
                 p.maxlen = std::max(p.maxlen, std::max(l1[q], l2[q]));
                 p.sum += l1[q] + l2[q];
             }
+            if (tr) {
+                const uint64_t *oo = tr->ops_off + first;
+                for (uint64_t q = a; q < b; ++q) {
+                    const uint64_t need = l1[q] + l2[q] + 1;
+                    p.ops += need;
+                    p.ops_bad |= (uint64_t)(oo[q + 1] < oo[q]) | (uint64_t)(oo[q + 1] - oo[q] < need);
+                }
+            }
             parts[(size_t)tid] = p;
         });
-        uint64_t lo = UINT64_MAX, hi = 0, maxlen = 0, sum = 0, badbits = 0;
+        uint64_t lo = UINT64_MAX, hi = 0, maxlen = 0, sum = 0, badbits = 0, ops_bytes = 0, ops_bad = 0;
         for (const auto &p : parts) {
             lo = std::min(lo, p.lo);
             hi = std::max(hi, p.hi);
             maxlen = std::max(maxlen, p.maxlen);
             sum += p.sum;
             badbits |= p.bad;
+            ops_bytes += p.ops;
+            ops_bad |= p.ops_bad;
         }
         if (badbits) {
             rc = GX_ERR_ARG;
@@ -1097,8 +1210,32 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
             rc = GX_ERR_UNSUPPORTED;   // long pairs or a scattered blob: not a read stream
             break;
         }
+        if (ops_bad) {
+            rc = GX_ERR_OPS_CAP;
+            break;
+        }
         rc = drain(k);                 // the chunk that used this lane NLANES rounds ago
         if (rc) break;
+        if (tr && L.ops_cap < ops_bytes) {   // lane k's buffers are idle: drain(k) waited for its last chunk
+            pool_free(c, L.ops);
+            L.ops = nullptr;
+            L.ops_cap = 0;
+            const size_t want = ops_bytes + ops_bytes / 4 + 64;
+            rc = pool_alloc(c, want, (void **)&L.ops);
+            if (rc) break;
+            L.ops_cap = want;
+            if (c->lane_ops_cap[k] < want) {
+                if (c->lane_ops_host[k]) cudaFreeHost(c->lane_ops_host[k]);
+                c->lane_ops_host[k] = nullptr;
+                c->lane_ops_cap[k] = 0;
+                if (cudaHostAlloc((void **)&c->lane_ops_host[k], want, cudaHostAllocDefault) != cudaSuccess) {
+                    cudaGetLastError();
+                    rc = GX_ERR_NOMEM;
+                    break;
+                }
+                c->lane_ops_cap[k] = want;
+            }
+        }
         const uint64_t span = hi > lo ? hi - lo : 0;
         if (L.blob_cap < span + 64) {
             pool_free(c, L.blob);
@@ -1114,13 +1251,23 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
         // (lane k's record buffer is free: drain(k) above waited for the chunk that used it)
         {
             uint4 *rec = c->lane_rec_host[k];
-            host_parallel(T, count, [&](int, uint64_t a, uint64_t b) {
+            uint32_t *oo = c->lane_opoff_host[k];
+            host_parallel(T, count, [&](int tid, uint64_t a, uint64_t b) {
                 for (uint64_t q = a; q < b; ++q)
                     rec[q] = make_uint4((uint32_t)(o1[q] - lo), (uint32_t)(o2[q] - lo), (uint32_t)l1[q], (uint32_t)l2[q]);
+                if (tr) {   // the same slices as pass 1: this slice's ops start after those of the slices before it
+                    uint64_t at = 0;
+                    for (int s = 0; s < tid; ++s) at += parts[(size_t)s].ops;
+                    for (uint64_t q = a; q < b; ++q) {
+                        oo[q] = (uint32_t)at;
+                        at += l1[q] + l2[q] + 1;
+                    }
+                }
             });
         }
         CKB(cudaMemcpyAsync(L.rec, c->lane_rec_host[k], count * sizeof(uint4), cudaMemcpyHostToDevice, st));
-        ReadsParams rp;
+        if (tr) CKB(cudaMemcpyAsync(L.opoff, c->lane_opoff_host[k], count * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        ReadsParams rp{};
         rp.blob = L.blob;
         rp.off1 = rp.off2 = nullptr;
         rp.len1 = rp.len2 = nullptr;
@@ -1134,13 +1281,51 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
         rp.h = sc.h;
         rp.is_local = is_local ? 1 : 0;
         rp.cells = cells ? L.cells : nullptr;
-        if (launch_reads(rp, (int)maxlen, c->sm_count, st, force32) != 0) {
-            rc = GX_ERR_UNSUPPORTED;
-            break;
+        if (tr) {
+            ReadsTbShape sh;
+            if (reads_tb_shape((int)maxlen, is_local != 0, c->sm_count, &sh) != 0) {
+                rc = GX_ERR_UNSUPPORTED;
+                break;
+            }
+            const uint64_t n_slots = (uint64_t)sh.grid * 8;
+            const size_t need = n_slots * sh.slot_words * 8;
+            if (codes_cap < need) {
+                // the previous chunk's kernel may still use the old scratch: let it finish before the block is reused
+                if (prev_lane >= 0) CKB(cudaEventSynchronize(c->lane_k1[prev_lane]));
+                pool_free(c, codes);
+                codes = nullptr;
+                codes_cap = 0;
+                rc = pool_alloc(c, need, (void **)&codes);
+                if (rc) break;
+                codes_cap = need;
+            }
+            ReadsTbParams tp;
+            static_cast<ReadsParams &>(tp) = rp;
+            tp.codes = codes;
+            tp.slot_words = sh.slot_words;
+            tp.n_slots = (uint32_t)n_slots;
+            tp.ops_off = L.opoff;
+            tp.ops = L.ops;
+            tp.ops_bytes = L.ops_cap;
+            tp.tb = L.tb;
+            tp.check = check;
+            if (prev_lane >= 0) CKB(cudaStreamWaitEvent(st, c->lane_k1[prev_lane], 0));
+            CKB(cudaEventRecord(c->lane_k0[k], st));
+            sh.kern<<<sh.grid, 256, 0, st>>>(tp);
+            CKB(cudaGetLastError());
+            CKB(cudaEventRecord(c->lane_k1[k], st));
+            prev_lane = k;
+            CKB(cudaMemcpyAsync(c->lane_tb_host[k], L.tb, count * sizeof(ReadTb), cudaMemcpyDeviceToHost, st));
+            CKB(cudaMemcpyAsync(c->lane_ops_host[k], L.ops, ops_bytes, cudaMemcpyDeviceToHost, st));
+        } else {
+            if (launch_reads(rp, (int)maxlen, c->sm_count, st, force32) != 0) {
+                rc = GX_ERR_UNSUPPORTED;
+                break;
+            }
+            CKB(cudaGetLastError());
+            CKB(cudaMemcpyAsync(c->lane_scores_host[k], L.scores, count * 4, cudaMemcpyDeviceToHost, st));
+            if (cells) CKB(cudaMemcpyAsync(c->lane_cells_host[k], L.cells, count * 4, cudaMemcpyDeviceToHost, st));
         }
-        CKB(cudaGetLastError());
-        CKB(cudaMemcpyAsync(c->lane_scores_host[k], L.scores, count * 4, cudaMemcpyDeviceToHost, st));
-        if (cells) CKB(cudaMemcpyAsync(c->lane_cells_host[k], L.cells, count * 4, cudaMemcpyDeviceToHost, st));
         CKB(cudaEventRecord(c->lane_done[k], st));
         L.first = first;
         L.count = count;
@@ -1148,6 +1333,19 @@ static int score_batch_streamed(const uint8_t *blob, uint64_t blob_len, const ui
     }
 #undef CKB
     for (int k = 0; k < NL && rc == GX_OK; ++k) rc = drain(k);
+    if (rc == GX_OK && tr && n_pairs) {
+        uint32_t site = 0;
+        const cudaError_t e = cudaMemcpy(&site, check, sizeof site, cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) rc = fail_cuda(e, "cudaMemcpy(check)");
+        else if (site) {
+            g_err = "checked build: device bounds check failed at site " + std::to_string(site);
+            rc = GX_ERR_INTERNAL;
+        } else {
+            host_parallel(T, n_pairs, [&](int, uint64_t a, uint64_t b) {
+                for (uint64_t q = a; q < b; ++q) tr->out[q].fill_ms = kernel_ms;
+            });
+        }
+    }
     if (rc != GX_OK) {
         for (int k = 0; k < NL; ++k) cudaStreamSynchronize(c->lane_stream[k]);
         cudaGetLastError();
@@ -2166,6 +2364,17 @@ int gx_score_batch_cells(const uint8_t *seq_blob, uint64_t blob_len, const uint6
         start_j[q] = res[q].start_j;
     }
     return GX_OK;
+}
+GX_GUARD_END
+
+int gx_align_reads(const uint8_t *seq_blob, uint64_t blob_len, const uint64_t *off1, const uint64_t *len1, const uint64_t *off2,
+                   const uint64_t *len2, uint64_t n_pairs, gx_scores sc, int is_local, gx_result *out, uint8_t *ops_blob,
+                   const uint64_t *ops_off) try {
+    if ((!seq_blob && blob_len) || ((!off1 || !len1 || !off2 || !len2 || !out || !ops_blob || !ops_off) && n_pairs))
+        return GX_ERR_ARG;
+    const ReadsTrace tr{out, ops_blob, ops_off};
+    return score_batch_streamed(seq_blob, blob_len, off1, len1, off2, len2, n_pairs, sc, is_local, nullptr, nullptr, nullptr, false,
+                                &tr);
 }
 GX_GUARD_END
 

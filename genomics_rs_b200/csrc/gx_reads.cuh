@@ -13,14 +13,31 @@
 // TRACK (local only): also the start cell, the last cell in row-major order that attains the table maximum
 // (algo.rs:306-323), (m, n) when that maximum is 0.  By the argument above no cell outside the table can tie a
 // positive maximum, so only the zero rule needs handling.  Output: one uint32 per pair, i << 16 | j.
+//
+// TB (gx_align_reads): also the alignment.  Every step a lane stores the 2-bit direction codes of its K cells
+// (0 S, 1 I, 2 D: the order retrace tests them, as gx_fill.cuh stores them) as one 8-byte word into its warp's scratch
+// slot, [step][lane], which the warp's next pairs overwrite: code memory is (resident warps x slot), whatever the batch.
+// After the last step the group that filled a pair walks it (reads_walk): the walk of one group overlaps the fill of
+// the other resident warps.  Local instances start from the TRACK start cell.  Codes of padded rows and columns are
+// stored but never read.
 #pragma once
 #include <cstdlib>
+#include <type_traits>
 
 #include "gx_common.cuh"
 
 namespace gx {
 
 constexpr int READS_MAX_LEN = 640;
+
+// traceback result of one pair (gx_align_reads), 20 bytes on the wire; the host expands it into gx_result.  Counters
+// stay below 2^16 (m + n + 1 <= 1281) and n_ops is their sum.
+struct ReadTb {
+    int score;
+    uint32_t start, end;     // i << 16 | j: the start cell and the last emitted cell
+    uint32_t match_mis;      // matches | mismatches << 16
+    uint32_t ext_open;       // gap_extensions | opening_gaps << 16
+};
 
 struct ReadsParams;
 
@@ -36,6 +53,99 @@ struct ReadsParams {
     int a, b, g, h, is_local;
     uint32_t *cells;      // local start cells (i << 16 | j), or null: score only
 };
+
+// the TB kernels' parameters (a separate type: the other instances keep theirs, and their code)
+struct ReadsTbParams : ReadsParams {
+    unsigned long long *codes;   // scratch: warp w's slot at codes + w * slot_words, word [step * 32 + lane]
+    uint64_t slot_words;         // 32 * (longest length of the kernel's class + G - 1)
+    uint32_t n_slots;            // warps of the grid
+    const uint32_t *ops_off;     // per pair: its first op byte in `ops`
+    uint8_t *ops;
+    uint64_t ops_bytes;
+    ReadTb *tb;
+    uint32_t *check;             // checked build: where a failed bounds check records its site
+};
+
+// Traceback walk of one pair by the group that filled it (retrace, algo.rs:287-441, as gx_walk.cuh and the oracle's
+// compact walk do it): from (i, j), the off-by-one label is_match(i, j) with None == None at i = m / j = n, open/extend
+// labels from the previous direction, the checked_sub moves, stop at (0, 0) after a move; a local walk runs on through
+// zero cells and stops on row or column 0, a global one follows row 0 / column 0 to (0, 0).  Lane x of the group looks
+// x cells ahead in the current direction; a ballot gives the run of equal codes, and each lane labels and stores its
+// own op of the run.  grp: the group's columns of the slot (word [step * 32 + lane of group]).
+template <int G, int K, bool LOCAL>
+__device__ __forceinline__ void reads_walk(const ReadsTbParams &P, uint64_t q, const uint8_t *s1, const uint8_t *s2, int m, int n,
+                                           int score, uint32_t i, uint32_t j, const unsigned long long *grp, uint32_t gofs) {
+    const uint32_t gbase = (threadIdx.x & 31) / G * G;
+    const unsigned gmask = (G == 32) ? 0xffffffffu : ((1u << G) - 1u) << gbase;
+    const uint32_t x = (threadIdx.x & 31) - gbase;
+    const uint32_t obase = P.ops_off[q];
+    uint8_t *ops = P.ops + obase;
+    auto code = [&](uint32_t ci, uint32_t cj) -> uint32_t {   // interior cell (ci, cj): row ci-1 is step ci-1+l of lane l
+        const uint32_t l = (cj - 1u) / K, k = (cj - 1u) - l * K;
+        const uint64_t w = (uint64_t)(ci - 1u + l) * 32u + l;
+        GX_CHECK(P.check, gofs + w < P.slot_words && ci >= 1u && ci <= (uint32_t)m && cj >= 1u && cj <= (uint32_t)n, 31);
+        return (uint32_t)(grp[w] >> (2u * k)) & 3u;
+    };
+    auto store = [&](uint32_t idx, uint32_t op) {
+        GX_CHECK(P.check, idx <= (uint32_t)(m + n) && (uint64_t)obase + idx < P.ops_bytes, 32);
+        ops[idx] = (uint8_t)op;
+    };
+    const uint32_t start = i << 16 | j;
+    uint32_t nops = 0, prevc = 0, nm = 0, nx = 0, ne = 0, no = 0, ei = i, ej = j;
+    if (i == 0u && j == 0u) {
+        // only for m == n == 0: one Match at (0, 0) (None == None), then both checked_subs fail
+        if (x == 0u) store(0u, 0u);
+        nops = nm = 1u;
+    } else {
+        bool walking = i != 0u && j != 0u;
+        uint32_t c0 = walking ? code(i, j) : 0u;
+        while (walking) {
+            const uint32_t di = (c0 != 1u) ? 1u : 0u, dj = (c0 != 2u) ? 1u : 0u;
+            const uint32_t ci = i - x * di, cj = j - x * dj;
+            const bool inside = (di == 0u || x < i) && (dj == 0u || x < j);
+            const uint32_t cx = inside ? code(ci, cj) : 3u;
+            const uint32_t same = (__ballot_sync(gmask, cx == c0) & gmask) >> gbase;
+            const uint32_t run = min((uint32_t)__ffs((int)~same) - 1u, (uint32_t)G);   // >= 1: lane 0 holds c0
+            const uint32_t c_next = __shfl_sync(gmask, cx, (int)(run & (G - 1u)), G);
+            const bool mine = x < run;
+            uint32_t op;
+            if (c0 == 0u) {
+                const int a = (mine && ci < (uint32_t)m) ? (int)__ldg(s1 + ci) : -1;
+                const int b = (mine && cj < (uint32_t)n) ? (int)__ldg(s2 + cj) : -1;
+                const uint32_t hit = (uint32_t)__popc(__ballot_sync(gmask, mine && a == b) & gmask);
+                nm += hit;
+                nx += run - hit;
+                op = (a == b) ? 0u : 1u;
+            } else {
+                const uint32_t opens = (c0 != prevc) ? 1u : 0u;   // last_choice differs (algo.rs:373-379, 388-394)
+                op = ((c0 == 1u) ? 2u : 3u) + ((x == 0u && opens) ? 2u : 0u);
+                no += opens;
+                ne += run - opens;
+            }
+            if (mine) store(nops + x, op);
+            ei = i - (run - 1u) * di;
+            ej = j - (run - 1u) * dj;
+            i -= run * di;
+            j -= run * dj;
+            nops += run;
+            prevc = c0;
+            if (i == 0u || j == 0u) break;
+            c0 = (run < (uint32_t)G) ? c_next : code(i, j);   // a shorter run ended at an interior cell a lane has read
+        }
+        // global: row 0 holds only insert scores, column 0 only delete scores (algo.rs:204-220); (0, 0) is never emitted
+        if (!LOCAL && (i == 0u) != (j == 0u)) {
+            const uint32_t c = (i == 0u) ? 1u : 2u, left = i + j, opens = (c != prevc) ? 1u : 0u;
+            for (uint32_t b = 0; b < left; b += G)
+                if (b + x < left) store(nops + b + x, ((c == 1u) ? 2u : 3u) + ((b + x == 0u && opens) ? 2u : 0u));
+            no += opens;
+            ne += left - opens;
+            nops += left;
+            ei = (i == 0u) ? 0u : 1u;
+            ej = (i == 0u) ? 1u : 0u;
+        }
+    }
+    if (x == 0u) P.tb[q] = ReadTb{score, start, ei << 16 | ej, nm | nx << 16, ne | no << 16};
+}
 
 // start cell of a local pair from its best (V, i, j): the zero rule of gx_walk.cuh applies to an empty table too
 __device__ __forceinline__ uint32_t reads_cell(int v, uint32_t i, uint32_t j, int m, int n) {
@@ -59,9 +169,10 @@ __device__ __forceinline__ void reads_pair(const ReadsParams &P, uint64_t q, boo
     }
 }
 
-template <int G, int K, bool LOCAL, bool TRACK>
-__global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
+template <int G, int K, bool LOCAL, bool TRACK, bool TB>
+__global__ void __launch_bounds__(256) gx_reads_kernel(const std::conditional_t<TB, ReadsTbParams, ReadsParams> P) {
     static_assert(!TRACK || (LOCAL && K <= 32), "start cells: local only, column index in 5 bits");
+    static_assert(!TB || (TRACK == LOCAL && 2 * K <= 64), "traceback: local walks start at the start cell; K codes in 8 bytes");
     constexpr unsigned FULLM = 0xffffffffu;
     constexpr int GPW = 32 / G;  // groups per warp
     const int lane = threadIdx.x & 31;
@@ -71,6 +182,11 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
     const uint32_t n_warps = (gridDim.x * blockDim.x) >> 5;
     const int g = P.g, hg = P.h + P.g, h = P.h;
     const int ap = P.a - hg, bp = P.b - hg;
+    unsigned long long *slot = nullptr;   // TB: this warp's code slot
+    if constexpr (TB) {
+        GX_CHECK(P.check, warp_global < P.n_slots, 30);
+        slot = P.codes + (uint64_t)warp_global * P.slot_words;
+    }
 
     for (uint64_t base = (uint64_t)warp_global * GPW; base < P.n_pairs; base += (uint64_t)n_warps * GPW) {
         const uint64_t q = base + gw;
@@ -113,12 +229,14 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
             const bool active = LOCAL ? true : (r >= 0 && r < m);  // global: state is frozen outside rows 0..m-1
             int e = el, irun = il, ed = vd;
             int rkey = 0;   // TRACK: largest (V << 5) | k of this row: the last column that attains the row's maximum
+            uint32_t cw[2] = {0u, 0u};   // TB: the step's codes, cell k at bits 2k of the 8-byte word
 #pragma unroll
             for (int k = 0; k < K; ++k) {
                 const int In = LOCAL ? __viaddmax_s32_relu(irun, g, e) : __viaddmax_s32(irun, g, e);
                 const int Dn = LOCAL ? __viaddmax_s32_relu(du[k], g, eu[k]) : __viaddmax_s32(du[k], g, eu[k]);
                 const int Sn = ed + ((c1 == c2[k]) ? ap : bp);
                 const int Vn = LOCAL ? __vimax3_s32_relu(In, Dn, Sn) : __vimax3_s32(In, Dn, Sn);
+                if (TB) cw[k >> 4] |= ((Sn == Vn) ? 0u : (In == Vn) ? 1u : 2u) << (2 * (k & 15));
                 ed = eu[k];
                 const int En = Vn + hg;
                 if (LOCAL) {
@@ -142,8 +260,15 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
                 best = rkey;
                 brow = r;
             }
+            if constexpr (TB) {
+                const uint64_t w = (uint64_t)t * 32u + (uint32_t)lane;
+                GX_CHECK(P.check, w < P.slot_words, 30);
+                slot[w] = (unsigned long long)cw[1] << 32 | cw[0];
+            }
         }
+        if constexpr (TB) __syncwarp();   // the group's code stores before its walk's loads
         int score;
+        uint32_t si = (uint32_t)m, sj = (uint32_t)n;   // TB: where the walk starts
         if (TRACK) {
             // (V, i, j) of the group's best cell: the largest 64-bit key V << 32 | i << 16 | j.  A cell outside the table
             // (r < 0, r >= m or column >= n) may be a lane's best but never ties a positive table maximum, so it can
@@ -153,7 +278,13 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
 #pragma unroll
             for (int off = G / 2; off > 0; off >>= 1) key = max(key, __shfl_xor_sync(FULLM, key, off));
             score = (m == 0 || n == 0) ? 0 : (int)(key >> 32);
-            if (have && lg == 0) P.cells[q] = reads_cell(score, (uint32_t)key >> 16, (uint32_t)key & 0xffffu, m, n);
+            if constexpr (TB) {
+                const uint32_t cell = reads_cell(score, (uint32_t)key >> 16, (uint32_t)key & 0xffffu, m, n);
+                si = cell >> 16;
+                sj = cell & 0xffffu;
+            } else if (have && lg == 0) {
+                P.cells[q] = reads_cell(score, (uint32_t)key >> 16, (uint32_t)key & 0xffffu, m, n);
+            }
         } else if (LOCAL) {
             score = best;
 #pragma unroll
@@ -172,7 +303,9 @@ __global__ void __launch_bounds__(256) gx_reads_kernel(const ReadsParams P) {
             else if (m == 0) score = h + n * g;
             else if (n == 0) score = h + m * g;
         }
-        if (have && lg == 0) {
+        if constexpr (TB) {
+            if (have) reads_walk<G, K, LOCAL>(P, q, s1, s2, m, n, score, si, sj, slot + gw * G, (uint32_t)(gw * G));
+        } else if (have && lg == 0) {
             P.scores[q] = score;
         }
     }
@@ -362,10 +495,35 @@ static int launch_reads_gk(const ReadsParams &rp, int sm_count, cudaStream_t st)
     uint64_t cap = (uint64_t)sm_count * 8;
     int grid = (int)(want < cap ? want : cap);
     if (grid < 1) grid = 1;
-    if (rp.is_local && rp.cells) gx_reads_kernel<G, K, true, true><<<grid, threads, 0, st>>>(rp);
-    else if (rp.is_local) gx_reads_kernel<G, K, true, false><<<grid, threads, 0, st>>>(rp);
-    else gx_reads_kernel<G, K, false, false><<<grid, threads, 0, st>>>(rp);
+    if (rp.is_local && rp.cells) gx_reads_kernel<G, K, true, true, false><<<grid, threads, 0, st>>>(rp);
+    else if (rp.is_local) gx_reads_kernel<G, K, true, false, false><<<grid, threads, 0, st>>>(rp);
+    else gx_reads_kernel<G, K, false, false, false><<<grid, threads, 0, st>>>(rp);
     return 0;
+}
+
+// Traceback kernels (gx_align_reads), the 32-bit kernel's classes.  The grid is every CTA the device holds at once, so
+// that each warp owns one code slot for the whole launch; a slot holds the longest pair of the class.
+using ReadsKernel = void (*)(const ReadsTbParams);
+struct ReadsTbShape {
+    ReadsKernel kern;
+    int grid;               // CTAs of 256 threads
+    uint64_t slot_words;    // 8-byte code words per warp slot
+};
+template <int G, int K>
+static int reads_tb_shape_gk(bool local, int sm_count, ReadsTbShape *sh) {
+    sh->kern = local ? gx_reads_kernel<G, K, true, true, true> : gx_reads_kernel<G, K, false, false, true>;
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sh->kern, 256, 0) != cudaSuccess || per_sm < 1) return -1;
+    sh->grid = per_sm * sm_count;
+    sh->slot_words = 32ull * (uint64_t)(G * K + G - 1);
+    return 0;
+}
+// -1: max_len is longer than the longest class, or the occupancy query failed
+static int reads_tb_shape(int max_len, bool local, int sm_count, ReadsTbShape *sh) {
+    if (max_len <= 8 * 19) return reads_tb_shape_gk<8, 19>(local, sm_count, sh);
+    if (max_len <= 16 * 20) return reads_tb_shape_gk<16, 20>(local, sm_count, sh);
+    if (max_len <= 32 * 20) return reads_tb_shape_gk<32, 20>(local, sm_count, sh);
+    return -1;
 }
 
 // returns -1 if max_len is not supported by this kernel family; *bits (if given) = lane width of the kernel launched.

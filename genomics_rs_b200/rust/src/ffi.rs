@@ -77,4 +77,9 @@ extern "C" {
         seq_blob: *const u8, blob_len: u64, off1: *const u64, len1: *const u64, off2: *const u64, len2: *const u64,
         n_pairs: u64, sc: gx_scores, is_local: c_int, scores: *mut i64, start_i: *mut u64, start_j: *mut u64,
     ) -> c_int;
+    // gx_align_batch(.., GX_FLAG_TRACEBACK)'s results for short-read sets (pairs <= 640 bp), streamed on the read kernel
+    pub fn gx_align_reads(
+        seq_blob: *const u8, blob_len: u64, off1: *const u64, len1: *const u64, off2: *const u64, len2: *const u64,
+        n_pairs: u64, sc: gx_scores, is_local: c_int, out: *mut gx_result, ops_blob: *mut u8, ops_off: *const u64,
+    ) -> c_int;
 }

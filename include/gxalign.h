@@ -131,6 +131,23 @@ int gx_score_batch_cells(const uint8_t *seq_blob, uint64_t blob_len,
                          gx_scores sc, int is_local,
                          int64_t *scores, uint64_t *start_i, uint64_t *start_j);
 
+/* ---- traceback for short-read sets (BASELINE config 4 with alignments): for every pair exactly the gx_result and op
+ * bytes of gx_align_batch(..., GX_FLAG_TRACEBACK), computed by the inter-task read kernel (fill, direction codes in a
+ * per-warp scratch slot, walk by the lane group that filled the pair) and streamed in chunks of 2^18 pairs like
+ * gx_score_batch, for any n_pairs (0 included).  Device memory does not grow with n_pairs.  Arguments and the ops_off
+ * contract are gx_align_batch's.  Differences: lcs_at_first_max is 0, fill_ms is the summed device time of the call's
+ * read kernels, walk_ms is 0 (the walk runs inside them).  20 bytes per pair plus len1 + len2 + 1 op bytes come back.
+ * Status: GX_ERR_UNSUPPORTED when a pair is longer than 640 bp, when the batch is local with s_mismatch >= 0, or when a
+ * chunk's bytes are too scattered in seq_blob for one span copy (gx_align_batch handles those batches);
+ * GX_ERR_OPS_CAP when ops_off[p+1] - ops_off[p] < len1[p] + len2[p] + 1; GX_ERR_ARG for null pointers or a sequence
+ * outside seq_blob; GX_ERR_SCORES / GX_ERR_RANGE as gx_check_scores for 640 x 640 (local: also
+ * 640 * max(s_match, 0) < 2^26).  After an error the contents of out and ops_blob are unspecified. */
+int gx_align_reads(const uint8_t *seq_blob, uint64_t blob_len,
+                   const uint64_t *off1, const uint64_t *len1,
+                   const uint64_t *off2, const uint64_t *len2, uint64_t n_pairs,
+                   gx_scores sc, int is_local,
+                   gx_result *out, uint8_t *ops_blob, const uint64_t *ops_off);
+
 /* ---- the same, split into phases so that callers can keep inputs resident in HBM, overlap
  * copies, and time the kernels alone.  gx_align_batch == create + upload + execute + fetch (+ destroy, deferred).
  * gx_plan_execute never returns a wrong result for speed's sake: a resident-strips fill that gives up waiting is
